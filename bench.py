@@ -2,7 +2,7 @@
 """Benchmark of the NPI-GNN hot path (BASELINE.json metric: enclosing subgraphs/sec of a
 training step -- GPU extraction + gather + forward + backward + Adam -- at batch 200).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 N = 1 workload: BASELINE.json configs[1] -- synthetic bipartite graph of NPInter2 shape
 (4,636 RNA + 449 protein, ~9.9 k positives + balanced negatives, fold 0 masked), 2-hop
@@ -507,6 +507,15 @@ def timed_steps(run_step, K, sync, flush=None):
     return float(sum(a.elapsed_time(b) for a, b in pairs))
 
 
+def dump_outputs(dirname, arrays):
+    """--dump-outputs: what the timed path computed in its last step, one float32 DIR/<name>.npy per array.  Every
+    input is seeded, so two builds run with the same arguments can be compared output for output.  The arrays are
+    batch-sized or the 97,602-float parameter buffer: a few MB in all."""
+    os.makedirs(dirname, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 # The dominant kernel is ranked by KERNEL, as the ncu launch list groups launches: entry points that launch the same kernel
 # are one family (the transposed aggregation runs under npi_sage_aggregate_bwd for layers 2-3 and under npi_csr_gather_sum
 # for the two gathers of the per-context backward of layer 1).  Entry points that are a sequence of many small integer
@@ -572,10 +581,10 @@ def bench_scoring(args, world, rank, local):
     if args.impl == "reference":
         if rank != 0:
             return
-        steps = min(K, 40)
-        r = cpu_scoring_run(steps, 2, 200)
+        steps = K
+        r = cpu_scoring_run(steps, W, 200)
         print(json.dumps({"impl": "reference", "metric": SCORE_METRIC, "value": r["value"], "unit": SCORE_UNIT, "n_gpus": args.gpus,
-                          "steps": steps, "warmup": 2, "ms_per_step": 1e3 * r["seconds"] / steps, "higher_is_better": True,
+                          "steps": steps, "warmup": W, "ms_per_step": 1e3 * r["seconds"] / steps, "higher_is_better": True,
                           "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic", "config": config,
                           "cpu_baseline": {"value": r["value"], "unit": SCORE_UNIT, "cores": r["cores"], "kind": "port",
                                            "sample": "%d eval forwards of 200 pairs (oracle)" % steps},
@@ -595,8 +604,8 @@ def bench_scoring(args, world, rank, local):
     mine = allp[rank * per:(rank + 1) * per]
     need = (W + K) * SB
     if need > len(mine):
-        K = max(1, len(mine) // SB - W)
-        need = (W + K) * SB
+        raise SystemExit("--steps %d: this GPU's share of the sweep has %d batches of %d pairs, %d of them warm-up"
+                         % (K, len(mine) // SB, SB, W))
     mine = mine[:need]                                        # this rank's slice, first (W+K) batches
     ps = PairSet(g, mine, np.zeros(len(mine), dtype=np.int32), h=2)
     params = FlatParams(g.F, device).init_reference(torch.Generator().manual_seed(0))
@@ -631,6 +640,9 @@ def bench_scoring(args, world, rank, local):
     snap = dict(L.CALL_COUNTS)
     ms = sweep(False)
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        last = (W + K - 1) * SB
+        dump_outputs(args.dump_outputs, {"prob": out[last:last + SB], "logp": sc.engine.logp[:SB]})
     ms = D.max_over_ranks(ms, device) if world > 1 else ms
     ms_e2e = sweep(True)
     ms_e2e = D.max_over_ranks(ms_e2e, device) if world > 1 else ms_e2e
@@ -693,13 +705,11 @@ CPU_STEPS_DEFAULT = {"npinter2": 30, "rpi2241": 200, "x100": 3, "real_h1": 60, "
 def reference_line(args, name):
     """`--impl reference`: the reference's CPU path restated (oracle/), all host threads, K timed steps after W
     warm-up steps of the same workload, config, metric and unit as our arm (a step of x100 is a 256-subgraph
-    sample of the 4096-subgraph global batch -- said in `sample`)."""
+    sample of the 4096-subgraph global batch -- said in `sample`; it takes seconds, so pass a small --steps)."""
     wl = WORKLOADS[name]
     BPR = per_rank_batch(wl, 1)
     cpu_batch = min(BPR, 256) if name == "x100" else BPR
     steps, warm = args.steps, args.warmup
-    if name == "x100":
-        steps, warm = min(steps, 3), min(warm, 1)
     r = cpu_reference_run(wl, steps, warm, cpu_batch)
     world = args.gpus
     config = workload_config(wl, per_rank_batch(wl, world), world)
@@ -769,6 +779,11 @@ def training_workload(name, args, world, rank, local, device, K, W, detail, D=No
     ms = D.max_over_ranks(ms, device) if world > 1 else ms
     clocks = sampler.stop() if rank == 0 else None
     value = K * GBATCH / (ms * 1e-3)
+    if detail and rank == 0 and args.dump_outputs:       # before the end-to-end pass below trains further
+        out = {"logp": tr.engine.logp[:BPR], "loss": tr.engine.loss, "params": tr.params.flat}
+        if exchange is None:       # the gradient Adam applied (the peer exchange sums it inside Adam, it is never stored)
+            out["grads"] = tr._grads_slot[tr.engine.slot].flat      # the slot of the last step, not of the last capture
+        dump_outputs(args.dump_outputs, out)
 
     snap = dict(L.CALL_COUNTS)                           # launches per step, counted from an eager step
     tr._enqueue_fwd_bwd(BPR, GBATCH)
@@ -996,8 +1011,8 @@ def node2vec_stage(args, device, reps=5):
     return res
 
 
-def scoring_sample(args, device, K=20, W=3):
-    """Config 5 in short for `other_workloads`: the first (W+K) batches of the candidate-pair sweep on one GPU."""
+def scoring_sample(args, device, K, W):
+    """Config 5 for `other_workloads`: the first (W+K) batches of the candidate-pair sweep on one GPU."""
     from npi_gnn_b200 import synth
     from npi_gnn_b200.engine import FlatParams, algorithmic_bytes
     from npi_gnn_b200.graph import BipartiteGraph, PairSet
@@ -1007,6 +1022,8 @@ def scoring_sample(args, device, K=20, W=3):
     g = BipartiteGraph(d["edges"], d["is_rna"], d["table"], device=device)
     g.set_mask(synth.masked_pairs(d))
     mine = synth.all_candidate_pairs(d)[:(W + K) * SB]
+    if len(mine) < (W + K) * SB:
+        raise ValueError("--steps %d: the sweep has only %d batches of %d pairs" % (K, len(mine) // SB, SB))
     ps = PairSet(g, mine, np.zeros(len(mine), dtype=np.int32), h=2)
     params = FlatParams(g.F, device).init_reference(torch.Generator().manual_seed(0))
     sc = Scorer(ps, params, batch_size=SB)
@@ -1066,7 +1083,16 @@ def main():
     ap.add_argument("--exchange", default="peer", choices=["peer", "nccl"],
                     help="N > 1: gradient sum over peer memory fused into Adam (default) or an NCCL all-reduce")
     ap.add_argument("--score-batch", type=int, default=2048, help="scoring workload: candidate pairs per forward")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path computed in its last step as DIR/<name>.npy (float32): the log-probabilities "
+                         "of the batch, its loss, the gradient and the updated parameters (scoring: the batch's probabilities "
+                         "and log-probabilities).  Under --gpus > 1: rank 0's share of the batch and loss, the summed gradient, "
+                         "no gradient with the peer exchange")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     args.warmup = max(args.warmup, 3)
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -1105,7 +1131,7 @@ def main():
     nb = tr.num_batches()
     dropin = None
     if world == 1 and not args.no_dropin and name != "x100":
-        dropin = dropin_e2e(ps, g, BPR, max(4, min(K, 12)), 3, device)
+        dropin = dropin_e2e(ps, g, BPR, K, W, device)
     line["e2e"]["dropin_value"] = dropin["value"] if dropin else None
     line["e2e"]["dropin_prefetch_value"] = dropin["prefetch_value"] if dropin else None
     line["e2e"]["dropin"] = dropin
@@ -1154,13 +1180,13 @@ def main():
         del tr, ps
         torch.cuda.empty_cache()
         others = {}
-        for nm, k, w, cs in (("real_h1", 60, 5, 40), ("real_h2", 40, 5, 10), ("rpi2241", 60, 5, 100), ("x100", 3, 3, 1)):
+        for nm, cs in (("real_h1", 40), ("real_h2", 10), ("rpi2241", 100), ("x100", 1)):     # cs: CPU-sample steps
             try:
-                others[nm] = other_training_workload(nm, args, device, k, w, cs)
+                others[nm] = other_training_workload(nm, args, device, K, W, cs)
             except Exception as ex:                      # a failing side workload must not take the bench line down
                 others[nm] = {"error": "%s: %s" % (type(ex).__name__, ex)}
         try:
-            others["scoring"] = scoring_sample(args, device)
+            others["scoring"] = scoring_sample(args, device, K, W)
         except Exception as ex:
             others["scoring"] = {"error": "%s: %s" % (type(ex).__name__, ex)}
         try:

@@ -1,6 +1,6 @@
 """Run the REFERENCE's own extractor (src/classes.py:652-733) in this container.
 
-Container-only helper (needs /root/reference): it registers a minimal ``torch_geometric``
+Needs a checkout of the reference (REF_ROOT below): it registers a minimal ``torch_geometric``
 stub so that ``src/classes.py`` imports unchanged (its imports are at src/classes.py:1-5),
 rebuilds the reference's object graph from a RawDataset exactly as
 src/generate_edgelist.py:61-98 and src/generate_dataset.py:204-216 do, and calls
@@ -15,11 +15,21 @@ import os
 import sys
 import types
 
-REF_ROOT = os.environ.get("NPI_REFERENCE_ROOT", "/root/reference")
+# a checkout of the reference: $NPI_REFERENCE_ROOT, else oracle/_ref (git-ignored, never committed).  The tests that
+# read it are skipped when it is absent (marker `reference`); the tools that read it stop in require_reference().
+REF_ROOT = os.environ.get("NPI_REFERENCE_ROOT") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")
 
 
 def reference_available():
     return os.path.exists(os.path.join(REF_ROOT, "src", "classes.py"))
+
+
+def require_reference():
+    """REF_ROOT, or one clear error when no reference tree is there."""
+    if not reference_available():
+        raise SystemExit("no reference tree at %s: put a checkout of AshuiRUA/NPI-GNN there or set NPI_REFERENCE_ROOT"
+                         % REF_ROOT)
+    return REF_ROOT
 
 
 def _install_stub():
@@ -59,8 +69,7 @@ def _install_stub():
 
 
 def import_reference_classes():
-    if not reference_available():
-        raise RuntimeError("reference tree not present at %s" % REF_ROOT)
+    require_reference()
     _install_stub()
     if REF_ROOT not in sys.path:
         sys.path.insert(0, REF_ROOT)

@@ -10,7 +10,7 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "reference: needs /root/reference (build container only)")
+    config.addinivalue_line("markers", "reference: needs a checkout of the reference at $NPI_REFERENCE_ROOT or oracle/_ref")
 
 
 def pytest_collection_modifyitems(config, items):
@@ -22,4 +22,4 @@ def pytest_collection_modifyitems(config, items):
         if "gpu" in item.keywords and not has_gpu:
             item.add_marker(pytest.mark.skip(reason="no CUDA device"))
         if "reference" in item.keywords and not has_ref:
-            item.add_marker(pytest.mark.skip(reason="/root/reference not present"))
+            item.add_marker(pytest.mark.skip(reason="no reference tree at %s" % ref_import.REF_ROOT))

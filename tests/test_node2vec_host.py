@@ -8,10 +8,10 @@ import numpy as np
 import pytest
 
 from npi_gnn_b200 import node2vec as n2v
-from oracle import node2vec as on2v
+from oracle import node2vec as on2v, ref_import
 from tests.common import GOLD
 
-REF = "/root/reference"
+REF = ref_import.REF_ROOT
 
 
 def test_edgelist_round_trip_and_training_graph(tmp_path):
@@ -66,7 +66,7 @@ def test_word2vec_text_format(tmp_path):
     assert np.allclose(emb[nodes], vec, rtol=1e-6) and not emb[[1, 3, 5, 6, 8, 10, 11]].any()
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree only in the build container")
+@pytest.mark.reference
 def test_flags_and_files_against_the_live_reference():
     src = open(os.path.join(REF, "node2vec-master/src/main.py")).read()
     ref_flags = {}

@@ -53,16 +53,18 @@ def test_case_study_kat(thr):
     assert pos == exp["positives"]
 
 
+@pytest.mark.reference
 @pytest.mark.parametrize("proj", ["1223_1", "1223_1_noKmer"])
 def test_live_every_shipped_fold0_checkpoint(proj):
     """The shipped checkpoints of fold 0 (result/<proj>/model_0_fold/{5..50}) against the
     `testing dataset` lines of result/<proj>/log_0.txt (tests/golden/kat.json carries the ten implied
     confusion matrices per variant): exact known answers computed by the authors' PyG-1.4.2 stack.
-    The checkpoints are read from the reference tree, so this runs where /root/reference exists; five
+    The checkpoints are read from the reference tree, so this runs where that tree is (ref_import.REF_ROOT); seven
     travel as fixtures (test_confusion_matrix_kat), four more per variant are checked here by
     default and all ten with NPI_ALL_KATS=1 (all twenty reproduce exactly)."""
     import os
-    root = "/root/reference/result/%s/model_0_fold" % proj
+    from oracle import ref_import
+    root = os.path.join(ref_import.REF_ROOT, "result", proj, "model_0_fold")
     if not os.path.isdir(root):
         pytest.skip("reference tree not present")
     torch.set_flush_denormal(True)
@@ -81,16 +83,17 @@ def test_live_every_shipped_fold0_checkpoint(proj):
         assert onet.confusion(m, batches) == (exp["TP"], exp["FN"], exp["TN"], exp["FP"]), (proj, ep)
 
 
+@pytest.mark.reference
 @pytest.mark.parametrize("fold", [1, 2, 3, 4])
 def test_live_other_folds_of_project_1223_1(fold):
     """Folds 1-4 of project 1223_1 are shipped too (key sets, per-fold node2vec embedding, ten
     checkpoints and a log per fold and feature variant): the fold's graph and table are rebuilt from
     the raw files (oracle/refdata.py), the test subgraphs extracted and two checkpoints per variant
     compared with their log lines -- 16 more exact known answers (all ten epochs per fold, 80, with
-    NPI_ALL_KATS=1).  Container only: needs /root/reference."""
+    NPI_ALL_KATS=1).  Needs the reference tree (ref_import.REF_ROOT)."""
     import os
-    from oracle import khop, khop_cwrap, refdata
-    ref = "/root/reference"
+    from oracle import khop, khop_cwrap, ref_import, refdata
+    ref = ref_import.REF_ROOT
     if not os.path.isdir(os.path.join(ref, "result", "1223_1", "model_%d_fold" % fold)):
         pytest.skip("reference tree not present")
     torch.set_flush_denormal(True)

@@ -9,7 +9,7 @@ import numpy as np
 import pytest
 import torch
 
-from tests.common import npinter2_oracle_graph
+from tests.common import load_kat, npinter2_oracle_graph
 
 REF_FLAGS = {        # src/train_with_twoDataset.PY:26-43  (flag -> default)
     "trainingName": None, "trainingDatasetName": None, "testingDatasetName": None, "inMemory": 1,
@@ -63,20 +63,19 @@ def test_lr_rule_cadence_and_log_format():
     assert b.line() == "epoch: 15, MCC: 0.9, ACC: 0.95, Pre: 0.9, Sen: 0.9, Spe: 0.9"
 
 
-@pytest.mark.reference
 def test_shipped_log_lines_match_the_format():
-    """Every metric line of the reference's own logs is reproduced byte for byte by metric_line()."""
-    from oracle import ref_import
+    """Every metric line of the reference's own logs that tests/golden/kat.json carries (the testing-dataset lines of
+    result/1223_1/log_0.txt and result/1223_1_noKmer/log_0.txt, verbatim) is reproduced byte for byte by metric_line()."""
     from npi_gnn_b200 import train_shell as ts
-    path = os.path.join(ref_import.REF_ROOT, "result", "1223_1", "log_0.txt")
+    lines = [e["line"] for proj in load_kat()["confusion"].values() for e in proj.values()]
     n = 0
-    for line in open(path, encoding="utf-8", errors="replace").read().splitlines():
+    for line in lines:
         m = re.match(r"^(Epoch: \d{3}, \w+ dataset|result, \w+ dataset), Accuracy: ([\d.]+), Precision: ([\d.]+), "
                      r"Sensitivity: ([\d.]+), Specificity: ([\d.]+), MCC: (-?[\d.]+)$", line)
         if m:
             assert ts.metric_line(m.group(1), tuple(float(v) for v in m.groups()[1:])) == line
             n += 1
-    assert n >= 20
+    assert n == len(lines) and n >= 20
 
 
 def test_run_refuses_cpu_and_bad_inmemory():

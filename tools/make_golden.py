@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Generate tests/golden/ from the reference tree (run in the build container only).
 
-  python tools/make_golden.py            # needs /root/reference
+  python tools/make_golden.py            # needs the reference tree (oracle/ref_import.py: REF_ROOT)
 
 What is produced and where it comes from
   npinter2_fold0.npz   the reference's shipped NPInter2 inputs for project 1223_1 / fold 0 in
@@ -33,7 +33,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from oracle import refdata, khop, ref_import  # noqa: E402
 
-REF = ref_import.REF_ROOT
+REF = ref_import.require_reference()
 OUT = os.path.join(ROOT, "tests", "golden")
 
 

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
-"""Golden vectors for the node2vec stage from the REFERENCE'S OWN code (build container only):
-imports /root/reference/node2vec-master/src/node2vec.py (the only patch: `np.int = int`, an alias
+"""Golden vectors for the node2vec stage from the REFERENCE'S OWN code (needs the reference tree, oracle/ref_import.py):
+imports <reference>/node2vec-master/src/node2vec.py (the only patch: `np.int = int`, an alias
 numpy >= 1.24 removed), builds the graph like main.py:read_graph (:63-76) and stores the alias tables
 (J, q) of preprocess_transition_probs for
   * a small NON-bipartite graph with triangles (all three branches of get_alias_edge), p = 0.5, q = 2,
@@ -15,8 +15,9 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+from oracle import ref_import                            # noqa: E402
 np.int = int                                             # noqa: removed alias the reference still uses (node2vec.py:114)
-sys.path.insert(0, "/root/reference/node2vec-master/src")
+sys.path.insert(0, os.path.join(ref_import.require_reference(), "node2vec-master", "src"))
 import networkx as nx                                    # noqa: E402
 import node2vec as ref                                   # noqa: E402
 

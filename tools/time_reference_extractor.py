@@ -2,7 +2,7 @@
 """Time the REFERENCE'S OWN CPython extractor (src/classes.py:652-733, imported under a torch_geometric
 stub by oracle/ref_import.py) and the oracle's C restatement on one host core, on the shipped NPInter2
 project 1223_1 / fold 0 (SURVEY 8d: "also time the reference's own CPython extractor ... for the
-extraction-only comparison").  Container only (needs /root/reference); writes profiles/ref_extractor_cpu.json.
+extraction-only comparison").  Needs the reference tree (oracle/ref_import.py: REF_ROOT); writes profiles/ref_extractor_cpu.json.
 
     python tools/time_reference_extractor.py [n_pairs]
 """
@@ -18,7 +18,7 @@ sys.path.insert(0, ROOT)
 from oracle import khop, khop_cwrap, refdata, ref_import  # noqa: E402
 
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 2000
-ds, keys, table = refdata.load_project(ref_import.REF_ROOT, "1223_1", "NPInter2", 0)
+ds, keys, table = refdata.load_project(ref_import.require_reference(), "1223_1", "NPInter2", 0)
 cannot = keys["set_interactionKey_test"] + keys["set_negativeInteractionKey_test"]
 pool = keys["set_interactionKey_train"] + keys["set_negativeInteractionKey_train"]
 rng = np.random.default_rng(20211223)

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
-"""Times the REFERENCE'S OWN node2vec stage (build container only; imports
-/root/reference/node2vec-master/src/node2vec.py with the one patch `np.int = int`) on the real NPInter2
+"""Times the REFERENCE'S OWN node2vec stage (needs the reference tree, oracle/ref_import.py; imports
+<reference>/node2vec-master/src/node2vec.py with the one patch `np.int = int`) on the real NPInter2
 fold-0 training graph with main.py's defaults (p = q = 1, walk length 80): preprocess_transition_probs
 (all alias tables) and ONE pass of simulate_walks (the reference runs ten).  gensim is absent from this
 image, so Word2Vec itself cannot be timed.  Writes profiles/ref_node2vec_cpu.json."""
@@ -15,8 +15,9 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+from oracle import ref_import                            # noqa: E402
 np.int = int                                             # noqa
-sys.path.insert(0, "/root/reference/node2vec-master/src")
+sys.path.insert(0, os.path.join(ref_import.require_reference(), "node2vec-master", "src"))
 import networkx as nx                                    # noqa: E402
 import node2vec as ref                                   # noqa: E402
 
