@@ -533,6 +533,29 @@ int npi_scalar_axpy(float* acc, const float* x, float a, npi_stream_t stream);
 int npi_confusion_counts(const float* logp, const int32_t* y, int32_t B, float threshold,
                          int64_t* counts, npi_stream_t stream);
 
+/* Ranking metrics of n scored pairs (csrc/rank.cu): the threshold-free evaluation next to the confusion matrix of
+ * src/methods.py:87-127 -- the ROC AUC and PR summaries the reference's src/compare_withKmer_noKmer.py:39-74,213-368
+ * computes with sklearn from saved checkpoints.  The semantics are sklearn's (_binary_clf_curve, roc_curve,
+ * roc_auc_score, average_precision_score, precision_recall_curve, auc):
+ *  - the distinct scores in descending order are the thresholds r = 0 .. n_thresholds-1; -0.0 and +0.0 are one
+ *    threshold, +-inf are ordinary scores.  A NaN score sets status bit 0, a label other than 0 or 1 sets bit 1 (the
+ *    other outputs are then meaningless).
+ *  - tps[r] / fps[r] = labels 1 / labels 0 with score >= threshold r (cumulative): thresholds, fps / n_neg, tps / n_pos
+ *    equal roc_curve(y, s, drop_intermediate=False) without its leading inf point.
+ *  - twice_u = sum_r (fps[r] - fps[r-1]) * (tps[r] + tps[r-1]), tps[-1] = fps[-1] = 0: exact, twice the Mann-Whitney U
+ *    with ties counted one half; ROC AUC = twice_u / (2 n_pos n_neg).  twice_u < n^2 / 2 fits int64.
+ *  - areas[0] = average precision = sum_r (tps[r] - tps[r-1]) * tps[r] / (tps[r] + fps[r]) / n_pos (fp64).
+ *  - areas[1] = trapezoidal area under precision_recall_curve's points, its end point (recall 0, precision 1)
+ *    included: auc(recall, precision).
+ * summary (int64[4]) = {n_pos, n_neg, n_thresholds, twice_u}.  thresholds / tps / fps (nullable each) receive the curve
+ * in their first n_thresholds entries (n entries each).  1 <= n < 2^31.  Every output is bit-identical on reruns and
+ * under any permutation of the input (only run ends of the sorted scores are read; no float atomics).  17 launches, no
+ * host synchronisation; the workspace needs no initialisation. */
+int64_t npi_rank_workspace_bytes(int64_t n_max);
+int npi_rank_curve(const float* scores, const int32_t* labels, int64_t n, int64_t* summary, double* areas,
+                   float* thresholds, int32_t* tps, int32_t* fps, int32_t* status,
+                   void* workspace, int64_t workspace_bytes, npi_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------
  * node2vec on the GPU (the stage that produces the embedding columns of the feature table).
  * Replaces node2vec-master/src/node2vec.py and main.py:78-92 of the reference over a CSR with

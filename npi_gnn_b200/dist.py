@@ -57,6 +57,19 @@ def gather_rows(vec, device):
     return torch.stack(out).cpu()
 
 
+def gather_shards(t, total):
+    """The contiguous shards of a ``total``-entry 1-D device tensor (rank r holds entries [r*per, (r+1)*per) of it,
+    per = ceil(total / world), trailing shards short or empty) put back together in order on every rank: each shard
+    is padded to ``per`` entries for one all_gather_into_tensor and the padding is cut away."""
+    world = dist.get_world_size()
+    per = (total + world - 1) // world
+    buf = torch.zeros(per, dtype=t.dtype, device=t.device)
+    buf[:t.numel()].copy_(t)
+    out = torch.empty(per * world, dtype=t.dtype, device=t.device)
+    dist.all_gather_into_tensor(out, buf)
+    return out[:total]
+
+
 def sum_over_ranks(value, device):
     t = torch.tensor([float(value)], dtype=torch.float64, device=device)
     if dist.is_initialized():

@@ -476,6 +476,22 @@ def confusion_counts(logp, y, B, threshold, counts):
     L.call("npi_confusion_counts", L.ptr(logp), L.ptr(y), _i32(B), _f32(threshold), L.ptr(counts), _s())
 
 
+def rank_workspace_bytes(n_max):
+    return L.query("npi_rank_workspace_bytes", _i64(n_max))
+
+
+def rank_curve(scores, labels, summary, areas, status, ws, thresholds=None, tps=None, fps=None):
+    """ROC / PR curve and areas of float32 ``scores`` against int32 ``labels`` (include/npi.h npi_rank_curve):
+    summary int64[4] = {n_pos, n_neg, n_thresholds, twice_u}, areas float64[2] = {AP, trapezoidal PR AUC},
+    status int32[1]; the optional curve arrays take n entries each."""
+    n = scores.numel()
+    if labels.numel() != n or scores.dtype != torch.float32 or labels.dtype != torch.int32 \
+            or not (scores.is_contiguous() and labels.is_contiguous()):
+        raise L.NPIError("rank_curve: contiguous float32 scores and int32 labels of equal length expected")
+    L.call("npi_rank_curve", L.ptr(scores), L.ptr(labels), _i64(n), L.ptr(summary), L.ptr(areas), L.ptr(thresholds),
+           L.ptr(tps), L.ptr(fps), L.ptr(status), L.ptr(ws), _i64(ws.numel() * ws.element_size()), _s())
+
+
 # ----------------------------------------------------------------------------- operator-API helpers
 def filter_edges_coo(edge_index, new_id, out, count_dev):
     E = edge_index.shape[1]

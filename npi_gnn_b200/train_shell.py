@@ -19,6 +19,9 @@ module-level route instead: ``Net_1`` + ``torch.optim.Adam`` exactly as the refe
 Differences by design: paths are joined with os.path (the reference hard-codes ``.\\\\data\\\\dataset``
 Windows separators, :64-65); ``--seed`` (not in the reference) makes the two ``dataset.shuffle()``
 calls (:76-77), the parameter initialisation and dropout reproducible; ``--gpus`` is implied by torchrun.
+``--rankMetrics 1`` (not in the reference) adds one line after every testing-dataset metric line:
+'<same prefix>, AUROC: x.xxxxx, AP: x.xxxxx, PR-AUC(trapz): x.xxxxx' -- the ROC AUC and PR summaries of
+src/compare_withKmer_noKmer.py, from the same sweep (``Scorer.rank_metrics``); with 0 the artefacts are unchanged.
 """
 from __future__ import annotations
 
@@ -29,14 +32,14 @@ import time
 import torch
 
 from . import _lib as L
-from .trainer import Scorer, Trainer, metrics
+from .trainer import Scorer, Trainer, metrics, rank_metrics
 
 EVAL_EVERY = 5          # src/train_with_twoDataset.PY:163
 GAMMA = 0.95            # ExponentialLR(gamma=0.95) stepped only when the loss rose (:135,158-159)
 
 
 def build_parser():
-    """The reference's flags with its defaults (src/train_with_twoDataset.PY:26-43) + --seed/--dataRoot/--resultRoot."""
+    """The reference's flags with its defaults (src/train_with_twoDataset.PY:26-43) + --seed/--dataRoot/--resultRoot/--rankMetrics."""
     p = argparse.ArgumentParser(description="train Net_1 on two enclosing-subgraph datasets")
     p.add_argument("--trainingName", help="the name of this training")
     p.add_argument("--trainingDatasetName", help="the name of this object")
@@ -53,6 +56,8 @@ def build_parser():
     p.add_argument("--seed", default=None, type=int, help="(extension) seed for shuffle / init / dropout")
     p.add_argument("--dataRoot", default=os.path.join("data", "dataset"), help="(extension) where the datasets live")
     p.add_argument("--resultRoot", default="result", help="(extension) where logs and checkpoints go")
+    p.add_argument("--rankMetrics", default=0, type=int,
+                   help="(extension) 1: log AUROC, AP and trapezoidal PR AUC after every testing-dataset metric line")
     return p
 
 
@@ -63,6 +68,11 @@ def parse_args(argv=None):
 def metric_line(prefix, m):
     """'<prefix>, Accuracy: ..., MCC: ...' with the reference's 5-decimal formatting (:168,172,199,203)."""
     return "{}, Accuracy: {:.5f}, Precision: {:.5f}, Sensitivity: {:.5f}, Specificity: {:.5f}, MCC: {:.5f}".format(prefix, *m)
+
+
+def rank_line(prefix, r):
+    """'<prefix>, AUROC: ..., AP: ..., PR-AUC(trapz): ...' (--rankMetrics 1) from a ``rank_metrics`` dict."""
+    return "{}, AUROC: {:.5f}, AP: {:.5f}, PR-AUC(trapz): {:.5f}".format(prefix, r["auroc"], r["ap"], r["pr_auc_trapz"])
 
 
 def should_evaluate(epoch1, num_epochs):
@@ -141,11 +151,19 @@ class _FusedBackend:
     def set_lr(self, lr):
         self.tr.set_lr(lr)
 
-    def evaluate(self, which):
+    def _scorer(self, which):
         ds = self.train_ds if which == "train" else self.test_ds
         if which not in self._scorers:
             self._scorers[which] = Scorer(ds.pairset, self.tr.params, batch_size=self.B, index=ds._index)
-        return metrics(*self._scorers[which].confusion())
+        return self._scorers[which]
+
+    def evaluate(self, which):
+        return metrics(*self._scorer(which).confusion())
+
+    def evaluate_ranked(self, which):
+        """(metrics, rank_metrics dict) from one sweep of the dataset."""
+        r = self._scorer(which).rank_metrics()
+        return metrics(*r["confusion"]), r
 
     def state_dict(self):
         return {k: v.cpu() for k, v in self.tr.params.state_dict().items()}
@@ -182,16 +200,24 @@ class _ModuleBackend:
             g["lr"] = lr
 
     def evaluate(self, which):
+        return self.evaluate_ranked(which, rank=False)[0]
+
+    def evaluate_ranked(self, which, rank=True):
         from . import ops
         self.model.eval()
         counts = torch.zeros(4, dtype=torch.int64, device="cuda")
+        scores, labels = [], []
         with torch.no_grad():
             for data in self.loaders[which]:
                 data = data.to("cuda")
                 logp = self.model(data).contiguous()
                 ops.confusion_counts(logp, data.y.to(torch.int32), data.num_graphs, -1.0, counts)
+                if rank:
+                    scores.append(torch.exp(logp[:, 1]))
+                    labels.append(data.y.to(torch.int32))
         TP, FN, TN, FP = [int(v) for v in counts.cpu()]
-        return metrics(TP, FN, TN, FP)
+        r = rank_metrics(torch.cat(scores), torch.cat(labels)) if rank else None
+        return metrics(TP, FN, TN, FP), r
 
     def state_dict(self):
         return {k: v.detach().cpu() for k, v in self.model.state_dict().items()}
@@ -234,6 +260,17 @@ def run(args, train_dataset=None, test_dataset=None, echo=True):
     seed = args.seed if args.seed is not None else int(torch.initial_seed() & 0x7FFFFFFF)
     be = (_FusedBackend if fused else _ModuleBackend)(train_dataset, test_dataset, args, seed)
 
+    def evaluate_test(prefix):
+        """The testing-dataset metric line (+ the rank line under --rankMetrics 1, same sweep); returns the metrics."""
+        if not args.rankMetrics:
+            m = be.evaluate("test")
+            log.line(metric_line(prefix, m))
+            return m
+        m, r = be.evaluate_ranked("test")
+        log.line(metric_line(prefix, m))
+        log.line(rank_line(prefix, r))
+        return m
+
     sched, best, losses = LrOnLossIncrease(lr0), BestByMcc(), []
     for epoch in range(num_epochs):
         loss = be.train_epoch()
@@ -243,14 +280,12 @@ def run(args, train_dataset=None, test_dataset=None, echo=True):
         if should_evaluate(epoch + 1, num_epochs):
             m = be.evaluate("train")
             log.line(metric_line("Epoch: {:03d}, training dataset".format(epoch + 1), m))
-            m = be.evaluate("test")
-            log.line(metric_line("Epoch: {:03d}, testing dataset".format(epoch + 1), m))
+            m = evaluate_test("Epoch: {:03d}, testing dataset".format(epoch + 1))
             best.offer(epoch + 1, m)
             torch.save(be.state_dict(), os.path.join(model_dir, str(epoch + 1)))
     m_train = be.evaluate("train")
     log.line(metric_line("result, training dataset", m_train))
-    m_test = be.evaluate("test")
-    log.line(metric_line("result, testing dataset", m_test))
+    m_test = evaluate_test("result, testing dataset")
     best.offer(num_epochs, m_test)
     torch.save(be.state_dict(), os.path.join(model_dir, str(num_epochs)))
     log.f.write("\n")

@@ -390,6 +390,7 @@ class Scorer:
         self.device = g.device
         self.index = None if index is None else np.ascontiguousarray(index, dtype=np.int64)
         P = len(pairset) if self.index is None else len(self.index)
+        self.P, self.world_size = P, int(world_size)
         per = (P + world_size - 1) // world_size
         self.lo, self.hi = min(P, rank * per), min(P, (rank + 1) * per)
         self.B = int(batch_size)
@@ -502,6 +503,31 @@ class Scorer:
             torch.exp(logp[:cnt, 1], out=out[first - self.lo:first - self.lo + cnt])
         return out
 
+    def rank_metrics(self, curve=False):
+        """ROC AUC, average precision and trapezoidal PR AUC (``rank_metrics``) of the probabilities that
+        ``probabilities()`` returns against the pair labels, plus ``confusion`` = (TP, FN, TN, FP) of the argmax rule,
+        all from ONE sweep.  With world_size > 1 every rank's shard is gathered (torch.distributed must be initialised)
+        and every rank computes the same, bit-identical result over all pairs -- the confusion counts included."""
+        from . import dist as D
+        if self.world_size > 1 and not D.dist.is_initialized():
+            raise L.NPIError("Scorer.rank_metrics with world_size > 1 needs an initialised torch.distributed process group")
+        n = self.hi - self.lo
+        scores = torch.empty(n, dtype=torch.float32, device=self.device)
+        labels = torch.empty(n, dtype=torch.int32, device=self.device)
+        counts = torch.zeros(4, dtype=torch.int64, device=self.device)
+        for first, cnt, logp in self.batches():
+            o = first - self.lo
+            torch.exp(logp[:cnt, 1], out=scores[o:o + cnt])
+            labels[o:o + cnt].copy_(self.engine.y_b[:cnt])
+            ops.confusion_counts(logp, self.engine.y_b, cnt, -1.0, counts)
+        if self.world_size > 1:
+            scores = D.gather_shards(scores, self.P)
+            labels = D.gather_shards(labels, self.P)
+            D.allreduce_sum(counts)
+        out = rank_metrics(scores, labels, curve=curve)
+        out["confusion"] = tuple(int(v) for v in counts.cpu())
+        return out
+
 
 def metrics(TP, FN, TN, FP):
     """Accuracy, Precision, Sensitivity, Specificity, MCC exactly as src/methods.py:107-127."""
@@ -513,3 +539,44 @@ def metrics(TP, FN, TN, FP):
     mcc = (TP * TN - FP * FN) / den if den else 0
     spe = TN / (FP + TN) if (FP + TN) else 0
     return acc, pre, sen, spe, mcc
+
+
+def rank_metrics(scores, labels, curve=False):
+    """Threshold-free metrics of CUDA float32 ``scores`` against int32 0/1 ``labels`` in ONE call of npi_rank_curve and
+    one synchronising read: dict(auroc, ap, pr_auc_trapz, n_pos, n_neg, twice_u) -- sklearn's roc_auc_score,
+    average_precision_score and auc(recall, precision) over precision_recall_curve, the metrics of the reference's
+    src/compare_withKmer_noKmer.py.  ``curve=True`` adds the device tensors thresholds (float32), fpr, tpr, precision
+    and recall (float64), one entry per distinct score in descending order.  NaN scores or labels other than 0/1 raise
+    NPIError; a single class raises ValueError (ROC AUC is undefined)."""
+    L.require_cuda(scores, labels)
+    scores, labels = scores.reshape(-1).contiguous(), labels.reshape(-1).contiguous()
+    n = scores.numel()
+    dev = scores.device
+    res = torch.zeros(7, dtype=torch.int64, device=dev)     # summary[4] | areas[2] (fp64) | status (int32)
+    summary, areas, status = res[:4], res[4:6].view(torch.float64), res[6:7].view(torch.int32)[:1]
+    ws = torch.empty(ops.rank_workspace_bytes(max(n, 1)), dtype=torch.uint8, device=dev)
+    thr = tps = fps = None
+    if curve:
+        thr = torch.empty(n, dtype=torch.float32, device=dev)
+        tps = torch.empty(n, dtype=torch.int32, device=dev)
+        fps = torch.empty(n, dtype=torch.int32, device=dev)
+    ops.rank_curve(scores, labels, summary, areas, status, ws, thr, tps, fps)
+    h = res.cpu()
+    st = int(h[6:7].view(torch.int32)[0])
+    if st & 1:
+        raise L.NPIError("rank_metrics: NaN score")
+    if st & 2:
+        raise L.NPIError("rank_metrics: label other than 0 or 1")
+    n_pos, n_neg, T, twice_u = (int(v) for v in h[:4])
+    if n_pos == 0 or n_neg == 0:
+        raise ValueError("Only one class present in the labels: ROC AUC is not defined in that case")
+    a = h[4:6].view(torch.float64)
+    out = dict(auroc=twice_u / (2.0 * n_pos * n_neg), ap=float(a[0]), pr_auc_trapz=float(a[1]),
+               n_pos=n_pos, n_neg=n_neg, twice_u=twice_u)
+    if curve:
+        t, f = tps[:T].double(), fps[:T].double()
+        # divided by device tensors (t[-1] = n_pos, f[-1] = n_neg): a host scalar divisor becomes a multiplication by
+        # its reciprocal, which is not always the correctly rounded quotient sklearn's tps / tps[-1] gives
+        tpr = t / t[-1]
+        out.update(thresholds=thr[:T], fpr=f / f[-1], tpr=tpr, precision=t / (t + f), recall=tpr)
+    return out
