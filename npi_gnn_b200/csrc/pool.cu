@@ -302,7 +302,11 @@ __global__ void __launch_bounds__(H) readout_combine_kernel(const float* part, c
         if (av >= 0 && (a < 0 || mv > m || (mv == m && av < a))) { m = mv; a = av; }
         t += pp[sp * GR_PART + H + c];
     }
-    const float mean = t / (float)(gout[g + 1] - gout[g]);
+    // an empty graph (operator API only: a gap in `batch` or a `size` beyond it) reads 0 for max and mean, as
+    // PyG's scatter does; its argmax stays -1, so no row gets a max gradient
+    const int cnt = gout[g + 1] - gout[g];
+    if (cnt == 0) m = 0.f;
+    const float mean = cnt ? t / (float)cnt : 0.f;
     float* ro = readout + (int64_t)g * 2 * H;
     if (accumulate) { ro[c] += m; ro[H + c] += mean; }
     else { ro[c] = m; ro[H + c] = mean; }

@@ -49,15 +49,27 @@ def _csr_of(edge_index, N, check_symmetric=True):
     return rowptr, col
 
 
-def _graph_ptr_of(batch, N, device, num_graphs=None):
+def _graph_ptr_of(batch, N, device, num_graphs=None, size=None):
     """graph_ptr from a sorted PyG batch vector (one host sync: B = batch.max()+1, like PyG -- skipped when the
-    batch object carries ``num_graphs``, as PyG's ``Batch`` and this package's loaders do)."""
+    batch object carries ``num_graphs``, as PyG's ``Batch`` and this package's loaders do).  The kernels take each
+    graph's rows as one contiguous range, so the same sync also checks that ``batch`` is sorted.  ``size``: number
+    of graphs (PyG's ``size`` argument); graphs with no rows, in a gap of ``batch`` or past its end, are empty."""
     if batch is None:
         return torch.tensor([0, N], dtype=torch.int32, device=device)
     if num_graphs is not None:
         B = int(num_graphs)
+    elif N > 0:
+        top, unsorted = torch.stack([batch.max(), (batch[1:] < batch[:-1]).any().to(batch.dtype)]).tolist()
+        if unsorted:
+            raise L.NPIError("batch must be sorted (the rows of each graph contiguous, graphs in increasing order), "
+                             "as PyG's Batch builds it")
+        B = top + 1
     else:
-        B = int(batch.max().item()) + 1 if N > 0 else 0
+        B = 0
+    if size is not None:
+        if size < B:
+            raise L.NPIError("size=%d is smaller than batch.max()+1 = %d" % (size, B))
+        B = int(size)
     counts = torch.bincount(batch, minlength=B)
     gp = torch.zeros(B + 1, dtype=torch.int32, device=device)
     gp[1:] = torch.cumsum(counts, 0).to(torch.int32)
@@ -254,12 +266,14 @@ class _GlobalPoolFn(torch.autograd.Function):
 
 
 def global_max_pool(x, batch, size=None):
-    gp = _graph_ptr_of(batch, x.shape[0], x.device)
+    """PyG 1.4.2 ``global_max_pool``: [size or batch.max()+1, 128]; an empty graph gives 0.  ``batch`` must be sorted."""
+    gp = _graph_ptr_of(batch, x.shape[0], x.device, size=size)
     return _GlobalPoolFn.apply(x, gp, _i32(batch), True)
 
 
 def global_mean_pool(x, batch, size=None):
-    gp = _graph_ptr_of(batch, x.shape[0], x.device)
+    """PyG 1.4.2 ``global_mean_pool``: [size or batch.max()+1, 128]; an empty graph gives 0.  ``batch`` must be sorted."""
+    gp = _graph_ptr_of(batch, x.shape[0], x.device, size=size)
     return _GlobalPoolFn.apply(x, gp, _i32(batch), False)
 
 

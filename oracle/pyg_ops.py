@@ -93,11 +93,14 @@ def topk_pooling(x, edge_index, batch, weight, ratio=0.5, forced_perm=None):
 
 
 def global_max_pool(x, batch, num_graphs=None):
+    """Segment max; a graph with no rows gives 0 (PyG's scatter_ replaces the empty max fill with 0)."""
     if num_graphs is None:
         num_graphs = int(batch.max()) + 1
     out = torch.full((num_graphs, x.shape[1]), float("-inf"), dtype=x.dtype)
     idx = batch.view(-1, 1).expand(-1, x.shape[1])
-    return out.scatter_reduce(0, idx, x, reduce="amax", include_self=True)
+    out = out.scatter_reduce(0, idx, x, reduce="amax", include_self=True)
+    empty = torch.bincount(batch, minlength=num_graphs) == 0
+    return torch.where(empty.view(-1, 1), torch.zeros_like(out), out)
 
 
 def global_mean_pool(x, batch, num_graphs=None):
