@@ -218,20 +218,26 @@ int npi_gemm_tn_tc(const float* A, int32_t lda, int32_t K, const float* D, const
 /* h_i = act((sum_{j in row(i) U {i}} y_j)/(deg_i+1) + bias); y_j = Y[j] or, for the virtual input
  * layer (gid/dist non-NULL), Y[gid[j]] + dist[j]*w0 with Y the projected feature table and w0 the
  * label row of the weight.  Optional pooling score as in npi_sage_fwd. */
-/* Rows of a CSR with more than 128 entries ("hub" rows: a protein that interacts with most of a
- * subgraph) are cut into segments of 128 entries, one warp each, so that no single warp walks a
+/* Rows of a CSR with more than 16 entries ("hub" rows: a protein that interacts with most of a
+ * subgraph) are cut into segments of 32 entries, one warp each, so that no single warp walks a
  * 1000-entry row.  The segments are listed ONCE per CSR, when the CSR is produced (next to the
  * extraction / filter_adj), into hub_queue (counters, segment list, per-row arrival counters and
  * the buffer of partial sums; npi_hub_rows_bytes(e_max) bytes for a CSR of at most e_max entries);
  * the forward and the backward aggregation of that CSR both consume the list and leave the queue
- * ready for the next launch -- one launch at a time per queue. */
+ * ready for the next launch -- one launch at a time per queue.
+ * Initialisation: the queue needs no zeroed memory.  npi_hub_rows_build (and npi_filter_adj after
+ * npi_hub_rows_reset) writes the header, the segment list and every arrival counter a launch reads;
+ * every launch rewinds the counters it used.  (16 and 32 are the shipped NPI_AG_HUB /
+ * NPI_AG_SEG of csrc/hub.cuh.) */
 int64_t npi_hub_rows_bytes(int64_t e_max);
-/* row_order (nullable, 16 bytes per row, n_host rows): the rows with at most 128 entries BINNED BY
+/* row_order (nullable, 16 bytes per row, n_host rows): the rows with at most 16 entries BINNED BY
  * LENGTH CLASS -- {row, first entry, end, self payload} with self payload = gid[row] | dist[row] << 29
  * when gid/dist are given (virtual input layer), else the row id.  The 8-lane groups of a warp work in
  * lock step, so the pipelined aggregation kernels take four rows of the same class at a time; the
- * class totals live in the queue header.  The order inside a class is timing dependent and has no
- * influence on any result (rows are independent). */
+ * class totals live in the queue header (int32 hdr[4 + c] for classes c = 0..7: rows of 1, 2-3, 4-5,
+ * 6-7, 8-11, 12-16 entries, whole-warp rows, hub rows; a row of 0 entries is class 0).  Class 6 holds
+ * the rows of 17..NPI_AG_HUB entries and is empty at the shipped constants.  The order inside a class
+ * is timing dependent and has no influence on any result (rows are independent). */
 /* keep (nullable): only rows with keep[i] == i are listed -- the representative rows of npi_ctx_build: the
  * aggregation kernels then evaluate one row per layer-1 context and leave every other row of h/z/s untouched. */
 int npi_hub_rows_build(const int32_t* rowptr, const int32_t* n_dev, int32_t n_host, int64_t e_max,

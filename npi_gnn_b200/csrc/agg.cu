@@ -503,8 +503,8 @@ __global__ void __launch_bounds__(AG_THREADS, AG_PIPE_CTAS) aggregate_fwd_pipe_k
     const int n_long = hdr[HQ_CLS + 6];
     const int4* __restrict__ rows = a.rows;
 
-    // whole-warp rows (17..128 entries) first, one per warp: the warps that get one start their share
-    // of the short rows a little later instead of finishing the kernel alone
+    // whole-warp rows (AG_SHORT+1 .. AG_HUB entries; none at the shipped AG_HUB = AG_SHORT = 16) first, one per
+    // warp: the warps that get one start their share of the short rows a little later instead of finishing alone
     for (int64_t idx = n_short + warp0; idx < (int64_t)n_short + n_long; idx += nwarps) {
         const int4 R = rows[idx];
         int dsl = 0;
@@ -722,7 +722,7 @@ __global__ void __launch_bounds__(AG_THREADS, AG_PIPE_CTAS) aggregate_bwd_pipe_k
     const int n_long = hdr[HQ_CLS + 6];
     const int4* __restrict__ rows = a.rows;
 
-    for (int64_t idx = n_short + warp0; idx < (int64_t)n_short + n_long; idx += nwarps) {      // whole-warp rows
+    for (int64_t idx = n_short + warp0; idx < (int64_t)n_short + n_long; idx += nwarps) {      // whole-warp rows (class 6)
         const int4 R = rows[idx];
         const int ids = a.no_self ? -1 : (a.new_id ? a.new_id[R.x] : R.x);
         float4 accl = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -1130,6 +1130,8 @@ extern "C" int npi_sage_aggregate_fwd(const float* Y, const int32_t* gid, const 
     NPI_REQUIRE((gid == nullptr) == (dist == nullptr), "sage_aggregate_fwd: gid and dist come together");
     NPI_REQUIRE(!(pipelined && gid) || packed, "sage_aggregate_fwd: the pipelined virtual layer needs the packed entries");
     NPI_REQUIRE(!pipelined || row_order, "sage_aggregate_fwd: the pipelined kernel needs the binned row order of npi_hub_rows_build");
+    NPI_REQUIRE(((uintptr_t)row_order & 15) == 0 && ((uintptr_t)packed & 3) == 0,
+                "sage_aggregate_fwd: row_order must be 16-byte and packed 4-byte aligned");
     cudaStream_t st = (cudaStream_t)stream;
     AggFwdArgs a{Y, gid, dist, w0, rowptr, col, n_dev, n_host, bias, relu, pool_w, h, z, s, hub_queue, packed, (const int4*)row_order};
     if (pipelined) {
@@ -1150,6 +1152,8 @@ extern "C" int npi_sage_aggregate_bwd(const float* dpre, const int32_t* new_id, 
                                       int32_t* hub_queue, const void* packed, const void* row_order, npi_stream_t stream) {
     NPI_REQUIRE(dpre && rowptr && col && dxa && hub_queue, "sage_aggregate_bwd: null argument");
     NPI_REQUIRE(!packed || row_order, "sage_aggregate_bwd: the pipelined kernel needs the binned row order of npi_hub_rows_build");
+    NPI_REQUIRE(((uintptr_t)row_order & 15) == 0 && ((uintptr_t)packed & 7) == 0,
+                "sage_aggregate_bwd: row_order must be 16-byte and packed 8-byte aligned");
     AggBwdArgs a{dpre, new_id, rowptr, col, n_dev, n_host, dxa, hub_queue, (const int2*)packed, (const int4*)row_order, 0};
     if (packed) NPI_CHECK_CUDA(launch_dep(aggregate_bwd_pipe_kernel, agg_pipe_grid(n_host), AG_THREADS, 0, (cudaStream_t)stream, a));
     else aggregate_bwd_kernel<<<agg_grid(n_host), AG_THREADS, 0, (cudaStream_t)stream>>>(a);
@@ -1160,6 +1164,8 @@ extern "C" int npi_sage_aggregate_bwd(const float* dpre, const int32_t* new_id, 
 extern "C" int npi_csr_gather_sum(const float* src, const int32_t* rowptr, const void* packed, int32_t n_rows, float* out,
                                   int32_t* hub_queue, const void* row_order, npi_stream_t stream) {
     NPI_REQUIRE(src && rowptr && packed && out && hub_queue && row_order && n_rows > 0, "csr_gather_sum: bad argument");
+    NPI_REQUIRE(((uintptr_t)row_order & 15) == 0 && ((uintptr_t)packed & 7) == 0,
+                "csr_gather_sum: row_order must be 16-byte and packed 8-byte aligned");
     AggBwdArgs a{src, nullptr, rowptr, nullptr, nullptr, n_rows, out, hub_queue, (const int2*)packed, (const int4*)row_order, 1};
     // the per-context backward of conv1 uses it on CSRs whose work sits in a few long rows (a node of the graph occurs
     // in ~100 contexts of a batch) as well as on the class CSR: the grid is the full machine whatever n_rows is

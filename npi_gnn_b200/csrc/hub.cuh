@@ -23,7 +23,8 @@ constexpr int AG_SEG = NPI_AG_SEG;   // entries per segment of a hub row (one wa
 //                     [4+c] rows of length class c (c = 0..7, row_class below), [16+c] fill cursors
 //   int32 seg_row[cap], seg_base[cap]   row of segment s / first segment of that row (a row's
 //                                       segments are consecutive: segment s is part s - seg_base[s])
-//   int32 arrive[cap]                   arrive[base]: parts of the row finished (rewound by the last)
+//   int32 arrive[cap]                   arrive[base]: parts of the row finished, arrive[base+1+g]: segments of group g
+//                                       finished (two-level combine); zeroed by hub_list_row, rewound by the last
 //   int32 dsum[cap]                     integer label sum of a part (virtual input layer)
 //   float part[cap][128]                partial sums
 // sum_rows ceil(L/AG_SEG) <= E/AG_SEG + #hub rows <= E/AG_SEG + E/(AG_HUB+1)  (= hub_cap).
@@ -46,13 +47,17 @@ __host__ __device__ inline HubQueue hub_view(int32_t* buf, int cap) {
 
 // Length class of a row: the 8-lane groups of a warp work in lock step, two elements (entries, then
 // the row itself) per round, so a warp should hold four rows that need the same number of rounds.
-// Classes 0..5: 1, 2, 3, 4, 5-6, 7-9 rounds (short rows); 6: whole-warp rows; 7: hub rows (segments).
+// Classes 0..5: 1, 2, 3, 4, 5-6, 7-9 rounds (short rows); 6: whole-warp rows (AG_SHORT+1 .. AG_HUB entries: empty
+// at the shipped AG_HUB = AG_SHORT = 16, reachable in a -DNPI_AG_HUB build); 7: hub rows (segments).
 __host__ __device__ inline int row_class(int len) {
     return len <= 1 ? 0 : len <= 3 ? 1 : len <= 5 ? 2 : len <= 7 ? 3 : len <= 11 ? 4 : len <= AG_SHORT ? 5 : len <= AG_HUB ? 6 : 7;
 }
 
 // one row of `len` entries joins the queue: class histogram (the caller's shared-memory hist[N_CLS]) and, for a hub row,
-// its consecutive segment slots (slot order is timing dependent and irrelevant: rows are independent)
+// its consecutive segment slots (slot order is timing dependent and irrelevant: rows are independent).  Every arrival
+// counter a launch may use is zeroed here, so the queue works whatever memory it was allocated in: arrive[base] counts
+// the row, and a row of more than 2*HUB_GRP segments also counts its groups in arrive[base + 1 + g] (the two-level
+// combine of agg.cu).
 __device__ __forceinline__ void hub_list_row(const HubQueue& hq, int cap, int* hist, int row, int len) {
     atomicAdd(&hist[row_class(len)], 1);
     if (len > AG_HUB) {
@@ -60,7 +65,8 @@ __device__ __forceinline__ void hub_list_row(const HubQueue& hq, int cap, int* h
         const int base = atomicAdd(&hq.hdr[0], nseg);
         if (base + nseg <= cap) {
             for (int k = 0; k < nseg; ++k) { hq.seg_row[base + k] = row; hq.seg_base[base + k] = base; }
-            hq.arrive[base] = 0;
+            const int ncnt = nseg > 2 * HUB_GRP ? 1 + (nseg + HUB_GRP - 1) / HUB_GRP : 1;
+            for (int k = 0; k < ncnt; ++k) hq.arrive[base + k] = 0;
         }
     }
 }

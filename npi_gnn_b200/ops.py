@@ -293,8 +293,10 @@ def csr_gather_sum(src, rowptr, packed, n_rows, out, hubq, row_order):
 
 def hub_rows_build(rowptr, n_dev, n_host, e_max, hubq, gid=None, dist=None, row_order=None, keep=None):
     """List the hub-row segments of a CSR of at most e_max entries into ``hubq`` (uint8 buffer of
-    hub_rows_bytes(e_max)); with ``row_order`` (int32 [>= n_host, 4]) also the rows of at most 128
-    entries binned by length class (what the pipelined aggregation kernels walk)."""
+    hub_rows_bytes(e_max), any contents: the header and the counters of every listed segment are
+    written here); with ``row_order`` (int32 [>= n_host, 4], 16-byte aligned) also the rows of at most
+    16 entries binned by length class (what the pipelined aggregation kernels walk).  Hub rows have
+    more than 16 entries and are cut into segments of 32."""
     L.call("npi_hub_rows_build", L.ptr(rowptr), L.ptr(n_dev), _i32(n_host), _i64(e_max), L.ptr(hubq),
            _i64(hubq.numel() * hubq.element_size()), L.ptr(gid), L.ptr(dist), L.ptr(row_order), L.ptr(keep), _s(),
            count_as=None if row_order is None else "npi_hub_rows_build/order")

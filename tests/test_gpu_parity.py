@@ -513,7 +513,9 @@ def test_pipelined_aggregation_bit_identical_to_plain(npi, h, B, monkeypatch):
     """The software-pipelined aggregation kernels over the packed entry streams (what the engine
     launches) sum in the order of the plain dependent-chain kernels: log-probabilities, every
     intermediate activation, the loss and all gradients must be BIT-identical between the two
-    (short rows, whole-warp rows and hub segments all occur at h >= 2 on NPInter2)."""
+    (short rows and hub segments both occur at h >= 2 on NPInter2; the whole-warp tier is empty at
+    the shipped 16-entry hub threshold).  Neither kernel is checked against a reference here:
+    tests/test_gpu_aggregation.py does that."""
     from npi_gnn_b200.engine import FlatParams
     from npi_gnn_b200.graph import PairSet
     d, og, omask, g = npi
@@ -541,7 +543,7 @@ def test_pipelined_aggregation_bit_identical_to_plain(npi, h, B, monkeypatch):
     assert a["N"] == b["N"] and a["E"] == b["E"]
     if h >= 2:
         deg = (eng.rowptr[0][1:a["N"][0] + 1] - eng.rowptr[0][:a["N"][0]])
-        assert int(deg.max()) > 128 and int(((deg > 16) & (deg <= 128)).sum()) > 0      # all three tiers exercised
+        assert int(deg.max()) > 128 and int(((deg > 16) & (deg <= 128)).sum()) > 0      # hub rows of 1-4 and of > 4 segments
     for l in range(3):
         assert torch.equal(a["h"][l], b["h"][l]), "forward aggregation layer %d" % (l + 1)
         assert torch.equal(a["s"][l], b["s"][l])
