@@ -562,6 +562,24 @@ int npi_rank_curve(const float* scores, const int32_t* labels, int64_t n, int64_
                    float* thresholds, int32_t* tps, int32_t* fps, int32_t* status,
                    void* workspace, int64_t workspace_bytes, npi_stream_t stream);
 
+/* Top-k items of every group by score (csrc/topk.cu): the per-node ranking of a scoring sweep that the reference's
+ * case studies (src/case_study_negativeSample.py, src/case_study.py) read -- for an RNA its most likely protein
+ * partners, for a protein its most likely RNAs.
+ *  - item i (0 <= i < n) has score scores[i] and group group[i], 0 <= group[i] < num_groups.
+ *  - for every group g the first out_count[g] = min(k, |g|) entries of row g of out_pos / out_score ([num_groups, k],
+ *    row-major) are the items of g ranked by descending score; ties break by ascending i.  -0.0 and +0.0 are one value
+ *    (their order comes from i, not from the sign); +-inf are ordinary scores.  out_score is the input value, copied
+ *    bit for bit.  Entries past out_count[g] are out_pos = -1 and out_score = NaN; an empty group has out_count 0.
+ *  - status (int32[1]): bit 0 = a NaN score, bit 1 = a group id out of range; when either is set the other outputs are
+ *    meaningless.
+ * 1 <= k <= 1024, 1 <= n < 2^31, 1 <= num_groups < 2^24.  Outputs are bit-identical on reruns (no float atomics).
+ * 3 + 3 * npi_sort_passes(ceil(log2 num_groups)) launches (6 up to 512 groups, 9 up to 262,144, else 12), no host
+ * synchronisation, capturable in a CUDA graph; the workspace needs no initialisation. */
+int64_t npi_group_topk_workspace_bytes(int64_t n_max, int32_t num_groups);
+int npi_group_topk(const float* scores, const int32_t* group, int64_t n, int32_t num_groups, int32_t k,
+                   int32_t* out_pos, float* out_score, int32_t* out_count, int32_t* status,
+                   void* workspace, int64_t workspace_bytes, npi_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------
  * node2vec on the GPU (the stage that produces the embedding columns of the feature table).
  * Replaces node2vec-master/src/node2vec.py and main.py:78-92 of the reference over a CSR with

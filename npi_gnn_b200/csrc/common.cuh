@@ -150,6 +150,15 @@ __device__ __forceinline__ int block_excl_scan(int v, int* sh, int* total) {
     return inc - v + sh[w];
 }
 
+// Orderable key of a score for the ranking entry points (rank.cu, topk.cu): ascending key = descending score, -0.0 and
+// +0.0 one key, +-inf ordinary scores.
+__device__ __forceinline__ uint32_t rank_key(float s) {
+    uint32_t u = __float_as_uint(s);
+    if (s == 0.0f) u = 0u;                                   // -0.0 and +0.0 are one threshold
+    u = (u & 0x80000000u) ? ~u : (u | 0x80000000u);          // order-preserving map to uint32
+    return ~u;                                               // ascending key = descending score
+}
+
 __device__ __forceinline__ float4 ldg4(const float* p) { return __ldg(reinterpret_cast<const float4*>(p)); }
 __device__ __forceinline__ void st4(float* p, float4 v) { *reinterpret_cast<float4*>(p) = v; }
 __device__ __forceinline__ float4 add4(float4 a, float4 b) { return make_float4(a.x + b.x, a.y + b.y, a.z + b.z, a.w + b.w); }

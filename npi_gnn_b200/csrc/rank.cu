@@ -26,13 +26,6 @@ constexpr int RA_THREADS = 256;
 constexpr int RA_MAX_CTAS = 1024;                   // area partials (one per CTA), summed by the last CTA
 constexpr int64_t RK_ALIGN = 256;
 
-__device__ __forceinline__ uint32_t rank_key(float s) {
-    uint32_t u = __float_as_uint(s);
-    if (s == 0.0f) u = 0u;                                   // -0.0 and +0.0 are one threshold
-    u = (u & 0x80000000u) ? ~u : (u | 0x80000000u);          // order-preserving map to uint32
-    return ~u;                                               // ascending key = descending score
-}
-
 __device__ __forceinline__ float rank_score(uint32_t key) {
     const uint32_t o = ~key;
     return __uint_as_float((o & 0x80000000u) ? (o & 0x7fffffffu) : ~o);

@@ -116,6 +116,15 @@ class BipartiteGraph:
         hit = (ks[pos] == q) if len(ks) else np.zeros(len(q), dtype=bool)
         return np.where(hit, order[pos], -1).astype(np.int32)
 
+    def candidate_pairs(self):
+        """Every (rna, protein) pair that is not an edge, RNA-major in serial order: int32 [R * P - E, 2].  Negatives are
+        edges too (SURVEY 0.4), so these are the pairs that are neither a known interaction nor a sampled negative --
+        the list a case study scores.  Host only."""
+        r = np.nonzero(self.is_rna_h)[0].astype(np.int32)
+        p = np.nonzero(self.is_rna_h == 0)[0].astype(np.int32)
+        allp = np.stack([np.repeat(r, len(p)), np.tile(p, len(r))], 1)
+        return allp[self.edge_ids(allp) < 0]
+
     def _fold_mask(self):
         if len(self.col_h):
             ops.csr_fold_mask(self.col, self.eid, self.mask, self.colm)

@@ -494,6 +494,26 @@ def rank_curve(scores, labels, summary, areas, status, ws, thresholds=None, tps=
            L.ptr(tps), L.ptr(fps), L.ptr(status), L.ptr(ws), _i64(ws.numel() * ws.element_size()), _s())
 
 
+def group_topk_workspace_bytes(n_max, num_groups):
+    return L.query("npi_group_topk_workspace_bytes", _i64(n_max), _i32(num_groups))
+
+
+def group_topk(scores, group, num_groups, k, out_pos, out_score, out_count, status, ws):
+    """Top-``k`` items of every group of float32 ``scores`` / int32 ``group`` ids, by descending score with ties by
+    ascending position (include/npi.h npi_group_topk): out_pos int32 / out_score float32 [num_groups, k] (-1 / NaN past
+    the group's count), out_count int32[num_groups], status int32[1] (bit 0 NaN score, bit 1 group id out of range)."""
+    n = scores.numel()
+    if group.numel() != n or scores.dtype != torch.float32 or group.dtype != torch.int32 \
+            or not (scores.is_contiguous() and group.is_contiguous()):
+        raise L.NPIError("group_topk: contiguous float32 scores and int32 group ids of equal length expected")
+    if out_pos.numel() < num_groups * k or out_score.numel() < num_groups * k or out_count.numel() < num_groups:
+        raise L.NPIError("group_topk: outputs hold fewer than num_groups x k entries")
+    passes = L.query("npi_sort_passes", _i32(max(1, (int(num_groups) - 1).bit_length())))
+    L.call("npi_group_topk", L.ptr(scores), L.ptr(group), _i64(n), _i32(num_groups), _i32(k), L.ptr(out_pos),
+           L.ptr(out_score), L.ptr(out_count), L.ptr(status), L.ptr(ws), _i64(ws.numel() * ws.element_size()), _s(),
+           count_as=None if passes == 2 else "npi_group_topk/%dpass" % passes)
+
+
 # ----------------------------------------------------------------------------- operator-API helpers
 def filter_edges_coo(edge_index, new_id, out, count_dev):
     E = edge_index.shape[1]

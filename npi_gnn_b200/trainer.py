@@ -528,6 +528,32 @@ class Scorer:
         out["confusion"] = tuple(int(v) for v in counts.cpu())
         return out
 
+    def top_partners(self, k):
+        """The ``k`` most likely partners of every node, from ONE sweep of ``probabilities()``: the pairs grouped by their
+        RNA and by their protein (``top_k_by_group`` with the node serial as group id, so row s belongs to node s; rows of
+        nodes of the other type, or in no pair, have count 0).  Returns {"rna": ..., "protein": ...}, each
+        dict(partner, prob, count) of device tensors: partner int32 [num_nodes, k] = serial of the other endpoint by
+        descending probability (-1 past count), prob float32 [num_nodes, k] (NaN past count), count int32 [num_nodes].
+        Ties break by position in the pair set (in ``index`` order when a view was given).  With world_size > 1 every
+        rank's shard is gathered (torch.distributed must be initialised) and every rank computes the same,
+        bit-identical result over all pairs."""
+        from . import dist as D
+        if not 1 <= int(k) <= 1024:
+            raise ValueError("top_partners: k = %d outside 1..1024" % k)
+        if self.world_size > 1 and not D.dist.is_initialized():
+            raise L.NPIError("Scorer.top_partners with world_size > 1 needs an initialised torch.distributed process group")
+        probs = self.probabilities()
+        if self.world_size > 1:
+            probs = D.gather_shards(probs, self.P)
+        pairs = self.ps.pairs if self.index is None else self.ps.pairs[torch.from_numpy(self.index).to(self.device)]
+        out = {}
+        for name, own, other in (("rna", 0, 1), ("protein", 1, 0)):
+            r = top_k_by_group(probs, pairs[:, own].contiguous(), self.ps.graph.num_nodes, k)
+            hit = r["pos"] >= 0
+            partner = torch.where(hit, pairs[:, other][r["pos"].clamp(min=0).long()], -1)
+            out[name] = dict(partner=partner, prob=r["score"], count=r["count"])
+        return out
+
 
 def metrics(TP, FN, TN, FP):
     """Accuracy, Precision, Sensitivity, Specificity, MCC exactly as src/methods.py:107-127."""
@@ -580,3 +606,30 @@ def rank_metrics(scores, labels, curve=False):
         tpr = t / t[-1]
         out.update(thresholds=thr[:T], fpr=f / f[-1], tpr=tpr, precision=t / (t + f), recall=tpr)
     return out
+
+
+def top_k_by_group(scores, group, num_groups, k):
+    """The ``k`` highest of CUDA float32 ``scores`` in every group of int32 ``group`` ids (0 <= id < num_groups), in ONE
+    call of npi_group_topk and one synchronising read: dict(pos, score, count) of device tensors -- pos int32
+    [num_groups, k], the positions of the group's items by descending score with ties by ascending position (-0.0 and
+    +0.0 tie), -1 past count; score float32 [num_groups, k], those scores bit for bit, NaN past count; count int32
+    [num_groups] = min(k, group size).  NaN scores or group ids out of range raise NPIError; k outside 1..1024 raises
+    ValueError."""
+    if not 1 <= int(k) <= 1024:
+        raise ValueError("top_k_by_group: k = %d outside 1..1024" % k)
+    L.require_cuda(scores, group)
+    scores, group = scores.reshape(-1).contiguous(), group.reshape(-1).contiguous()
+    dev = scores.device
+    G, k = int(num_groups), int(k)
+    pos = torch.empty((G, k), dtype=torch.int32, device=dev)
+    score = torch.empty((G, k), dtype=torch.float32, device=dev)
+    count = torch.empty(G, dtype=torch.int32, device=dev)
+    status = torch.empty(1, dtype=torch.int32, device=dev)
+    ws = torch.empty(ops.group_topk_workspace_bytes(max(scores.numel(), 1), G), dtype=torch.uint8, device=dev)
+    ops.group_topk(scores, group, G, k, pos, score, count, status, ws)
+    st = int(status.item())
+    if st & 1:
+        raise L.NPIError("top_k_by_group: NaN score")
+    if st & 2:
+        raise L.NPIError("top_k_by_group: group id out of range [0, %d)" % G)
+    return dict(pos=pos, score=score, count=count)
