@@ -198,7 +198,7 @@ int npi_gemm_nn(const float* A, int32_t lda, const int32_t* m_dev, int32_t m_hos
  * (cp.async.bulk.tensor), the weights live in tensor memory.  K in 1..192 (transB: K in {32,64,96,128});
  * A and B 16-byte aligned, lda % 4 == 0; A must have at least m_host rows allocated (the tensor map
  * covers them; rows >= *m_dev are read but never stored).  single_pass bit 0: hi.hi product only
- * (plain TF32, diagnostic); bit 1: the register-staged A/B partner kernel (K % 32 == 0, K <= 128). */
+ * (plain TF32, diagnostic). */
 int npi_gemm_nn_tc(const float* A, int32_t lda, const int32_t* m_dev, int32_t m_host, int32_t K,
                    const float* B, int32_t transB, float* C, int32_t single_pass, npi_stream_t stream);
 /* out[K,128] = A[m,K]^T . D[m,128], rows split over CTAs, partials summed in a fixed order;
@@ -383,8 +383,6 @@ int npi_pool_gate_readout(const float* h, const float* s, const int32_t* perm,
                           void* workspace, int64_t workspace_bytes, int32_t phases, npi_stream_t stream);
 /* filter_adj on CSR: new row r = old row perm[r] with dropped sources removed and the rest
  * relabelled, order preserved.  rowptr_out[N'+1], col_out[<= E]; edge count in rowptr_out[N'].
- * packed_sel (nullable): the packed entries of npi_entry_pack_sel for the SAME CSR and selection -- both sweeps then
- * read new_id[col[k]] as one coalesced value per entry instead of chasing col -> new_id.
  * hub_queue / row_order (nullable; hub_e_max = the entry capacity the queue was sized for): the hub queue and the binned
  * row order of the NEW CSR are produced on the way (a row's segments need only its length, its record only its final
  * extent) -- what npi_hub_rows_build would do in two more kernels on the chain the next aggregation waits for.  The
@@ -392,7 +390,7 @@ int npi_pool_gate_readout(const float* h, const float* s, const int32_t* perm,
 int64_t npi_filter_adj_workspace_bytes(int32_t n_new_max);
 int npi_filter_adj(const int32_t* rowptr, const int32_t* col, const int32_t* perm,
                    const int32_t* new_id, const int32_t* nnew_dev, int32_t nnew_host,
-                   int32_t* rowptr_out, int32_t* col_out, const void* packed_sel,
+                   int32_t* rowptr_out, int32_t* col_out,
                    int32_t* hub_queue, int64_t hub_e_max, void* row_order,
                    void* workspace, int64_t workspace_bytes, npi_stream_t stream);
 int npi_hub_rows_reset(int32_t* hub_queue, npi_stream_t stream);
@@ -692,15 +690,6 @@ int64_t npi_tiny_partials_bytes(int32_t B);
 int npi_tiny_transpose(const float* w2, const float* w3, float* w2_t, float* w3_t, npi_stream_t stream);
 int npi_tiny_fwd(const npi_tiny_args_t* args, npi_stream_t stream);
 int npi_tiny_bwd(const npi_tiny_args_t* args, int32_t phases, npi_stream_t stream);
-/* Training step of every subgraph of a small batch in ONE launch: npi_tiny_fwd, then the head's forward and mean-NLL deltas
- * (npi_head_fwd_delta on readout / args->d_readout), then npi_tiny_bwd(phases = 1) -- same buffers, same results; what remains
- * of the step are the parameter gradients (npi_tiny_bwd(phases = 2), npi_head_bwd(phases = 2), npi_tiny_weight_grads), the
- * scalar loss (npi_head_fwd(phases = 2)) and the optimizer.  npi_tiny_transpose must have run on this step's weights. */
-int npi_tiny_step(const npi_tiny_args_t* args, const float* w1, const float* b1, const float* w2, const float* b2,
-                  const float* w3, const float* b3, int32_t training, const uint8_t* drop_mask_in, uint64_t seed,
-                  const int32_t* step_dev, const int32_t* sample_ids, int32_t sample_id_base, const int32_t* y,
-                  float loss_scale, float* a1, uint8_t* drop_mask_out, float* a2, float* logp,
-                  void* head_workspace, int64_t head_workspace_bytes, npi_stream_t stream);
 /* The three SAGEConv weight gradients of a small batch in ONE launch, fixed summation order (csrc/tiny.cu):
  *   d conv1.weight [F,128]  = sum_j x_j^T . dxa1_j over the n0 batch rows, x_j = [dist_j | table[gid_j][1:F]] (the virtual
  *                             input row, src/classes.py:706-717) -- the small-batch alternative to npi_gid_reduce +

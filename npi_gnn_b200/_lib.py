@@ -70,7 +70,7 @@ SIGNATURES = {
     "npi_pool_gate_readout_workspace_bytes": (_i64, [_i32]),
     "npi_pool_gate_readout": (C.c_int, [_vp, _vp, _vp, _vp, _i32, _vp, _vp, _i32, _vp, _vp, _i64, _i32, _vp]),
     "npi_filter_adj_workspace_bytes": (_i64, [_i32]),
-    "npi_filter_adj": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _i64, _vp, _vp, _i64, _vp]),
+    "npi_filter_adj": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _i64, _vp, _vp, _i64, _vp]),
     "npi_hub_rows_reset": (C.c_int, [_vp, _vp]),
     "npi_pool_bwd_workspace_bytes": (_i64, []),
     "npi_pool_bwd": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _vp, _i32, _vp, _vp, _vp, _vp, _i64, _i32, _vp]),
@@ -136,8 +136,6 @@ SIGNATURES = {
     "npi_tiny_transpose": (C.c_int, [_vp, _vp, _vp, _vp, _vp]),
     "npi_tiny_fwd": (C.c_int, [_TP, _vp]),
     "npi_tiny_bwd": (C.c_int, [_TP, _i32, _vp]),
-    "npi_tiny_step": (C.c_int, [_TP, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _vp, _u64, _vp, _vp, _i32, _vp, _f32, _vp, _vp, _vp, _vp,
-                                _vp, _i64, _vp]),
     "npi_tiny_weight_grads_workspace_bytes": (_i64, [_i32]),
     "npi_tiny_weight_grads": (C.c_int, [_vp, _i32, _i32, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _i32, _vp,
                                         _vp, _vp, _vp, _i32, _vp, _vp, _i64, _vp]),
@@ -185,7 +183,7 @@ KERNELS_PER_CALL = {
     "npi_confusion_counts": 1, "npi_rank_curve": 17, "npi_group_topk": 9, "npi_group_topk/1pass": 6, "npi_group_topk/3pass": 12,
     "npi_debug_stamp": 1, "npi_hub_rows_reset": 0, "npi_table_grad": 2, "npi_ctx_build": 2, "npi_sort_pairs_u32": 6, "npi_ctx_index_build": 22, "npi_ctx_class_pack": 1,
     "npi_ctx_scatter_max": 1, "npi_ctx_finish": 1, "npi_csr_gather_sum": 1, "npi_allreduce_adam_fused": 1, "npi_scalar_axpy": 1, "npi_peer_barrier": 1,
-    "npi_head_fwd_delta": 1, "npi_tiny_transpose": 1, "npi_tiny_fwd": 1, "npi_tiny_bwd": 2, "npi_tiny_bwd/phase": 1, "npi_tiny_weight_grads": 1, "npi_tiny_step": 1,
+    "npi_head_fwd_delta": 1, "npi_tiny_transpose": 1, "npi_tiny_fwd": 1, "npi_tiny_bwd": 2, "npi_tiny_bwd/phase": 1, "npi_tiny_weight_grads": 1,
     "npi_n2v_etab_scan": 1, "npi_n2v_alias_tables": 1, "npi_n2v_alias_from_probs": 1, "npi_n2v_walks": 1,
     "npi_n2v_vocab_count": 1, "npi_n2v_init_vectors": 1, "npi_n2v_skipgram": 1,
 }

@@ -19,7 +19,6 @@
 namespace npi {
 namespace tc {
 
-constexpr int TC_THREADS = 128;
 constexpr uint32_t TILE_BYTES = 128 * 128;      // [128][32] fp32
 constexpr uint32_t TMEM_COLS = 128;
 
@@ -38,15 +37,6 @@ __device__ __forceinline__ uint64_t make_desc(uint32_t saddr) {
 // instruction descriptor: D = f32, A = B = tf32, both K-major, N = 128, M = 128
 constexpr uint32_t IDESC = (1u << 4) | (2u << 7) | (2u << 10) | ((128u >> 3) << 17) | ((128u >> 4) << 24);
 
-__device__ __forceinline__ void mma_tf32(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t"
-        "}\n" ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(IDESC), "r"(accumulate)
-        : "memory");
-}
 __device__ __forceinline__ void mma_commit(uint32_t bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
 }
@@ -97,21 +87,6 @@ struct Args {
 };
 int make_tmap_rows(CUtensorMap* tmap, const float* A, int lda, int rows, int cols);
 
-// store one 16-byte chunk (4 consecutive k of row r) of a [128][32] tile, hi and lo parts
-__device__ __forceinline__ void put_chunk(uint8_t* hi_tile, uint8_t* lo_tile, int r, int chunk, float4 v) {
-    const uint32_t off = (uint32_t)(r * 128 + ((chunk ^ (r & 7)) << 4));
-    float4 h = make_float4(tf32_hi(v.x), tf32_hi(v.y), tf32_hi(v.z), tf32_hi(v.w));
-    float4 l = make_float4(tf32_lo(v.x, h.x), tf32_lo(v.y, h.y), tf32_lo(v.z, h.z), tf32_lo(v.w, h.w));
-    *reinterpret_cast<float4*>(hi_tile + off) = h;
-    *reinterpret_cast<float4*>(lo_tile + off) = l;
-}
-__device__ __forceinline__ void put_scalar(uint8_t* hi_tile, uint8_t* lo_tile, int r, int k, float v) {
-    const uint32_t off = (uint32_t)(r * 128 + ((((k >> 2) ^ (r & 7)) << 4) | ((k & 3) << 2)));
-    const float h = tf32_hi(v);
-    *reinterpret_cast<float*>(hi_tile + off) = h;
-    *reinterpret_cast<float*>(lo_tile + off) = tf32_lo(v, h);
-}
-
 
 // ------------------------------------------------------------------------------------------------
 // TMA-fed version with the WEIGHTS RESIDENT IN TENSOR MEMORY (the product path).
@@ -121,8 +96,8 @@ __device__ __forceinline__ void put_scalar(uint8_t* hi_tile, uint8_t* lo_tile, i
 // hi and lo parts of the 128 x K weight matrix take 2 x K of the 512 TMEM columns for the lifetime of
 // the CTA (K <= 128: two 128-column accumulators take the other 256; 128 < K <= 192, the 178-column
 // feature table of layer 1: one accumulator) -- so NO shared memory is spent on the
-// weights (the register-staged kernel below keeps 128 KB of W in smem and has room for only three
-// 32 KB operand stages) and the MMA reads half as many operand bytes from shared memory.  The "B"
+// weights (a register-staged design that kept 128 KB of W in smem had room for only three 32 KB
+// operand stages, and was measured slower) and the MMA reads half as many operand bytes from shared memory.  The "B"
 // operand is the streamed X tile [128 rows m][32 k], K-major SWIZZLE_128B -- exactly what a TMA box
 // load of the raw fp32 rows produces.
 //   warp 5 (one lane)  TMA producer: cp.async.bulk.tensor.2d of a 128 x 32 fp32 box (16 KB, rows beyond the
@@ -135,8 +110,8 @@ __device__ __forceinline__ void put_scalar(uint8_t* hi_tile, uint8_t* lo_tile, i
 //                      releases the stage to the TMA producer
 //   warps 0-3          epilogue: tcgen05.ld hands lane l of warp w the values C[m0 .. m0+31][32w + l]; a
 //                      store instruction of the warp therefore writes 32 CONSECUTIVE floats of one row of
-//                      C (128 B coalesced) with no register transpose (the register-staged kernel needs
-//                      160 shuffles per 32 x 32 block for the same effect)
+//                      C (128 B coalesced) with no register transpose (with C untransposed in TMEM, lane = row,
+//                      160 shuffles per 32 x 32 block are needed for the same effect)
 #ifndef NPI_TM_RAW
 #define NPI_TM_RAW 6
 #endif
@@ -401,178 +376,6 @@ __global__ void __launch_bounds__(TM_THREADS, 1) gemm_tc_tma_kernel(Args a, cons
 
 
 // ------------------------------------------------------------------------------------------------
-// Warp-specialised persistent version.  Roles inside one CTA (1 CTA per SM):
-//   warps 0-3    epilogue: TMEM -> registers -> global (warp w owns TMEM lanes 32w..32w+31)
-//   warp  4      MMA issuer (one elected lane) + TMEM allocation
-//   warps 5-16   three producer groups of 4 warps; group g fills smem stage g with the A slices
-//                s = g, g+3, g+6, ... (global -> registers -> hi/lo split -> swizzled smem), so three
-//                16 KB slices of A are in flight per SM while the tensor core works on a fourth.
-// Pipelines: full[stage]/empty[stage] between producers and the MMA issuer (tcgen05.commit frees a
-// stage when its MMAs have read it), tmem_full[acc]/tmem_empty[acc] between the issuer and the
-// epilogue over two 128-column accumulators, so tile i+1 is multiplied while tile i is written out.
-constexpr int WS_STAGES = 3;
-constexpr int WS_EPI_WARPS = 4;
-constexpr int WS_PROD_WARPS = 4 * WS_STAGES;
-constexpr int WS_THREADS = 32 * (WS_EPI_WARPS + 1 + WS_PROD_WARPS);     // 544
-constexpr uint32_t WS_TMEM_COLS = 256;
-
-__global__ void __launch_bounds__(WS_THREADS, 1) gemm_tc_ws_kernel(Args a) {
-    extern __shared__ uint8_t smem_raw[];
-    __shared__ __align__(8) uint64_t bar_full[WS_STAGES], bar_empty[WS_STAGES], bar_tfull[2], bar_tempty[2];
-    __shared__ uint32_t tmem_slot;
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int M = dev_size(a.m_dev, a.m_host);
-    const int KB = a.K / 32;
-    const int ntiles = (M + 127) / 128;
-    if ((int)blockIdx.x >= ntiles) return;            // uniform: nothing allocated yet
-
-    uint8_t* base = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-    uint8_t* sB_hi = base;                            // KB tiles
-    uint8_t* sB_lo = sB_hi + KB * TILE_BYTES;
-    uint8_t* sA = sB_lo + KB * TILE_BYTES;            // WS_STAGES x (hi tile | lo tile)
-
-    if (warp == WS_EPI_WARPS) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_slot)), "r"(WS_TMEM_COLS) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    if (tid == 0) {
-        for (int i = 0; i < WS_STAGES; ++i) { mbar_init(smem_u32(&bar_full[i]), 128); mbar_init(smem_u32(&bar_empty[i]), 1); }
-        for (int i = 0; i < 2; ++i) { mbar_init(smem_u32(&bar_tfull[i]), 1); mbar_init(smem_u32(&bar_tempty[i]), 32 * WS_EPI_WARPS); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    // ---- B operand (weights), resident, staged by the whole CTA
-    if (!a.transB) {
-        for (int e = tid; e < a.K * 32; e += WS_THREADS) {
-            const int k = e >> 5, n4 = (e & 31) * 4;
-            const float4 v = ldg4(a.B + (int64_t)k * 128 + n4);
-            uint8_t* th = sB_hi + (k >> 5) * TILE_BYTES;
-            uint8_t* tl = sB_lo + (k >> 5) * TILE_BYTES;
-            put_scalar(th, tl, n4 + 0, k & 31, v.x);
-            put_scalar(th, tl, n4 + 1, k & 31, v.y);
-            put_scalar(th, tl, n4 + 2, k & 31, v.z);
-            put_scalar(th, tl, n4 + 3, k & 31, v.w);
-        }
-    } else {
-        const int kq = a.K / 4;
-        for (int e = tid; e < 128 * kq; e += WS_THREADS) {
-            const int n = e / kq, k4 = (e % kq) * 4;
-            const float4 v = ldg4(a.B + (int64_t)n * a.K + k4);
-            put_chunk(sB_hi + (k4 >> 5) * TILE_BYTES, sB_lo + (k4 >> 5) * TILE_BYTES, n, (k4 & 31) >> 2, v);
-        }
-    }
-    fence_async_smem();
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem = tmem_slot;
-    const int my_tiles = (ntiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
-
-    if (warp < WS_EPI_WARPS) {
-        // ================= epilogue =================
-        for (int it = 0; it < my_tiles; ++it) {
-            const int row0 = ((int)blockIdx.x + it * (int)gridDim.x) * 128;
-            const int acc = it & 1;
-            mbar_wait(smem_u32(&bar_tfull[acc]), (uint32_t)((it >> 1) & 1));
-            tc_fence_after();
-            // tcgen05.ld hands lane l the 32 columns of ROW l: stored as is, every store instruction of the
-            // warp touches 32 different 128-byte lines, 16 bytes each -- ncu showed the kernel paced by those
-            // L1 wavefronts (l1tex 64 %, HBM 16 %; profiles/r01x_ncu.md).  A 32x32 register transpose (five
-            // shuffle-xor stages, static register indices) turns them into 128-byte coalesced row stores.
-            const int rbase = row0 + warp * 32;
-#pragma unroll
-            for (int cb = 0; cb < 4; ++cb) {
-                uint32_t r[32];
-                tmem_ld32(tmem + ((uint32_t)(warp * 32) << 16) + acc * 128 + cb * 32, r);
-                tmem_ld_wait();
-#pragma unroll
-                for (int sft = 16; sft > 0; sft >>= 1) {
-                    const bool up = (lane & sft) != 0;
-#pragma unroll
-                    for (int j = 0; j < 32; ++j) {
-                        if ((j & sft) == 0) {
-                            const uint32_t send = up ? r[j] : r[j | sft];
-                            const uint32_t recv = __shfl_xor_sync(0xffffffffu, send, sft);
-                            if (up) r[j] = recv; else r[j | sft] = recv;
-                        }
-                    }
-                }
-                // now r[j] on lane l = C[rbase + j][cb * 32 + l]
-                float* dst = a.C + (int64_t)rbase * 128 + cb * 32 + lane;
-#pragma unroll
-                for (int j = 0; j < 32; ++j)
-                    if (rbase + j < M) dst[(int64_t)j * 128] = __uint_as_float(r[j]);
-            }
-            tc_fence_before();
-            mbar_arrive(smem_u32(&bar_tempty[acc]));
-        }
-    } else if (warp == WS_EPI_WARPS) {
-        // ================= MMA issuer =================
-        if (lane == 0) {
-            int s = 0;
-            for (int it = 0; it < my_tiles; ++it) {
-                const int acc = it & 1;
-                mbar_wait(smem_u32(&bar_tempty[acc]), (uint32_t)(((it >> 1) & 1) ^ 1));
-                tc_fence_after();
-                const uint32_t d = tmem + acc * 128;
-                for (int kb = 0; kb < KB; ++kb, ++s) {
-                    const int st = s % WS_STAGES;
-                    mbar_wait(smem_u32(&bar_full[st]), (uint32_t)((s / WS_STAGES) & 1));
-                    tc_fence_after();
-                    const uint32_t ah = smem_u32(sA) + st * 2 * TILE_BYTES, al = ah + TILE_BYTES;
-                    const uint32_t bh = smem_u32(sB_hi) + kb * TILE_BYTES, bl = smem_u32(sB_lo) + kb * TILE_BYTES;
-#pragma unroll
-                    for (int ks = 0; ks < 4; ++ks) {
-                        const uint32_t ko = ks * 32;
-                        const uint32_t accum = (kb | ks) ? 1u : 0u;
-                        if (a.single_pass) {
-                            mma_tf32(d, make_desc(ah + ko), make_desc(bh + ko), accum);
-                        } else {
-                            mma_tf32(d, make_desc(al + ko), make_desc(bh + ko), accum);
-                            mma_tf32(d, make_desc(ah + ko), make_desc(bl + ko), 1u);
-                            mma_tf32(d, make_desc(ah + ko), make_desc(bh + ko), 1u);
-                        }
-                    }
-                    mma_commit(smem_u32(&bar_empty[st]));       // stage reusable once these MMAs have read it
-                }
-                mma_commit(smem_u32(&bar_tfull[acc]));          // accumulator complete
-            }
-        }
-        __syncwarp();
-    } else {
-        // ================= producers =================
-        const int g = (warp - WS_EPI_WARPS - 1) >> 2;                // stage owned by this group
-        const int t = tid - 32 * (WS_EPI_WARPS + 1) - g * 128;       // 0..127 inside the group
-        uint8_t* hi = sA + g * 2 * TILE_BYTES;
-        uint8_t* lo = hi + TILE_BYTES;
-        const int total = my_tiles * KB;
-        for (int s = g, u = 0; s < total; s += WS_STAGES, ++u) {
-            const int it = s / KB, kb = s % KB;
-            const int row0 = ((int)blockIdx.x + it * (int)gridDim.x) * 128;
-            float4 v[8];
-#pragma unroll
-            for (int q = 0; q < 8; ++q) {
-                const int e = t + q * 128;
-                const int gr = min(row0 + (e >> 3), M - 1);
-                v[q] = ldg4(a.A + (int64_t)gr * a.lda + kb * 32 + (e & 7) * 4);
-            }
-            mbar_wait(smem_u32(&bar_empty[g]), (uint32_t)((u & 1) ^ 1));
-#pragma unroll
-            for (int q = 0; q < 8; ++q) {
-                const int e = t + q * 128;
-                put_chunk(hi, lo, e >> 3, e & 7, v[q]);
-            }
-            fence_async_smem();
-            mbar_arrive(smem_u32(&bar_full[g]));
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == WS_EPI_WARPS)
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(WS_TMEM_COLS) : "memory");
-}
-
-
-// ------------------------------------------------------------------------------------------------
 // Weight gradient  out[128,128] = A[M,128]^T . D[M,128]  (dW = X^T . DXA of reference SAGEConv backward,
 // SURVEY Appendix A.2) on tcgen05: the reduction runs over the ROWS, so both operands are "MN-major"
 // for the tensor core -- a row of A (resp. D) holds the 128 values of the UMMA M (resp. N) dimension
@@ -581,8 +384,17 @@ __global__ void __launch_bounds__(WS_THREADS, 1) gemm_tc_ws_kernel(Args a) {
 // XORed with row & 3).  Slab of 32 rows: [4 column blocks of 32 floats][32 rows][128 B]; descriptor
 // LBO = 4096 B (between column blocks), SBO = 512 B (between 4-row atoms); one UMMA_K step = 8 rows.  Persistent CTAs take slabs round-robin (split over rows),
 // accumulate everything in ONE 128x128 fp32 TMEM tile and write it out once; the per-CTA partials
-// are summed in a fixed order by gemm_tn_reduce_kernel.  Same 3xTF32 split and the same
-// producer / MMA-issuer / epilogue warp roles as gemm_tc_ws_kernel.
+// are summed in a fixed order by gemm_tn_reduce_kernel.  Same 3xTF32 split as the projection above.
+// Warp roles inside one CTA (1 CTA per SM):
+//   warps 0-3    epilogue: TMEM -> registers -> global (warp w owns TMEM lanes 32w..32w+31)
+//   warp  4      MMA issuer (one elected lane) + TMEM allocation
+//   warps 5-16   three producer groups of 4 warps; group g fills smem stage g with the slabs s = g, g+3, g+6, ...
+//                (global -> registers -> hi/lo split -> swizzled smem), so three slabs are in flight per SM
+//                while the tensor core works on a fourth; tcgen05.commit frees a stage when its MMAs have read it
+constexpr int WS_STAGES = 3;
+constexpr int WS_EPI_WARPS = 4;
+constexpr int WS_PROD_WARPS = 4 * WS_STAGES;
+constexpr int WS_THREADS = 32 * (WS_EPI_WARPS + 1 + WS_PROD_WARPS);     // 544
 constexpr uint32_t TN_SLAB_ROWS = 32;
 constexpr uint32_t TN_OPER_BYTES = TN_SLAB_ROWS * 512;          // one operand slab (hi or lo): 16 KB
 constexpr uint32_t IDESC_MN = IDESC | (1u << 15) | (1u << 16);  // A and B MN-major
@@ -771,33 +583,22 @@ extern "C" int npi_gemm_nn_tc(const float* A, int32_t lda, const int32_t* m_dev,
                               const float* B, int32_t transB, float* C, int32_t single_pass, npi_stream_t stream) {
     NPI_REQUIRE(A && B && C, "gemm_nn_tc: null argument");
     NPI_REQUIRE(K >= 1 && K <= 192, "gemm_nn_tc: K must be in 1..192 (got %d)", K);
-    NPI_REQUIRE((K % 32 == 0 && K <= 128) || (!transB && !(single_pass & 2)),
-                "gemm_nn_tc: K = %d needs the TMA kernel with a [K,128] weight matrix (transB = 0)", K);
+    NPI_REQUIRE(!transB || (K % 32 == 0 && K <= 128), "gemm_nn_tc: transB needs K in {32, 64, 96, 128} (got %d)", K);
     NPI_REQUIRE(lda >= K && lda % 4 == 0 && (reinterpret_cast<uintptr_t>(A) & 15) == 0 && (reinterpret_cast<uintptr_t>(B) & 15) == 0,
                 "gemm_nn_tc: operands must be 16-byte aligned with lda %% 4 == 0");
+    NPI_REQUIRE(m_host > 0, "gemm_nn_tc: m_host must be positive");
     tc::Args a{A, lda, m_dev, m_host, K, B, transB, C, single_pass & 1};
-    const int KB = (K + 31) / 32;
     int tiles = (m_host + 127) / 128;
     int grid = num_sms();
-    if (tiles < grid) grid = tiles > 0 ? tiles : 1;
-    if (!(single_pass & 2)) {                    // product path: TMA loads, weights resident in tensor memory
-        CUtensorMap tmap;
-        NPI_REQUIRE(m_host > 0, "gemm_nn_tc: m_host must be positive");
-        if (int rc = tc::make_tmap_rows(&tmap, A, lda, m_host, K)) return rc;
-        const size_t smem = (size_t)(2 * tc::TM_OPS + tc::TM_RAW) * tc::TILE_BYTES + 1024;
-        static OncePerDevice configured;
-        if (configured.need()) {
-            NPI_CHECK_CUDA(cudaFuncSetAttribute(tc::gemm_tc_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        }
-        NPI_CHECK_CUDA(launch_dep(tc::gemm_tc_tma_kernel, grid, tc::TM_THREADS, smem, (cudaStream_t)stream, a, tmap));
-    } else {                                     // A/B partner: register-staged producers, weights in shared memory
-        const size_t smem = (size_t)(2 * KB + 2 * tc::WS_STAGES) * tc::TILE_BYTES + 1024;
-        static MaxPerDevice configured;
-        if (configured.need(smem)) {
-            NPI_CHECK_CUDA(cudaFuncSetAttribute(tc::gemm_tc_ws_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        }
-        tc::gemm_tc_ws_kernel<<<grid, tc::WS_THREADS, smem, (cudaStream_t)stream>>>(a);
+    if (tiles < grid) grid = tiles;
+    CUtensorMap tmap;
+    if (int rc = tc::make_tmap_rows(&tmap, A, lda, m_host, K)) return rc;
+    const size_t smem = (size_t)(2 * tc::TM_OPS + tc::TM_RAW) * tc::TILE_BYTES + 1024;
+    static OncePerDevice configured;
+    if (configured.need()) {
+        NPI_CHECK_CUDA(cudaFuncSetAttribute(tc::gemm_tc_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     }
+    NPI_CHECK_CUDA(launch_dep(tc::gemm_tc_tma_kernel, grid, tc::TM_THREADS, smem, (cudaStream_t)stream, a, tmap));
     NPI_CHECK_LAUNCH();
     return NPI_OK;
 }

@@ -1,5 +1,5 @@
-// MLP head of Net_1 (src/classes.py:74-80) as device functions shared by head.cu (one CTA per sample) and tiny.cu (inside the
-// per-subgraph training-step kernel).
+// MLP head of Net_1 (src/classes.py:74-80) as device functions shared by head_fwd_kernel and head_fwd_delta_kernel (head.cu, one
+// CTA per sample).
 #pragma once
 #include "common.cuh"
 
@@ -22,9 +22,9 @@ struct HeadSmem {
     uint8_t keep[D1];        // dropout decisions (1 when not training)
 };
 
-// forward of sample b by the whole CTA (NT threads: 512 in head.cu, 256 inside the per-subgraph step kernel of tiny.cu -- the
-// per-output arithmetic, a full-warp dot product, does not depend on it); leaves a1 (after dropout), a2, the log-probabilities and the
-// dropout decisions in S as well as in global memory; ends with a block barrier
+// forward of sample b by the whole CTA of NT threads (the per-output arithmetic, a full-warp dot product, does not depend on NT);
+// leaves a1 (after dropout), a2, the log-probabilities and the dropout decisions in S as well as in global memory; ends with a
+// block barrier
 template <int NT>
 __device__ __forceinline__ void head_fwd_body(HeadSmem& S, const int b,
     const float* readout, const float* w1, const float* b1, const float* w2, const float* b2,

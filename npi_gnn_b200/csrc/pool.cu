@@ -352,12 +352,9 @@ __device__ __forceinline__ void fa_locate(const FaRows& f, int pos, int& q, int&
     k = __shfl_sync(0xffffffffu, f.b, lo) + (pos - __shfl_sync(0xffffffffu, f.off, lo));
 }
 
-// sel (nullable): the packed entries {new_id[col[k]], weight} of npi_entry_pack_sel for the same CSR -- one coalesced load
-// per entry instead of the col -> new_id chase
 __global__ void __launch_bounds__(FA_THREADS) filter_count_kernel(const int32_t* rowptr, const int32_t* col, const int32_t* perm,
                                                                    const int32_t* new_id, const int32_t* nnew_dev, int nnew_host,
-                                                                   int32_t* rowptr_out, int32_t* partial, const int2* __restrict__ sel,
-                                                                   int32_t* hubq, int hubq_cap) {
+                                                                   int32_t* rowptr_out, int32_t* partial, int32_t* hubq, int hubq_cap) {
     __shared__ int sh[FA_THREADS / 32 + 2];
     __shared__ int s_cnt[FA_WARPS][32];
     __shared__ int s_hist[N_CLS];
@@ -379,13 +376,11 @@ __global__ void __launch_bounds__(FA_THREADS) filter_count_kernel(const int32_t*
             c[u] = -1; q[u] = 0;
             if (p0 + 32 * u < f.total) {                       // warp-uniform: chunks behind the end cost nothing
                 fa_locate(f, min(p, f.total - 1), q[u], k);
-                if (p < f.total) c[u] = sel ? sel[k].x : col[k];
+                if (p < f.total) c[u] = col[k];
             }
         }
-        if (!sel) {
 #pragma unroll
-            for (int u = 0; u < FA_CHUNKS; ++u) c[u] = (c[u] >= 0) ? new_id[c[u]] : -1;
-        }
+        for (int u = 0; u < FA_CHUNKS; ++u) c[u] = (c[u] >= 0) ? new_id[c[u]] : -1;
 #pragma unroll
         for (int u = 0; u < FA_CHUNKS; ++u)
             if (c[u] >= 0) atomicAdd(&s_cnt[warp][q[u]], 1);
@@ -428,8 +423,7 @@ __global__ void __launch_bounds__(1024) scan_partials_kernel(int32_t* partial, i
 __global__ void __launch_bounds__(FA_THREADS) filter_fill_kernel(const int32_t* rowptr, const int32_t* col, const int32_t* perm,
                                                                   const int32_t* new_id, const int32_t* nnew_dev, int nnew_host,
                                                                   int32_t* rowptr_out, int32_t* col_out, const int32_t* partial,
-                                                                  const int2* __restrict__ sel, int32_t* hubq, int hubq_cap,
-                                                                  int4* __restrict__ rows, int nchunks) {
+                                                                  int32_t* hubq, int hubq_cap, int4* __restrict__ rows, int nchunks) {
     __shared__ int s_pre[FA_THREADS + 1];
     __shared__ int s_hist[N_CLS], s_start[N_CLS];
     const int nnew = dev_size(nnew_dev, nnew_host);
@@ -479,13 +473,11 @@ __global__ void __launch_bounds__(FA_THREADS) filter_fill_kernel(const int32_t* 
             id[u] = -1;
             if (p0 + 32 * u < f.total) {                       // warp-uniform
                 fa_locate(f, min(p, f.total - 1), q, k);
-                if (p < f.total) id[u] = sel ? sel[k].x : col[k];
+                if (p < f.total) id[u] = col[k];
             }
         }
-        if (!sel) {
 #pragma unroll
-            for (int u = 0; u < FA_CHUNKS; ++u) id[u] = (id[u] >= 0) ? new_id[id[u]] : -1;
-        }
+        for (int u = 0; u < FA_CHUNKS; ++u) id[u] = (id[u] >= 0) ? new_id[id[u]] : -1;
 #pragma unroll
         for (int u = 0; u < FA_CHUNKS; ++u) {
             const unsigned b = __ballot_sync(0xffffffffu, id[u] >= 0);
@@ -725,7 +717,7 @@ extern "C" int64_t npi_filter_adj_workspace_bytes(int32_t n_new_max) {
 
 extern "C" int npi_filter_adj(const int32_t* rowptr, const int32_t* col, const int32_t* perm, const int32_t* new_id,
                               const int32_t* nnew_dev, int32_t nnew_host, int32_t* rowptr_out, int32_t* col_out,
-                              const void* packed_sel, int32_t* hub_queue, int64_t hub_e_max, void* row_order,
+                              int32_t* hub_queue, int64_t hub_e_max, void* row_order,
                               void* workspace, int64_t workspace_bytes, npi_stream_t stream) {
     NPI_REQUIRE(rowptr && col && perm && new_id && rowptr_out && col_out && workspace, "filter_adj: null argument");
     NPI_REQUIRE(!row_order || hub_queue, "filter_adj: row_order comes with hub_queue");
@@ -736,15 +728,14 @@ extern "C" int npi_filter_adj(const int32_t* rowptr, const int32_t* col, const i
     int nchunks = (nnew_host + FA_THREADS - 1) / FA_THREADS;
     int32_t* partial = (int32_t*)workspace;
     if (nchunks > 0) {
-        filter_count_kernel<<<nchunks, FA_THREADS, 0, st>>>(rowptr, col, perm, new_id, nnew_dev, nnew_host, rowptr_out, partial, (const int2*)packed_sel,
-                                                            hub_queue, hcap);
+        filter_count_kernel<<<nchunks, FA_THREADS, 0, st>>>(rowptr, col, perm, new_id, nnew_dev, nnew_host, rowptr_out, partial, hub_queue, hcap);
         NPI_CHECK_LAUNCH();
     }
     scan_partials_kernel<<<1, 1024, 0, st>>>(partial, nchunks, nnew_dev, nnew_host, rowptr_out);
     NPI_CHECK_LAUNCH();
     if (nchunks > 0) {
         filter_fill_kernel<<<nchunks, FA_THREADS, 0, st>>>(rowptr, col, perm, new_id, nnew_dev, nnew_host, rowptr_out, col_out, partial,
-                                                           (const int2*)packed_sel, hub_queue, hcap, (int4*)row_order, nchunks);
+                                                           hub_queue, hcap, (int4*)row_order, nchunks);
         NPI_CHECK_LAUNCH();
     }
     return NPI_OK;

@@ -25,7 +25,7 @@
 // edge list is never longer) -- no scan over the batch, hence no dependency between CTAs.
 // Sums run in a fixed order (CSR order then the self row; half-warps combined in order): reruns are bit-identical, and
 // layer 1's h is bit-identical to aggregate_fwd_kernel's.
-#include "head.cuh"
+#include "common.cuh"
 
 namespace npi {
 
@@ -404,7 +404,7 @@ __device__ __forceinline__ void tn_filter(const TnSmem& sm, const int* sRp, cons
 // through every phase once, so what it waits for is largely instruction fetch (the three-times-unrolled kernel was 111 KB of
 // SASS and every phase cost >= 1 us however small the subgraph) -- layers 2 and 3 now run out of the instruction cache
 __device__ __forceinline__ void tn_fwd_layer(const npi_tiny_args_t& a, const int L, int g, const TnSmem& sm, int base, float* xs, float* ys, float* hs,
-                                             float* pbuf, float& ro_max, float& ro_mean, const float* stage_after_l2) {
+                                             float* pbuf, float& ro_max, float& ro_mean) {
     const int tid = threadIdx.x, hw = tid >> 4, l16 = tid & 15;
     const int lo = a.graph_ptr[L][g];
     const int n = min(a.graph_ptr[L][g + 1] - lo, sm.cap);
@@ -428,10 +428,7 @@ __device__ __forceinline__ void tn_fwd_layer(const npi_tiny_args_t& a, const int
     } else {
         tn_bar_wait(sm.bar, (uint32_t)(L - 1) & 1u);                           // conv(L+1).weight has landed in shared memory
         tn_project(a.xp[Lm], sm.W, a.y[L], lo, n, xs, true, ys, pbuf);
-        if (tid == 0) {      // the next weight lands while this layer aggregates, sorts and gates
-            if (L == 1) tn_stage_weight(sm.W, a.weight[2], sm.bar);
-            else if (stage_after_l2) tn_stage_weight(sm.W, stage_after_l2, sm.bar);      // step kernel: conv3.weight^T for the backward
-        }
+        if (tid == 0 && L == 1) tn_stage_weight(sm.W, a.weight[2], sm.bar);      // conv3.weight lands while this layer aggregates, sorts and gates
         TN_STAMP(a.dxa[0], 1 + 5 * L);
         tn_aggregate<false>(a, L, lo, n, sm, sRpC, sColC, colg, a.y[L], ys, hs);
     }
@@ -503,7 +500,7 @@ __global__ void __launch_bounds__(TN_THREADS, 2) tiny_fwd_kernel(const __grid_co
     const int base = a.rowptr0[a.graph_ptr[0][g]];
     float ro_max = 0.f, ro_mean = 0.f;
 #pragma unroll 1
-    for (int L = 0; L < 3; ++L) tn_fwd_layer(a, L, g, sm, base, xs, ys, hs, pbuf, ro_max, ro_mean, nullptr);
+    for (int L = 0; L < 3; ++L) tn_fwd_layer(a, L, g, sm, base, xs, ys, hs, pbuf, ro_max, ro_mean);
     if (threadIdx.x < H) {
         a.readout[(int64_t)g * 2 * H + threadIdx.x] = ro_max;                  // x1 + x2 + x3 (src/classes.py:74)
         a.readout[(int64_t)g * 2 * H + H + threadIdx.x] = ro_mean;
@@ -698,51 +695,6 @@ __global__ void __launch_bounds__(TN_THREADS, 2) tiny_bwd_kernel(const __grid_co
     const int base = a.rowptr0[a.graph_ptr[0][g]];
 #pragma unroll 1
     for (int L = 2; L >= 0; --L) tn_bwd_layer(a, L, g, sm, base, xs, ds, gs, pbuf, sred, sdb);
-}
-
-// Training step of one subgraph in ONE launch: forward of the three layers, the MLP head with its mean-NLL deltas
-// (head.cuh), and the backward of the three layers -- nothing between them crosses a subgraph, so the grid-wide barriers that
-// two kernel boundaries put there only made every subgraph wait for the largest one twice more (forward 37 us + head 12 us +
-// backward 31 us as launches against ~45 us for the median subgraph straight through).  The weights follow each other through
-// the one shared-memory slot: conv2.weight, conv3.weight, conv3.weight^T, conv2.weight^T (barrier phases 0..3).
-struct TinyHeadArgs {
-    const float *w1, *b1, *w2, *b2, *w3, *b3;
-    int training; const uint8_t* mask_in; uint64_t seed; const int32_t* step_dev; const int32_t* sample_ids; int sample_id_base;
-    const int32_t* y; float scale;
-    float* a1; uint8_t* mask_out; float* a2; float* logp; float* ws;
-};
-
-__global__ void __launch_bounds__(TN_THREADS, 2) tiny_step_kernel(const __grid_constant__ npi_tiny_args_t a, const __grid_constant__ TinyHeadArgs hd,
-                                                                  int cap) {
-    pdl_trigger();
-    pdl_wait();
-    extern __shared__ __align__(128) unsigned char tn_smem[];
-    __shared__ __align__(16) float xs[TN_TILE * H], t1[TN_TILE * H], t2[TN_TILE * H], pbuf[8 * H];
-    __shared__ __align__(16) float sred[TN_WARPS][H + 4];
-    __shared__ __align__(16) float sdb[TN_WARPS][H];
-    __shared__ HeadSmem S;
-    __shared__ HeadDeltaSmem Dl;
-    const TnSmem sm = tn_carve(tn_smem, cap);
-    const int g = blockIdx.x;
-    if (g >= a.B) return;
-    if (threadIdx.x == 0) tn_bar_init(sm.bar);
-    __syncthreads();
-    if (threadIdx.x == 0) tn_stage_weight(sm.W, a.weight[1], sm.bar);
-    const int base = a.rowptr0[a.graph_ptr[0][g]];
-    float ro_max = 0.f, ro_mean = 0.f;
-#pragma unroll 1
-    for (int L = 0; L < 3; ++L) tn_fwd_layer(a, L, g, sm, base, xs, t1, t2, pbuf, ro_max, ro_mean, a.weight_t[2]);
-    if (threadIdx.x < H) {
-        a.readout[(int64_t)g * 2 * H + threadIdx.x] = ro_max;
-        a.readout[(int64_t)g * 2 * H + H + threadIdx.x] = ro_mean;
-    }
-    __syncthreads();
-    head_fwd_body<TN_THREADS>(S, g, a.readout, hd.w1, hd.b1, hd.w2, hd.b2, hd.w3, hd.b3, hd.training, hd.mask_in, hd.seed, hd.step_dev,
-                              hd.sample_ids, hd.sample_id_base, hd.a1, hd.mask_out, hd.a2, hd.logp);
-    head_delta_body<TN_THREADS>(S, Dl, g, hd.w1, hd.w2, hd.w3, hd.training, hd.y, hd.scale, hd.ws, const_cast<float*>(a.d_readout));
-    __syncthreads();
-#pragma unroll 1
-    for (int L = 2; L >= 0; --L) tn_bwd_layer(a, L, g, sm, base, xs, t1, t2, pbuf, sred, sdb);
 }
 
 // d_pool_w / d_bias of the three layers from the per-subgraph partials, fixed order: grid (128/32 column blocks, 3 layers),
@@ -1015,33 +967,5 @@ extern "C" int npi_tiny_weight_grads(const float* table, int32_t ld, int32_t F, 
         tiny_weight_grad_kernel<<<dim3(tiles, maxs, njobs), WG_WARPS * 32, 0, (cudaStream_t)stream>>>(jobs);
     }
     NPI_CHECK_LAUNCH();
-    return NPI_OK;
-}
-
-extern "C" int npi_tiny_step(const npi_tiny_args_t* a, const float* w1, const float* b1, const float* w2, const float* b2,
-                             const float* w3, const float* b3, int32_t training, const uint8_t* drop_mask_in, uint64_t seed,
-                             const int32_t* step_dev, const int32_t* sample_ids, int32_t sample_id_base, const int32_t* y,
-                             float loss_scale, float* a1, uint8_t* drop_mask_out, float* a2, float* logp,
-                             void* head_workspace, int64_t head_workspace_bytes, npi_stream_t stream) {
-    int rc = tiny_check_common(a, "tiny_step");
-    if (rc != NPI_OK) return rc;
-    NPI_REQUIRE(a->T && a->w_label && a->gid && a->dist && a->weight[1] && a->weight[2] && a->y[1] && a->y[2] && a->readout, "tiny_step: null argument");
-    for (int l = 0; l < 3; ++l) NPI_REQUIRE(a->bias[l] && a->batch[l] && a->xp[l] && a->dpre[l] && a->dxa[l], "tiny_step: null layer buffer (layer %d)", l);
-    NPI_REQUIRE(a->d_readout && a->weight_t[1] && a->weight_t[2] && a->dxp[0] && a->dxp[1] && a->partials, "tiny_step: null backward argument");
-    NPI_REQUIRE((((uintptr_t)a->weight[1] | (uintptr_t)a->weight[2] | (uintptr_t)a->weight_t[1] | (uintptr_t)a->weight_t[2]) & 15) == 0,
-                "tiny_step: weights must be 16-byte aligned (bulk copy)");
-    NPI_REQUIRE(w1 && b1 && w2 && b2 && w3 && b3 && y && a1 && a2 && logp && head_workspace, "tiny_step: null head argument");
-    NPI_REQUIRE(head_workspace_bytes >= (int64_t)a->B * DW * (int64_t)sizeof(float), "tiny_step: head workspace too small (npi_head_bwd_workspace_bytes)");
-    if (a->B <= 0) return NPI_OK;
-    const int cap = tn_cap(a->max_graph_nodes);
-    static OncePerDevice cfg;
-    if (cfg.need()) {
-        NPI_CHECK_CUDA(cudaFuncSetAttribute(tiny_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tn_smem_bytes(TN_MAX_NODES)));
-        // two CTAs of ~113 KB per SM need (almost) the whole 228 KB as shared memory
-        NPI_CHECK_CUDA(cudaFuncSetAttribute(tiny_step_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    }
-    TinyHeadArgs hd{w1, b1, w2, b2, w3, b3, training, drop_mask_in, seed, step_dev, sample_ids, sample_id_base, y, loss_scale,
-                    a1, drop_mask_out, a2, logp, (float*)head_workspace};
-    NPI_CHECK_CUDA(launch_dep(tiny_step_kernel, a->B, TN_THREADS, tn_smem_bytes(cap), (cudaStream_t)stream, *a, hd, cap));
     return NPI_OK;
 }

@@ -20,20 +20,10 @@ from . import ops
 # nsys / ncu --nvtx timeline groups by; enabled with NPI_NVTX=1 (a no-op context manager otherwise).
 _NVTX = os.environ.get("NPI_NVTX", "0") == "1"
 _STAMPS = os.environ.get("NPI_STAMPS", "0") == "1"
-# where the index structures of the per-context backward are forked (Engine._fork_index): fwd_start, or one of the hook
-# points fwd_agg0..2 / fwd_topk0..2 / fwd_end
-_INDEX_AT = os.environ.get("NPI_INDEX_AT", "fwd_start")
-# measured: the extra launch in front of filter_adj lengthens the auxiliary chain the next aggregation waits for
-# (0.675 -> 0.705 ms, gpurun_out/r3r) although both sweeps get cheaper -- off
-_FILTER_PACKED = os.environ.get("NPI_FILTER_PACKED", "0") == "1"
 # hub queue / row order of the filtered CSRs inside filter_adj's kernels (three launches on the chain the next aggregation
-# waits for instead of five): "auto" = for small batches only -- 0.247 -> 0.240 ms on RPI2241 (3 k rows), but 0.677 -> 0.684 ms
-# at 215 k rows, where the count kernel's hub rows write their segment lists inside the sweep (gpurun_out/r3s)
-_FILTER_HUB = os.environ.get("NPI_FILTER_HUB", "auto")
+# waits for instead of five) for batches of up to this many rows only -- 0.247 -> 0.240 ms on RPI2241 (3 k rows), but
+# 0.677 -> 0.684 ms at 215 k rows, where the count kernel's hub rows write their segment lists inside the sweep
 SMALL_BATCH_ROWS = 65536
-# projections of fewer rows than this run on the SIMT kernel (NPI_SMALL_GEMM_ROWS): the tcgen05 kernel's fixed cost
-# (tensor-memory allocation, weight staging, barrier set-up: ~9 us) is most of a tiny projection
-_SMALL_GEMM_ROWS = int(os.environ.get("NPI_SMALL_GEMM_ROWS", "0"))
 
 
 class _Range:
@@ -403,29 +393,22 @@ class Engine:
     rows = property(lambda self: [self.cur.rows0 if self.pipelined else None] + self._rows12)
 
     # ------------------------------------------------------------------ batch assembly
-    def load_pairs(self, pairset, first=0, count=None, pair_index=None, slot=None, stage="all"):
+    def load_pairs(self, pairset, first=0, count=None, pair_index=None, slot=None):
         """Device-side batch assembly + GPU extraction of ``count`` pairs of ``pairset``
         (indices first..first+count-1, or pair_index[:count]) into batch slot ``slot`` (default:
-        the current one).  Enqueued on the current stream.  ``stage``: "extract" = batch assembly + the h-hop extraction
-        only, "index" = everything derived from the extracted batch (packed entries, contexts, row lists), "all" = both --
-        the trainer enqueues the two stages on different streams (trainer._enqueue_overlapped)."""
+        the current one), then everything derived from the extracted batch (packed entries, contexts, row lists).
+        Enqueued on the current stream."""
         B = self.B if count is None else int(count)
         if B > self.B:
             raise L.NPIError("batch of %d exceeds engine capacity %d" % (B, self.B))
         g = pairset.graph
         sl = self.cur if slot is None else self.slots[int(slot) & 1]
-        if stage in ("all", "extract"):
-            gp = sl.gptrs if B == self.B else torch.zeros(4, B + 1, dtype=torch.int32, device=self.device)
-            ops.batch_prepare(pair_index, first, B, pairset.pairs, pairset.y, pairset.n_all, pairset.e_all, RATIO,
-                              sl.pairs_b, sl.y_b, gp, sl.edge_ptr, sl.sizes)
-            sl.gp = gp
-            ops.khop_fill(g, sl.pairs_b, B, pairset.h, pairset.max_nodes, gp[0], sl.edge_ptr, sl.gid, sl.dist,
-                          sl.rowptr0, sl.col0, pairset.khop_ws, pairset.num_ctas, overflow=self.overflow)
-            sl.cur_B = B
-            self.graph = g
-            self.dense_x = None
-            if stage == "extract":
-                return
+        gp = sl.gptrs if B == self.B else torch.zeros(4, B + 1, dtype=torch.int32, device=self.device)
+        ops.batch_prepare(pair_index, first, B, pairset.pairs, pairset.y, pairset.n_all, pairset.e_all, RATIO,
+                          sl.pairs_b, sl.y_b, gp, sl.edge_ptr, sl.sizes)
+        sl.gp = gp
+        ops.khop_fill(g, sl.pairs_b, B, pairset.h, pairset.max_nodes, gp[0], sl.edge_ptr, sl.gid, sl.dist,
+                      sl.rowptr0, sl.col0, pairset.khop_ws, pairset.num_ctas, overflow=self.overflow)
         lean = self.ctx_bwd or self.tiny   # forward and backward of layer 1 walk the contexts / the subgraphs: no per-row lists needed
         if not lean:
             if self.pipelined:
@@ -487,7 +470,7 @@ class Engine:
     def _table_grad(self, g, gv, ws_tc=None):
         """conv1.weight gradient through the feature table: table^T . G + label row, last link of the step's chain."""
         ws_tc = self.ws_tn_tc if ws_tc is None else ws_tc
-        if g.num_nodes <= SMALL_TABLE_ROWS and os.environ.get("NPI_TABLE_GRAD", "small") == "small":
+        if g.num_nodes <= SMALL_TABLE_ROWS:
             ops.table_grad(g.table, self.G, g.num_nodes, self.label_part, gv["conv1.weight"], self.ws_tg, K=self.F)
         elif self.t_gemm_tc and self.F <= 256:     # tcgen05: one pass per 128 table columns
             ops.gemm_tn_tc(g.table, self.G, None, g.num_nodes, self.label_part, gv["conv1.weight"], ws_tc, K=self.F)
@@ -514,13 +497,11 @@ class Engine:
             kw.update(d_pool_w=[gv["pool%d.weight" % (l + 1)] for l in range(3)], d_bias=[gv["conv%d.bias" % (l + 1)] for l in range(3)])
         return ops.tiny_args(**kw)
 
-    def _forward_tiny(self, v, step=None):
-        """T = table . conv1.weight, then one launch for conv1..3 + pool1..3 + readout (a CTA per subgraph).  ``step``
-        (training, drop_mask, seed, step_dev, sample_ids, sample_id_base, loss_scale): the same launch goes on with the head,
-        its mean-NLL deltas and the per-subgraph backward (ops.tiny_step)."""
+    def _forward_tiny(self, v):
+        """T = table . conv1.weight, then one launch for conv1..3 + pool1..3 + readout (a CTA per subgraph)."""
         g, W = self.graph, v["conv1.weight"]
         _nvtx_push("forward/per-subgraph")
-        if self.F <= 192 and self.t_gemm_tc and g.num_nodes >= _SMALL_GEMM_ROWS:
+        if self.F <= 192 and self.t_gemm_tc:
             ops.gemm_nn_tc(g.table, None, g.num_nodes, self.F, W, False, self.T)
         else:
             ops.gemm_nn(g.table, None, g.num_nodes, self.F, W, False, self.T)
@@ -529,14 +510,7 @@ class Engine:
         if self.need_backward:
             with self._branch():         # W^T of conv2 / conv3 for the backward's dX = DXA . W^T
                 ops.tiny_transpose(v["conv2.weight"], v["conv3.weight"], self._wt[0], self._wt[1])
-        if step is not None:
-            self._join()                 # the transposed weights are read by the same launch
-            training, drop_mask, seed, step_dev, sample_ids, sample_id_base, loss_scale = step
-            ops.tiny_step(self._tiny_args(v), v["lin1.weight"], v["lin1.bias"], v["lin2.weight"], v["lin2.bias"], v["lin3.weight"],
-                          v["lin3.bias"], training, drop_mask, seed, step_dev, sample_ids, sample_id_base, self.y_b, loss_scale,
-                          self.a1, self.drop_mask, self.a2, self.logp, self.ws_head)
-        else:
-            ops.tiny_fwd(self._tiny_args(v))
+        ops.tiny_fwd(self._tiny_args(v))
         for name in ("fwd_topk0", "fwd_agg1", "fwd_topk1", "fwd_agg2", "fwd_topk2"):
             self._hook(name)
         _nvtx_pop()
@@ -547,9 +521,7 @@ class Engine:
         sz, g = self._size_views, self.graph
         _nvtx_push("backward/per-subgraph")
         ta = self._tiny_args(v, gv)
-        if not getattr(self, "_tiny_step_done", False):      # else: forward() ran the per-subgraph backward in the step kernel
-            ops.tiny_bwd(ta, phases=1)
-        self._tiny_step_done = False
+        ops.tiny_bwd(ta, phases=1)
         self._stamp("bwd_tiny")
         self._hook("bwd_l1")
         with self._branch():
@@ -618,26 +590,18 @@ class Engine:
         """defer_loss: sum the scalar loss on the auxiliary stream (joined by backward(); for callers
         that always run backward() right after -- nothing on the device waits for the loss).
         fuse_head_delta: the head's forward also leaves the mean-NLL deltas and d_readout (one launch instead of two on the
-        chain); backward() with the same loss_scale and no explicit d_logp then skips that phase (NPI_HEAD_FUSE=0: never)."""
+        chain); backward() with the same loss_scale and no explicit d_logp then skips that phase."""
         if self.extract_only:
             raise L.NPIError("this engine was built with extract_only=True")
         B = self.cur_B
         v = params.views()
         sz = self._size_views
         gp = self._gp
-        index_pending = self.ctx_bwd and self._dedup0()
-        if index_pending and _INDEX_AT == "fwd_start":
+        if self.ctx_bwd and self._dedup0():
             self._fork_index()
-            index_pending = False
         self._stamp("fwd_start")
-        if loss_scale is None:
-            loss_scale = 1.0 / B
-        # training step of a small batch: forward, head + deltas and the per-subgraph backward in ONE launch (NPI_TINY_FUSE=1; measured: no faster than the three launches, off by default)
-        step_fused = (self._tiny_on() and fuse_head_delta and compute_loss and self.need_backward
-                      and os.environ.get("NPI_TINY_FUSE", "0") == "1" and os.environ.get("NPI_HEAD_FUSE", "1") != "0")
-        self._tiny_step_done = False
         if self._tiny_on():
-            self._forward_tiny(v, step=(training, drop_mask, seed, step_dev, sample_ids, sample_id_base, loss_scale) if step_fused else None)
+            self._forward_tiny(v)
         for l in (() if self._tiny_on() else range(3)):
             _nvtx_push("forward/conv%d+pool%d" % (l + 1, l + 1))
             W, bias, pw = v["conv%d.weight" % (l + 1)], v["conv%d.bias" % (l + 1)], v["pool%d.weight" % (l + 1)]
@@ -648,7 +612,7 @@ class Engine:
                              self.h[l], self.z[l], self.s[l])
             elif l == 0 and self.dense_x is None:
                 g = self.graph       # project the V-row feature table once, gather 128-wide rows of it
-                if self.F <= 192 and self.t_gemm_tc and g.num_nodes >= _SMALL_GEMM_ROWS:     # tcgen05 + TMA: the table is streamed once, K = F columns
+                if self.F <= 192 and self.t_gemm_tc:     # tcgen05 + TMA: the table is streamed once, K = F columns
                     ops.gemm_nn_tc(g.table, None, g.num_nodes, self.F, W, False, self.T)
                 else:
                     ops.gemm_nn(g.table, None, g.num_nodes, self.F, W, False, self.T)
@@ -661,10 +625,7 @@ class Engine:
             else:
                 x = self.dense_x if l == 0 else self.xp[l - 1]
                 y = self.big if l == 0 else self.ybuf
-                if x.shape[1] == H and l > 0 and self.n_cap[l] < _SMALL_GEMM_ROWS:
-                    ops.gemm_nn(x, sz[l], self.n_cap[l], H, W, False, y)
-                    self._stamp("fwd_gemm%d" % l)
-                elif x.shape[1] == H and l > 0:      # 128-wide pooled features: tcgen05 (3xTF32) projection
+                if x.shape[1] == H and l > 0:      # 128-wide pooled features: tcgen05 (3xTF32) projection
                     ops.gemm_nn_tc(x, sz[l], self.n_cap[l], H, W, False, y)
                     self._stamp("fwd_gemm%d" % l)
                 elif l == 0 and self.F <= 192 and self.t_gemm_tc:      # dense x, row-padded staging buffer
@@ -677,7 +638,7 @@ class Engine:
                                        pipelined=self.pipelined)
             self._hook("fwd_agg%d" % l)
             dd = l == 0 and self._dedup0()      # layer 1 evaluated per context: h/z/s live at the representative rows
-            fused_hub = l < 2 and self.pipelined and (_FILTER_HUB == "1" or (_FILTER_HUB == "auto" and self.n_cap[0] <= SMALL_BATCH_ROWS))
+            fused_hub = l < 2 and self.pipelined and self.n_cap[0] <= SMALL_BATCH_ROWS
             if fused_hub:
                 with self._branch():     # header of the next CSR's hub queue: zeroed next to the top-k, off the chain
                     ops.hub_rows_reset(self.hubq[l + 1])
@@ -687,26 +648,19 @@ class Engine:
             self._hook("fwd_topk%d" % l)
             if l < 2:
                 # filter_adj only feeds the NEXT aggregation: it runs on the auxiliary stream next to
-                # gating/readout and the next layer's projection (joined in the next iteration)
-                # The packed entries {new_id[col], 1/(deg+1)} of this layer come FIRST when they exist: filter_adj's two
-                # sweeps then read one coalesced value per entry instead of chasing col -> new_id (NPI_FILTER_PACKED=0:
-                # the chase).  They are also what the transposed aggregation of this layer reads in the backward pass.
-                packed = None
-                if self.sel is not None and _FILTER_PACKED:
-                    with self._branch():
-                        ops.entry_pack_sel(self.rowptr[l], self.col[l], self.new_id[l], sz[l], self.n_cap[l], self.sel[l])
-                    packed = self.sel[l]
+                # gating/readout and the next layer's projection (joined in the next iteration).  It chases col -> new_id
+                # itself: packing the entries first lengthened the chain the next aggregation waits for (0.675 -> 0.705 ms)
                 with self._branch():
                     if fused_hub:        # hub queue + row order of the filtered CSR come out of filter_adj's own kernels
                         ops.filter_adj(self.rowptr[l], self.col[l], self.perm[l], self.new_id[l], sz[l + 1], self.n_cap[l + 1],
-                                       self.rowptr[l + 1], self.col[l + 1], self.ws_filter, packed_sel=packed,
+                                       self.rowptr[l + 1], self.col[l + 1], self.ws_filter,
                                        hubq=self.hubq[l + 1], hub_e_max=self.e_cap, row_order=self.rows[l + 1])
                     else:
                         ops.filter_adj(self.rowptr[l], self.col[l], self.perm[l], self.new_id[l], sz[l + 1], self.n_cap[l + 1],
-                                       self.rowptr[l + 1], self.col[l + 1], self.ws_filter, packed_sel=packed)
+                                       self.rowptr[l + 1], self.col[l + 1], self.ws_filter)
                         ops.hub_rows_build(self.rowptr[l + 1], sz[l + 1], self.n_cap[l + 1], self.e_cap, self.hubq[l + 1],
                                            None, None, self.rows[l + 1])
-            if self.sel is not None and not (dd and self.ctx_bwd) and not (l < 2 and _FILTER_PACKED):
+            if self.sel is not None and not (dd and self.ctx_bwd):
                 # packed entries for the transposed aggregation of this layer (backward): auxiliary stream
                 with self._branch():
                     ops.entry_pack_sel(self.rowptr[l], self.col[l], self.new_id[l], sz[l], self.n_cap[l], self.sel[l])
@@ -727,10 +681,7 @@ class Engine:
                    self.y_b if compute_loss else None, loss_scale, self.a1, self.drop_mask, self.a2, self.logp,
                    self.loss if compute_loss else None)
         self._head_delta_scale = None
-        if step_fused:               # the step kernel ran the head already
-            self._head_delta_scale = float(loss_scale)
-            self._tiny_step_done = True
-        elif fuse_head_delta and compute_loss and self.need_backward and os.environ.get("NPI_HEAD_FUSE", "1") != "0":
+        if fuse_head_delta and compute_loss and self.need_backward:
             ops.head_fwd_delta(self.readout, B, v["lin1.weight"], v["lin1.bias"], v["lin2.weight"], v["lin2.bias"],
                                v["lin3.weight"], v["lin3.bias"], training, drop_mask, seed, step_dev, sample_ids, sample_id_base,
                                self.y_b, loss_scale, self.a1, self.drop_mask, self.a2, self.logp, self.d_readout, self.ws_head)
@@ -767,7 +718,6 @@ class Engine:
         fused = getattr(self, "_head_delta_scale", None)
         self._head_delta_scale = None
         fused = fused is not None and d_logp is None and fused == float(loss_scale)       # forward() left the deltas already
-        self._tiny_step_done = getattr(self, "_tiny_step_done", False) and fused          # ... and ran the per-subgraph backward on them
         if not fused:
             ops.head_bwd(self.readout, B, v["lin1.weight"], v["lin2.weight"], v["lin3.weight"], self.a1,
                          self.drop_mask if self._last_training else None, self.a2, self.logp, self.y_b, loss_scale, d_logp,
@@ -839,10 +789,7 @@ class Engine:
                         ops.gemm_tn_tc(self.xp[l - 1], dxa, sz[l], self.n_cap[l], None, gv["conv%d.weight" % (l + 1)], self.ws_tn_tc)
                     else:
                         ops.gemm_tn(self.xp[l - 1], dxa, sz[l], self.n_cap[l], H, None, gv["conv%d.weight" % (l + 1)], self.ws_tn)
-                if self.n_cap[l] < _SMALL_GEMM_ROWS:
-                    ops.gemm_nn(dxa, sz[l], self.n_cap[l], H, W, True, self.dxp[l - 1])
-                else:
-                    ops.gemm_nn_tc(dxa, sz[l], self.n_cap[l], H, W, True, self.dxp[l - 1])
+                ops.gemm_nn_tc(dxa, sz[l], self.n_cap[l], H, W, True, self.dxp[l - 1])
                 self._stamp("bwd_gemm%d" % l)
                 d_xp = self.dxp[l - 1]
             elif self.dense_x is not None:
@@ -888,8 +835,6 @@ class Engine:
         fn = self.hooks.get(name)
         if fn is not None:
             fn()
-        if name == _INDEX_AT and self.ctx_bwd and self._dedup0():
-            self._fork_index()
         self._stamp(name)
 
     def _stamp(self, name):

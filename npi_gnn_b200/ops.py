@@ -156,12 +156,10 @@ def filter_adj_workspace_bytes(n_new_max):
     return L.query("npi_filter_adj_workspace_bytes", _i32(n_new_max))
 
 
-def filter_adj(rowptr, col, perm, new_id, nnew_dev, nnew_host, rowptr_out, col_out, ws, packed_sel=None, hubq=None, hub_e_max=0,
-               row_order=None):
-    """packed_sel: entry_pack_sel of the same CSR and selection (one coalesced load per entry instead of col -> new_id).
-    hubq / row_order: hub queue and binned row order of the NEW CSR built on the way (header zeroed by hub_rows_reset)."""
+def filter_adj(rowptr, col, perm, new_id, nnew_dev, nnew_host, rowptr_out, col_out, ws, hubq=None, hub_e_max=0, row_order=None):
+    """hubq / row_order: hub queue and binned row order of the NEW CSR built on the way (header zeroed by hub_rows_reset)."""
     L.call("npi_filter_adj", L.ptr(rowptr), L.ptr(col), L.ptr(perm), L.ptr(new_id), L.ptr(nnew_dev), _i32(nnew_host),
-           L.ptr(rowptr_out), L.ptr(col_out), L.ptr(packed_sel), L.ptr(hubq), _i64(hub_e_max), L.ptr(row_order),
+           L.ptr(rowptr_out), L.ptr(col_out), L.ptr(hubq), _i64(hub_e_max), L.ptr(row_order),
            L.ptr(ws), _i64(ws.numel() * ws.element_size()), _s())
 
 
@@ -415,15 +413,6 @@ def tiny_weight_grads(table, F, gid, dist, dxa1, n0_dev, n0_host, d_w1, ws, x1=N
            L.ptr(x1), L.ptr(dxa2), L.ptr(n1_dev), _i32(n1_host), L.ptr(d_w2),
            L.ptr(x2), L.ptr(dxa3), L.ptr(n2_dev), _i32(n2_host), L.ptr(d_w3),
            L.ptr(ws), _i64(ws.numel() * ws.element_size()), _s())
-
-
-def tiny_step(args, w1, b1, w2, b2, w3, b3, training, drop_mask_in, seed, step_dev, sample_ids, sample_id_base, y, loss_scale,
-              a1, drop_mask_out, a2, logp, head_ws):
-    """tiny_fwd + head_fwd_delta + tiny_bwd(phases=1) in one launch (training step of a small batch)."""
-    L.call("npi_tiny_step", C.byref(args), L.ptr(w1), L.ptr(b1), L.ptr(w2), L.ptr(b2), L.ptr(w3), L.ptr(b3),
-           _i32(1 if training else 0), L.ptr(drop_mask_in), _u64(seed), L.ptr(step_dev), L.ptr(sample_ids), _i32(sample_id_base),
-           L.ptr(y), _f32(loss_scale), L.ptr(a1), L.ptr(drop_mask_out), L.ptr(a2), L.ptr(logp),
-           L.ptr(head_ws), _i64(head_ws.numel() * head_ws.element_size()), _s())
 
 
 def tiny_fwd(args):

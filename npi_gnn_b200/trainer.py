@@ -55,19 +55,6 @@ def shard_of_batch(order, per_rank_batch, world_size, rank, gb, cost=None):
     return idx[mine], len(idx)
 
 
-PREFETCH_POINTS = ("start", "fwd_agg0", "fwd_topk0", "fwd_agg1", "fwd_topk1", "fwd_agg2", "fwd_topk2", "fwd_end", "bwd_l1")
-
-
-_DEBUG_NO_PREFETCH = os.environ.get("NPI_DEBUG_NO_PREFETCH", "0") == "1"
-_KHOP_INLINE = os.environ.get("NPI_KHOP_INLINE", "0") == "1"
-# NPI_STREAM_PRIORITY=1: the captured step runs its critical chain on a HIGH-priority stream (kernel nodes inherit the
-# priority of the stream they were captured on), the extraction stream and the engine's auxiliary / index streams keep the
-# default.  Measured (tools/step_timeline.py, gpurun_out/r3f): the chain's GEMMs no longer queue behind the weight-gradient
-# GEMMs of the auxiliary stream (37 -> 19 us, 57 -> 29 us), but those then delay the NEXT links by the same amount --
-# the step is work-bound, not order-bound (0.6915 vs 0.6834 ms).  Off by default.
-_PRIO = -1 if os.environ.get("NPI_STREAM_PRIORITY", "0") == "1" else 0
-
-
 class Trainer:
     def __init__(self, pairset, batch_size=200, lr=1e-3, weight_decay=1e-3, seed=0, params=None,
                  world_size=1, rank=0, use_cuda_graph=True, allreduce=None, order=None, exchange=None, balance=True):
@@ -131,14 +118,6 @@ class Trainer:
         self.use_graph = bool(use_cuda_graph)
         self._graphs = {}                 # slot parity -> (fwd/bwd[/update] graph, update graph or None)
         self._side = None                 # side stream of the prefetching extraction
-        # where in the step the next batch's extraction is forked.  Its 200 fat CTAs (1024 threads, 76 KB of
-        # shared memory) take whole SMs for ~100 us: forked at the start they squeeze the first aggregation
-        # (the most bandwidth-hungry kernel of the step); forked behind it they sit next to the per-graph
-        # top-k kernels, which are latency bound.  Measured over the hook points (profiles/r03a): 234 k
-        # subgraphs/s at "start", 242 k at "fwd_agg0", 237-240 k anywhere later in the forward pass.
-        self.prefetch_at = os.environ.get("NPI_PREFETCH_AT", "fwd_agg0")
-        if self.prefetch_at not in PREFETCH_POINTS:
-            raise L.NPIError("NPI_PREFETCH_AT=%r: expected one of %s" % (self.prefetch_at, ", ".join(PREFETCH_POINTS)))
         self._slot_gb = [None, None]      # which global batch each engine slot currently holds
         self.kernel_launches_per_step = None
 
@@ -165,9 +144,9 @@ class Trainer:
         return n0, e0, mx
 
     # ------------------------------------------------------------------ one step
-    def _enqueue_extract(self, count, slot, stage="all"):
+    def _enqueue_extract(self, count, slot):
         """Batch assembly + GPU extraction (+ by-serial index) of the pairs in pair_index[slot]."""
-        self.engine.load_pairs(self.ps, count=count, pair_index=self.pair_index[slot], slot=slot, stage=stage)
+        self.engine.load_pairs(self.ps, count=count, pair_index=self.pair_index[slot], slot=slot)
 
     def _enqueue_compute(self, global_count):
         """Forward + loss + backward on the engine's current slot; gradients (pre-scaled by
@@ -223,25 +202,18 @@ class Trainer:
         nxt = 1 - self.engine.slot
 
         def fork():
-            if _DEBUG_NO_PREFETCH and torch.cuda.is_current_stream_capturing():
-                return                  # timing experiments only: the captured step without its side stream (stale batches)
-            if _KHOP_INLINE:            # the extraction's 1024-thread CTAs on the main stream, the small index kernels beside it
-                self._enqueue_extract(self.B, nxt, stage="extract")
             self._side.wait_stream(torch.cuda.current_stream(self.device))
             with torch.cuda.stream(self._side):
-                self._enqueue_extract(self.B, nxt, stage="index" if _KHOP_INLINE else "all")
-        at = self.prefetch_at
-        if at == "start":
-            fork()
+                self._enqueue_extract(self.B, nxt)
+        # the extraction's 200 fat CTAs (1024 threads, 76 KB of shared memory) take whole SMs for ~100 us: forked behind the
+        # first aggregation, the most bandwidth-hungry kernel of the step, they sit next to the latency-bound per-graph top-k
+        # kernels (242 k subgraphs/s, against 234 k forked at the start of the step and 237-240 k later in the forward pass)
+        self.engine.hooks = {"fwd_agg0": fork}
+        try:
             self._enqueue_compute(GB)
-        else:                 # fork later in the step (engine hook): the extraction's 200 fat CTAs stay out of the way of
-            self.engine.hooks = {at: fork}          # the first, bandwidth-hungry kernels
-            try:
-                self._enqueue_compute(GB)
-            finally:
-                self.engine.hooks = {}
-        if not (_DEBUG_NO_PREFETCH and torch.cuda.is_current_stream_capturing()):
-            main.wait_stream(self._side)
+        finally:
+            self.engine.hooks = {}
+        main.wait_stream(self._side)
 
     def _state(self):
         return (self.params.flat, self.m, self.v, self.step_dev, self.loss_acc)
@@ -253,7 +225,8 @@ class Trainer:
         GB = self.B * self.world_size
         if self._side is None:
             self._side = torch.cuda.Stream(device=self.device)
-        s = torch.cuda.Stream(device=self.device, priority=_PRIO)
+        # default priority: a high-priority chain only made the auxiliary stream's GEMMs delay later links (0.6915 vs 0.6834 ms)
+        s = torch.cuda.Stream(device=self.device)
         s.wait_stream(torch.cuda.current_stream(self.device))
         keep = [t.clone() for t in self._state()]
         self.engine.use_slot(slot)
@@ -439,7 +412,7 @@ class Scorer:
     def _capture(self, slot):
         if self._side is None:
             self._side = torch.cuda.Stream(device=self.device)
-        s = torch.cuda.Stream(device=self.device, priority=_PRIO)
+        s = torch.cuda.Stream(device=self.device)
         s.wait_stream(torch.cuda.current_stream(self.device))
         self.engine.use_slot(slot)
         with torch.cuda.stream(s):                       # warm-up outside capture (lazy kernel attributes)

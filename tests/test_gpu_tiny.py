@@ -216,9 +216,7 @@ def test_tiny_scorer_matches_per_layer_scorer():
 @pytest.mark.parametrize("tiny", [True, False])
 def test_fused_head_delta_is_bit_identical(tiny):
     """forward(fuse_head_delta=True) followed by backward() gives the same bits as the separate calls: head forward +
-    mean-NLL deltas in one launch (both engine paths), and on the per-subgraph path forward + head + deltas + per-subgraph
-    backward in ONE launch (npi_tiny_step)."""
-    import os
+    mean-NLL deltas in one launch (both engine paths)."""
     from npi_gnn_b200 import _lib
     from npi_gnn_b200.engine import Engine, FlatParams
     B = 200
@@ -227,20 +225,14 @@ def test_fused_head_delta_is_bit_identical(tiny):
     eng = Engine(g.F, B, n0, e0, mx, device="cuda", graph=g, tiny=tiny, contexts=False)
     eng.load_pairs(ps, 0, B)
     out = []
-    variants = [(False, "0"), (True, "0")] + ([(True, "1")] if tiny else [])
-    for fuse, step_env in variants:
+    for fuse in (False, True):
         grads = FlatParams(g.F, "cuda")
-        before = {k: _lib.CALL_COUNTS.get(k, 0) for k in ("npi_head_fwd_delta", "npi_tiny_step")}
-        os.environ["NPI_TINY_FUSE"] = step_env
-        try:
-            logp = eng.forward(params, training=True, seed=7, compute_loss=True, fuse_head_delta=fuse).clone()
-            eng.backward(params, grads)
-        finally:
-            os.environ.pop("NPI_TINY_FUSE", None)
+        before = _lib.CALL_COUNTS.get("npi_head_fwd_delta", 0)
+        logp = eng.forward(params, training=True, seed=7, compute_loss=True, fuse_head_delta=fuse).clone()
+        eng.backward(params, grads)
         torch.cuda.synchronize()
-        used = {k: _lib.CALL_COUNTS.get(k, 0) - before[k] for k in before}
-        step = fuse and tiny and step_env == "1"
-        assert used == {"npi_head_fwd_delta": 1 if (fuse and not step) else 0, "npi_tiny_step": 1 if step else 0}, used
+        used = _lib.CALL_COUNTS.get("npi_head_fwd_delta", 0) - before
+        assert used == (1 if fuse else 0), used
         out.append((logp, grads.flat.clone(), eng.d_readout.clone(), float(eng.loss[0])))
     for o in out[1:]:
         assert torch.equal(out[0][0], o[0]) and torch.equal(out[0][2], o[2]) and torch.equal(out[0][1], o[1])

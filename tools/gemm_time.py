@@ -22,19 +22,18 @@ res = []
 for M in (128, 148 * 128, 53790, 107579, 4 * 107579):
     A = torch.randn(M, 128, device=dev)
     C = torch.empty(M, 128, device=dev)
-    for legacy in (0, 2):
-        ts = []
-        for i in range(12):
-            flush.zero_()
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record()
-            ops.gemm_nn_tc(A, None, M, 128, W, i & 1, C, single_pass=legacy)
-            e1.record()
-            torch.cuda.synchronize()
-            ts.append(e0.elapsed_time(e1) * 1e3)
-        us = float(np.median(ts[2:]))
-        gbs = 2 * M * 512 / us / 1e3
-        res.append(dict(M=M, kernel="register-staged (A/B partner)" if legacy else "tma + tmem weights", us=us, alg_GBps=gbs, frac=gbs / peak))
-        print(res[-1], flush=True)
+    ts = []
+    for i in range(12):
+        flush.zero_()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        ops.gemm_nn_tc(A, None, M, 128, W, i & 1, C)
+        e1.record()
+        torch.cuda.synchronize()
+        ts.append(e0.elapsed_time(e1) * 1e3)
+    us = float(np.median(ts[2:]))
+    gbs = 2 * M * 512 / us / 1e3
+    res.append(dict(M=M, us=us, alg_GBps=gbs, frac=gbs / peak))
+    print(res[-1], flush=True)
 if len(sys.argv) > 1:
     json.dump(res, open(sys.argv[1], "w"), indent=1)

@@ -29,7 +29,7 @@ MAP = {
     "npi_ctx_finish": [("ctx_finish_kernel", 1, {0: 0})],
     "npi_pool_bwd": [("pool_bwd_kernel", 2, {0: 0, 2: 1}), ("pool_bwd_kernel", 3, {0: 0, 2: 1, 4: 2})],      # odd occurrences = the partial reduce (phase 2)
     "npi_pool_gate_readout": [("gate_readout_kernel", 3, {0: 0, 2: 1, 4: 2})],   # odd occurrences = the readout combine (phase 2)
-    "npi_gemm_nn_tc": [("tc::gemm_tc_tma_kernel", 5, {0: 0, 1: 1, 2: 2, 3: 3, 4: 4}), ("tc::gemm_tc_ws_kernel", 4, {0: 0, 1: 1, 2: 2, 3: 3})],
+    "npi_gemm_nn_tc": [("tc::gemm_tc_tma_kernel", 5, {0: 0, 1: 1, 2: 2, 3: 3, 4: 4})],
     "npi_gemm_tn_tc": [("tc::gemm_tn_tc_kernel", 2, {0: 0, 1: 1})],
     "npi_gid_reduce": [("gid_reduce_kernel", 1, {0: 0})],
     "npi_khop_fill": [("khop_kernel<1, 1>", 1, {0: 0})],
