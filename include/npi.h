@@ -578,6 +578,41 @@ int npi_group_topk(const float* scores, const int32_t* group, int64_t n, int32_t
                    int32_t* out_pos, float* out_score, int32_t* out_count, int32_t* status,
                    void* workspace, int64_t workspace_bytes, npi_stream_t stream);
 
+/* Filtered rank of every held-out interaction among its group's candidates (csrc/grouprank.cu): MRR, Hits@K and the
+ * per-group ROC AUC of a scoring sweep -- for each RNA, where its true partners rank among all the proteins it could
+ * pair with, and for each protein among its RNAs (the question of the reference's src/case_study.py and
+ * src/case_study_negativeSample.py, and the link-prediction reading of them).
+ *  - inputs: scores float32[n]; labels int32[n], 1 = query (a held-out interaction), 0 = competitor (a sampled negative
+ *    or an unlabelled candidate pair); group int32[n], 0 <= group < num_groups; hits_k: HOST array of n_hits int32,
+ *    1 <= n_hits <= 8, every K >= 1.
+ *  - per query i of group g: above_i = competitors of g with a score strictly greater than s_i, tied_i = competitors of g
+ *    with a score equal to s_i.  Scores compare as rank_key does: -0.0 and +0.0 are equal, +-inf are ordinary scores.
+ *    The other queries of g never compete (the filtered setting).
+ *  - rank_i = above_i + tied_i / 2 + 1, the mean of the optimistic rank above + 1 and the pessimistic rank
+ *    above + tied + 1 (ties get half credit, as in OGB's MRR).  Comparisons use 2 rank = 2 above + tied + 2 in integers;
+ *    1 / rank is computed in fp64.
+ *  - per group (device, num_groups entries each): n_pos, n_neg (int32); twice_u (int64) = sum over the queries of g of
+ *    2 (n_neg[g] - above_i - tied_i) + tied_i.  twice_u / (2 n_pos n_neg) equals sklearn's roc_auc_score on the group's
+ *    items.
+ *  - summary (device int64[3 + n_hits]) = {n_queries, n_unranked, n_groups_scored, hits[0 .. n_hits-1]}: n_queries =
+ *    queries whose group has at least one competitor (the ranked queries); n_unranked = queries in groups without a
+ *    competitor, left out of MRR and Hits (their counts are 0 / 0); n_groups_scored = groups with both classes;
+ *    hits[h] = ranked queries with 2 above + tied + 2 <= 2 K_h.  sum_rr (device double[1]) = sum of 1 / rank over the
+ *    ranked queries.
+ *  - above / tied (nullable each, int32[n], input order): the counts of every query, -1 for competitors.
+ *  - status (int32[1]): bit 0 = a NaN score, bit 1 = a label other than 0 or 1, bit 2 = a group id out of range; when any
+ *    bit is set the other outputs are meaningless.
+ * 1 <= n < 2^31, 1 <= num_groups < 2^24.  Every output is bit-identical on reruns and under any permutation of the input
+ * (the per-item outputs follow their items): each tie run of (group, score) contributes one term npos_run / rank at its
+ * run end, whose sorted index does not depend on the input order; no float atomics.  21 + 3 *
+ * npi_sort_passes(ceil(log2 num_groups)) launches (24 up to 512 groups, 27 up to 262,144, else 30), no host
+ * synchronisation, capturable in a CUDA graph; the workspace needs no initialisation. */
+int64_t npi_group_rank_workspace_bytes(int64_t n_max, int32_t num_groups);
+int npi_group_rank(const float* scores, const int32_t* labels, const int32_t* group, int64_t n, int32_t num_groups,
+                   const int32_t* hits_k, int32_t n_hits, int32_t* n_pos, int32_t* n_neg, int64_t* twice_u,
+                   int64_t* summary, double* sum_rr, int32_t* above, int32_t* tied, int32_t* status,
+                   void* workspace, int64_t workspace_bytes, npi_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------
  * node2vec on the GPU (the stage that produces the embedding columns of the feature table).
  * Replaces node2vec-master/src/node2vec.py and main.py:78-92 of the reference over a CSR with

@@ -9,7 +9,7 @@ All compute goes through the C ABI of libnpi.so (include/npi.h); nothing falls b
 from ._lib import NPIError  # noqa: F401
 from .graph import BipartiteGraph, PairSet  # noqa: F401
 from .engine import Engine, FlatParams  # noqa: F401
-from .trainer import Trainer, Scorer, metrics, rank_metrics, top_k_by_group  # noqa: F401
+from .trainer import Trainer, Scorer, group_rank_metrics, metrics, rank_metrics, top_k_by_group  # noqa: F401
 from .nn import Net_1, SAGEConv, TopKPooling, global_max_pool, global_mean_pool  # noqa: F401
 from .data import (Data, Batch, DataLoader, EnclosingSubgraphDataset,  # noqa: F401
                    LncRNA_Protein_Interaction_dataset_1hop_1220_InMemory)

@@ -21,6 +21,17 @@ int launch_gemm_tn_reduce(const float* part, int G, int ktiles, int K, const flo
 // out[i] = sum of in[0..i), *total (nullable) = sum of all n; tile_sums: >= ceil(n / 4096) ints of scratch (sort.cu)
 int launch_excl_scan_i32(const int32_t* in, int64_t n, int32_t* out, int32_t* total, int32_t* tile_sums, cudaStream_t st);
 
+// Key bits of a radix sort by group id: ceil(log2 num_groups), at least 1 (topk.cu, grouprank.cu).
+inline int group_bits(int32_t num_groups) {
+    int b = 1;
+    while (((int64_t)1 << b) < num_groups) ++b;
+    return b;
+}
+// gptr[g] = first of the n group-sorted keys >= g, for g = 0 .. num_groups (one launch); *status = OR of the ntiles
+// per-tile status bits 0..2 (topk.cu)
+int launch_group_bounds(const uint32_t* keys, int64_t n, int32_t num_groups, const int32_t* tile_status, int ntiles,
+                        int32_t* gptr, int32_t* status, cudaStream_t st);
+
 // cudaFuncSetAttribute(MaxDynamicSharedMemorySize) is a PER-DEVICE attribute: "configured once" flags are
 // kept per device (a process that drives a second GPU configures the kernels there too).
 struct OncePerDevice {
@@ -150,8 +161,8 @@ __device__ __forceinline__ int block_excl_scan(int v, int* sh, int* total) {
     return inc - v + sh[w];
 }
 
-// Orderable key of a score for the ranking entry points (rank.cu, topk.cu): ascending key = descending score, -0.0 and
-// +0.0 one key, +-inf ordinary scores.
+// Orderable key of a score for the ranking entry points (rank.cu, topk.cu, grouprank.cu): ascending key = descending
+// score, -0.0 and +0.0 one key, +-inf ordinary scores.
 __device__ __forceinline__ uint32_t rank_key(float s) {
     uint32_t u = __float_as_uint(s);
     if (s == 0.0f) u = 0u;                                   // -0.0 and +0.0 are one threshold

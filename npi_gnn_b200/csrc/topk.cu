@@ -53,12 +53,6 @@ static int64_t topk_layout(int64_t n, int32_t num_groups, char* ws, TopkWs* w) {
     return off;
 }
 
-static int group_bits(int32_t num_groups) {
-    int b = 1;
-    while (((int64_t)1 << b) < num_groups) ++b;
-    return b;
-}
-
 __global__ void __launch_bounds__(KK_THREADS) topk_key_kernel(const float* __restrict__ scores, const int32_t* __restrict__ group,
                                                               int64_t n, int32_t num_groups, uint32_t* __restrict__ keys,
                                                               int32_t* __restrict__ vals, int32_t* __restrict__ tile_status) {
@@ -97,9 +91,17 @@ __global__ void __launch_bounds__(TB_THREADS) topk_bounds_kernel(const uint32_t*
     if (blockIdx.x == 0) {
         int st = 0;
         for (int t = threadIdx.x; t < ntiles; t += TB_THREADS) st |= tile_status[t];
-        st = (__syncthreads_or(st & 1) ? 1 : 0) | (__syncthreads_or(st & 2) ? 2 : 0);
+        st = (__syncthreads_or(st & 1) ? 1 : 0) | (__syncthreads_or(st & 2) ? 2 : 0) | (__syncthreads_or(st & 4) ? 4 : 0);
         if (threadIdx.x == 0) *status = st;
     }
+}
+
+int launch_group_bounds(const uint32_t* keys, int64_t n, int32_t num_groups, const int32_t* tile_status, int ntiles,
+                        int32_t* gptr, int32_t* status, cudaStream_t st) {
+    topk_bounds_kernel<<<(int)(((int64_t)num_groups + TB_THREADS) / TB_THREADS), TB_THREADS, 0, st>>>(keys, n, num_groups, tile_status,
+                                                                                                     ntiles, gptr, status);
+    NPI_CHECK_LAUNCH();
+    return NPI_OK;
 }
 
 __global__ void __launch_bounds__(TK_THREADS) group_topk_kernel(const float* __restrict__ scores, const int32_t* __restrict__ pos_sorted,
@@ -241,9 +243,8 @@ extern "C" int npi_group_topk(const float* scores, const int32_t* group, int64_t
     const bool in_b = npi_sort_passes(bits) & 1;
     const uint32_t* keys = in_b ? w.keys_b : w.keys_a;
     const int32_t* vals = in_b ? w.vals_b : w.vals_a;
-    topk_bounds_kernel<<<(int)(((int64_t)num_groups + TB_THREADS) / TB_THREADS), TB_THREADS, 0, st>>>(keys, n, num_groups, w.tile_status,
-                                                                                                     ntiles, w.gptr, status);
-    NPI_CHECK_LAUNCH();
+    rc = launch_group_bounds(keys, n, num_groups, w.tile_status, ntiles, w.gptr, status, st);
+    if (rc != NPI_OK) return rc;
     static OncePerDevice once;
     if (once.need())
         NPI_CHECK_CUDA(cudaFuncSetAttribute(group_topk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TK_STAGE * 4));

@@ -503,6 +503,34 @@ def group_topk(scores, group, num_groups, k, out_pos, out_score, out_count, stat
            count_as=None if passes == 2 else "npi_group_topk/%dpass" % passes)
 
 
+def group_rank_workspace_bytes(n_max, num_groups):
+    return L.query("npi_group_rank_workspace_bytes", _i64(n_max), _i32(num_groups))
+
+
+def group_rank(scores, labels, group, num_groups, hits_k, n_pos, n_neg, twice_u, summary, sum_rr, status, ws, above=None, tied=None):
+    """Filtered rank of every query (label 1) among the competitors (label 0) of its group (include/npi.h npi_group_rank):
+    float32 ``scores``, int32 ``labels`` / ``group`` ids; ``hits_k`` a host sequence of 1..8 cut-offs K.  Outputs: n_pos /
+    n_neg int32 and twice_u int64 [num_groups]; summary int64[3 + len(hits_k)] = {n_queries, n_unranked, n_groups_scored,
+    hits...}; sum_rr float64[1]; status int32[1] (bit 0 NaN score, bit 1 label not 0/1, bit 2 group id out of range);
+    optional above / tied int32[n] in input order (-1 for competitors)."""
+    n = scores.numel()
+    if labels.numel() != n or group.numel() != n or scores.dtype != torch.float32 or labels.dtype != torch.int32 \
+            or group.dtype != torch.int32 or not (scores.is_contiguous() and labels.is_contiguous() and group.is_contiguous()):
+        raise L.NPIError("group_rank: contiguous float32 scores, int32 labels and int32 group ids of equal length expected")
+    G, nh = int(num_groups), len(hits_k)
+    outs = ((n_pos, torch.int32, G), (n_neg, torch.int32, G), (twice_u, torch.int64, G), (summary, torch.int64, 3 + nh),
+            (sum_rr, torch.float64, 1), (status, torch.int32, 1), (above, torch.int32, n), (tied, torch.int32, n))
+    for t, dt, size in outs:
+        if t is not None and (t.dtype != dt or not t.is_contiguous() or t.numel() < size):
+            raise L.NPIError("group_rank: outputs of the wrong dtype or holding too few entries (num_groups = %d, n = %d, %d hits)"
+                             % (G, n, nh))
+    ks = (_i32 * max(nh, 1))(*[int(k) for k in hits_k])
+    passes = L.query("npi_sort_passes", _i32(max(1, (G - 1).bit_length())))
+    L.call("npi_group_rank", L.ptr(scores), L.ptr(labels), L.ptr(group), _i64(n), _i32(G), ks, _i32(nh), L.ptr(n_pos),
+           L.ptr(n_neg), L.ptr(twice_u), L.ptr(summary), L.ptr(sum_rr), L.ptr(above), L.ptr(tied), L.ptr(status), L.ptr(ws),
+           _i64(ws.numel() * ws.element_size()), _s(), count_as=None if passes == 2 else "npi_group_rank/%dpass" % passes)
+
+
 # ----------------------------------------------------------------------------- operator-API helpers
 def filter_edges_coo(edge_index, new_id, out, count_dev):
     E = edge_index.shape[1]

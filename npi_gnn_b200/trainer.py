@@ -527,6 +527,37 @@ class Scorer:
             out[name] = dict(partner=partner, prob=r["score"], count=r["count"])
         return out
 
+    def partner_ranks(self, hits=(1, 3, 10)):
+        """Where every held-out interaction ranks among its node's candidates, per RNA and per protein, from ONE sweep of
+        ``probabilities()`` and the pair labels: ``group_rank_metrics`` with the pairs grouped by their RNA ("rna") and by
+        their protein ("protein"), node serials as group ids.  Pairs with label 1 are the queries, pairs with label 0
+        their competitors; returns {"rna": ..., "protein": ...} of group_rank_metrics dicts (MRR, Hits@K, per-node AUC).
+
+        Intended use: build the graph with the test pairs masked, then score one pair set made of the test positives
+        (label 1), the test negatives (label 0) and ``BipartiteGraph.candidate_pairs()`` (label 0)::
+
+            cand = g.candidate_pairs()
+            pairs = np.concatenate([test_pos, test_neg, cand])
+            y = np.concatenate([np.ones(len(test_pos)), np.zeros(len(test_neg)), np.zeros(len(cand))])
+            Scorer(PairSet(g, pairs, y), params).partner_ranks()
+
+        Honours an ``index`` view.  The result does not depend on the order of the pairs.  With world_size > 1 every
+        rank's shard is gathered (torch.distributed must be initialised) and every rank computes the same, bit-identical
+        result over all pairs."""
+        from . import dist as D
+        ks = _hits_cutoffs(hits, "partner_ranks")
+        if self.world_size > 1 and not D.dist.is_initialized():
+            raise L.NPIError("Scorer.partner_ranks with world_size > 1 needs an initialised torch.distributed process group")
+        probs = self.probabilities()
+        if self.world_size > 1:
+            probs = D.gather_shards(probs, self.P)
+        pairs, labels = self.ps.pairs, self.ps.y
+        if self.index is not None:
+            idx = torch.from_numpy(self.index).to(self.device)
+            pairs, labels = pairs[idx], labels[idx]
+        return {name: group_rank_metrics(probs, labels, pairs[:, own].contiguous(), self.ps.graph.num_nodes, ks)
+                for name, own in (("rna", 0), ("protein", 1))}
+
 
 def metrics(TP, FN, TN, FP):
     """Accuracy, Precision, Sensitivity, Specificity, MCC exactly as src/methods.py:107-127."""
@@ -606,3 +637,73 @@ def top_k_by_group(scores, group, num_groups, k):
     if st & 2:
         raise L.NPIError("top_k_by_group: group id out of range [0, %d)" % G)
     return dict(pos=pos, score=score, count=count)
+
+
+def _hits_cutoffs(hits, who):
+    """The Hits@K cut-offs as a tuple of ints: 1..8 of them, every K in 1 .. 2^31 - 1 (ValueError otherwise)."""
+    try:
+        ks = tuple(int(k) for k in hits)
+    except (TypeError, ValueError):
+        raise ValueError("%s: hits must be a sequence of integer cut-offs K, got %r" % (who, hits)) from None
+    if not 1 <= len(ks) <= 8 or any(not 1 <= k < 1 << 31 for k in ks):
+        raise ValueError("%s: hits = %r, expected 1 to 8 cut-offs K >= 1" % (who, hits))
+    return ks
+
+
+def group_rank_metrics(scores, labels, group, num_groups, hits=(1, 3, 10), per_item=False):
+    """Filtered ranking of CUDA float32 ``scores`` per group of int32 ``group`` ids (0 <= id < num_groups), in ONE call of
+    npi_group_rank and one synchronising read.  Items with ``labels`` 1 are queries (held-out interactions), items with
+    label 0 their competitors (sampled negatives, unlabelled candidates).  Each query is ranked among the competitors of
+    its group only, the group's other queries left out: rank = above + tied / 2 + 1 (ties get half credit, -0.0 and +0.0
+    tie).  Returns dict:
+      mrr              mean of 1 / rank over the ranked queries (those whose group has a competitor)
+      hits             {K: fraction of the ranked queries with rank <= K}
+      n_queries, n_unranked, n_groups_scored   ranked queries, queries of groups without a competitor, groups with both
+                       classes
+      auc_macro        fp64 mean of the defined per-group ROC AUCs (NaN if there is none)
+      n_pos, n_neg     int32 [num_groups] device tensors; twice_u int64 [num_groups], the exact 2 x Mann-Whitney U
+      auc              float64 [num_groups] device tensor, twice_u / (2 n_pos n_neg), NaN without both classes
+      above, tied      (per_item=True) int32 [n] device tensors in input order, -1 for competitors
+    NaN scores, labels other than 0/1 or group ids out of range raise NPIError.  A bad ``hits`` (1 to 8 cut-offs K >= 1)
+    or num_groups < 1 raises ValueError before the device is touched; no ranked query raises ValueError (MRR is
+    undefined)."""
+    ks = _hits_cutoffs(hits, "group_rank_metrics")
+    G = int(num_groups)
+    if G < 1:
+        raise ValueError("group_rank_metrics: num_groups = %d, expected >= 1" % G)
+    L.require_cuda(scores, labels, group)
+    scores, labels, group = (t.reshape(-1).contiguous() for t in (scores, labels, group))
+    n, nh, dev = scores.numel(), len(ks), scores.device
+    res = torch.zeros(16, dtype=torch.int64, device=dev)    # summary[3 + nh] | sum_rr | sum of defined AUCs | status
+    summary = res[:3 + nh]
+    sum_rr, auc_sum = res[11:12].view(torch.float64), res[12:13].view(torch.float64)
+    status = res[13:14].view(torch.int32)[:1]
+    n_pos = torch.empty(G, dtype=torch.int32, device=dev)
+    n_neg = torch.empty(G, dtype=torch.int32, device=dev)
+    twice_u = torch.empty(G, dtype=torch.int64, device=dev)
+    above = torch.empty(n, dtype=torch.int32, device=dev) if per_item else None
+    tied = torch.empty(n, dtype=torch.int32, device=dev) if per_item else None
+    ws = torch.empty(ops.group_rank_workspace_bytes(max(n, 1), G), dtype=torch.uint8, device=dev)
+    ops.group_rank(scores, labels, group, G, ks, n_pos, n_neg, twice_u, summary, sum_rr, status, ws, above, tied)
+    both = (n_pos > 0) & (n_neg > 0)
+    auc = torch.where(both, twice_u.double() / (2.0 * n_pos.double() * n_neg.double()), float("nan"))
+    auc_sum.copy_(torch.where(both, auc, 0.0).sum().reshape(1))
+    h = res.cpu()
+    st = int(h[13:14].view(torch.int32)[0])
+    if st & 1:
+        raise L.NPIError("group_rank_metrics: NaN score")
+    if st & 2:
+        raise L.NPIError("group_rank_metrics: label other than 0 or 1")
+    if st & 4:
+        raise L.NPIError("group_rank_metrics: group id out of range [0, %d)" % G)
+    nq, nu, ng = (int(v) for v in h[:3])
+    if nq == 0:
+        raise ValueError("group_rank_metrics: no query has a competitor in its group: MRR is not defined in that case")
+    f = h[11:13].view(torch.float64)
+    out = dict(mrr=float(f[0]) / nq, hits={k: int(h[3 + i]) / nq for i, k in enumerate(ks)},
+               n_queries=nq, n_unranked=nu, n_groups_scored=ng,
+               auc_macro=float(f[1]) / ng if ng else float("nan"),
+               n_pos=n_pos, n_neg=n_neg, twice_u=twice_u, auc=auc)
+    if per_item:
+        out.update(above=above, tied=tied)
+    return out
