@@ -613,6 +613,36 @@ int npi_group_rank(const float* scores, const int32_t* labels, const int32_t* gr
                    int64_t* summary, double* sum_rr, int32_t* above, int32_t* tied, int32_t* status,
                    void* workspace, int64_t workspace_bytes, npi_stream_t stream);
 
+/* Input attribution of scored pairs (csrc/attrib.cu): why the model scores a pair as it does, in terms of the nodes and
+ * the input features of its enclosing subgraph -- the follow-up question to the case-study ranking of the reference's
+ * src/case_study.py and src/case_study_negativeSample.py (which proteins does this lncRNA interact with, and why).
+ *  - for a pair p let t(p) be its target: logp[p, c] for a class c, or p_c = exp(logp[p, c]).  The network runs in
+ *    evaluation mode (no dropout), exactly the forward the scoring sweep runs.  Every discrete decision is the one that
+ *    forward took (top-k selections, ReLU masks, the row global_max_pool routes to): the usual piecewise gradient.
+ *  - row i of p's subgraph has the layer-1 input x_i of width F: x_i[0] = (float)dist[i] (the structural label),
+ *    x_i[c] = table[gid[i] * ld + c] for 1 <= c < F (npi_features_t, virtual form).
+ *  - input: dxa [n_rows, 128] (16-byte aligned), the gradient of the batch's targets with respect to the projected
+ *    layer-1 rows x_i . W1 -- what the backward pass leaves after the transposed layer-1 aggregation
+ *    (npi_sage_aggregate_bwd, or npi_tiny_bwd phase 1 on the small-subgraph path) when it is seeded with
+ *    d_logp[b] = e_c (or p_c e_c) for every pair b.  Subgraphs are disjoint row ranges and nothing in evaluation mode
+ *    couples the pairs of a batch, so one backward pass gives every pair its own gradient.  It must be per row: the
+ *    per-context backward of conv1 (npi_csr_gather_sum over contexts) sums rows of different subgraphs.
+ *  - w1 = conv1.weight [F, 128] row-major; graph_ptr [B + 1] = rows of pair b at the input layer (npi_batch_prepare).
+ *  - outputs: grad_x[i][c] = d t(p) / d x_i[c] = (dxa_i . W1^T)[c]  ([n_rows, F] row-major; NULL = not written);
+ *             node_attr[i] = sum_c x_i[c] grad_x[i][c]  (gradient x input per row);
+ *             feature_attr[p][c] = sum over the rows i of p of x_i[c] grad_x[i][c]  ([B, F] row-major).
+ *    The rows used are those below min(n_rows, graph_ptr[B]); n_rows (host) sizes the grid and the workspace.
+ * 1 <= F <= 256, B >= 1, n_rows >= 0, ld >= F.  SIMT fp32 (the backward pass before it costs far more).  Every sum has
+ * a fixed order: a pair's rows are summed in chunks of 32 counted from its first row, and a pair of several chunks adds
+ * their partials in chunk order (a CTA per pair), so the outputs are bit-identical on reruns and a pair's sums do not
+ * depend on where it sits in its batch.  No float atomics, no host synchronisation, three launches (two when n_rows is
+ * 0); the workspace (npi_input_attribution_workspace_bytes) needs no initialisation. */
+int64_t npi_input_attribution_workspace_bytes(int32_t n_rows, int32_t B, int32_t F);
+int npi_input_attribution(const float* dxa, const int32_t* gid, const uint8_t* dist, const int32_t* graph_ptr, int32_t B,
+                          int32_t n_rows, const float* table, int32_t ld, int32_t F, const float* w1,
+                          float* node_attr, float* feature_attr, float* grad_x,
+                          void* workspace, int64_t workspace_bytes, npi_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------
  * node2vec on the GPU (the stage that produces the embedding columns of the feature table).
  * Replaces node2vec-master/src/node2vec.py and main.py:78-92 of the reference over a CSR with

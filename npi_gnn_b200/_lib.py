@@ -124,6 +124,8 @@ SIGNATURES = {
     "npi_group_topk": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _i64, _vp]),
     "npi_group_rank_workspace_bytes": (_i64, [_i64, _i32]),
     "npi_group_rank": (C.c_int, [_vp, _vp, _vp, _i64, _i32, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]),
+    "npi_input_attribution_workspace_bytes": (_i64, [_i32, _i32, _i32]),
+    "npi_input_attribution": (C.c_int, [_vp, _vp, _vp, _vp, _i32, _i32, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _i64, _vp]),
     "npi_scalar_axpy": (C.c_int, [_vp, _vp, _f32, _vp]),
     "npi_peer_header_bytes": (_i64, []),
     "npi_peer_alloc": (C.c_int, [_i64, C.POINTER(_vp), C.c_char_p]),
@@ -184,6 +186,7 @@ KERNELS_PER_CALL = {
     "npi_filter_edges_coo": 3, "npi_readout_bwd": 1, "npi_head_fwd": 2, "npi_head_bwd": 2, "npi_head_bwd/phase": 1, "npi_pool_bwd/phase": 1, "npi_head_fwd/phase": 1, "npi_pool_gate_readout/phase": 1, "npi_adam_l2_step": 1,
     "npi_confusion_counts": 1, "npi_rank_curve": 17, "npi_group_topk": 9, "npi_group_topk/1pass": 6, "npi_group_topk/3pass": 12,
     "npi_group_rank": 27, "npi_group_rank/1pass": 24, "npi_group_rank/3pass": 30,
+    "npi_input_attribution": 3, "npi_input_attribution/no_rows": 2,
     "npi_debug_stamp": 1, "npi_hub_rows_reset": 0, "npi_table_grad": 2, "npi_ctx_build": 2, "npi_sort_pairs_u32": 6, "npi_ctx_index_build": 22, "npi_ctx_class_pack": 1,
     "npi_ctx_scatter_max": 1, "npi_ctx_finish": 1, "npi_csr_gather_sum": 1, "npi_allreduce_adam_fused": 1, "npi_scalar_axpy": 1, "npi_peer_barrier": 1,
     "npi_head_fwd_delta": 1, "npi_tiny_transpose": 1, "npi_tiny_fwd": 1, "npi_tiny_bwd": 2, "npi_tiny_bwd/phase": 1, "npi_tiny_weight_grads": 1,

@@ -531,6 +531,35 @@ def group_rank(scores, labels, group, num_groups, hits_k, n_pos, n_neg, twice_u,
            _i64(ws.numel() * ws.element_size()), _s(), count_as=None if passes == 2 else "npi_group_rank/%dpass" % passes)
 
 
+def input_attribution_workspace_bytes(n_rows, B, F):
+    return L.query("npi_input_attribution_workspace_bytes", _i32(n_rows), _i32(B), _i32(F))
+
+
+def input_attribution(dxa, gid, dist, graph_ptr, B, n_rows, table, F, w1, node_attr, feature_attr, ws, grad_x=None):
+    """Gradient x input of every pair's target over the layer-1 input rows of its subgraph (include/npi.h
+    npi_input_attribution): dxa float32 [>= n_rows, 128], gid int32 / dist uint8 [>= n_rows], graph_ptr int32 [>= B + 1],
+    table float32 [V, ld] (row stride ld >= F, unit column stride), w1 float32 [F, 128].  Outputs: node_attr float32
+    [>= n_rows], feature_attr float32 [B, F] and optional grad_x float32 [n_rows, F], all contiguous."""
+    B, n_rows, F = int(B), int(n_rows), int(F)
+    f32 = torch.float32
+    ok = (dxa.dtype == f32 and dxa.dim() == 2 and dxa.shape[1] == H and dxa.is_contiguous() and dxa.shape[0] >= n_rows
+          and gid.dtype == torch.int32 and gid.is_contiguous() and gid.numel() >= n_rows
+          and dist.dtype == torch.uint8 and dist.is_contiguous() and dist.numel() >= n_rows
+          and graph_ptr.dtype == torch.int32 and graph_ptr.is_contiguous() and graph_ptr.numel() >= B + 1
+          and table.dtype == f32 and table.dim() == 2 and table.stride(1) == 1 and table.stride(0) >= F
+          and w1.dtype == f32 and w1.is_contiguous() and tuple(w1.shape) == (F, H)
+          and node_attr.dtype == f32 and node_attr.is_contiguous() and node_attr.numel() >= n_rows
+          and feature_attr.dtype == f32 and feature_attr.is_contiguous() and feature_attr.numel() >= B * F
+          and (grad_x is None or (grad_x.dtype == f32 and grad_x.is_contiguous() and grad_x.numel() >= n_rows * F)))
+    if not ok:
+        raise L.NPIError("input_attribution: expected contiguous float32 dxa [>= %d, 128], int32 gid, uint8 dist, int32 graph_ptr "
+                         "[>= %d], a float32 table of row stride >= F, w1 [%d, 128] and float32 outputs node_attr [>= %d], "
+                         "feature_attr [%d, %d] (and grad_x [%d, %d])" % (n_rows, B + 1, F, n_rows, B, F, n_rows, F))
+    L.call("npi_input_attribution", L.ptr(dxa), L.ptr(gid), L.ptr(dist), L.ptr(graph_ptr), _i32(B), _i32(n_rows), L.ptr(table),
+           _i32(table.stride(0)), _i32(F), L.ptr(w1), L.ptr(node_attr), L.ptr(feature_attr), L.ptr(grad_x), L.ptr(ws),
+           _i64(ws.numel() * ws.element_size()), _s(), count_as=None if n_rows > 0 else "npi_input_attribution/no_rows")
+
+
 # ----------------------------------------------------------------------------- operator-API helpers
 def filter_edges_coo(edge_index, new_id, out, count_dev):
     E = edge_index.shape[1]

@@ -559,6 +559,138 @@ class Scorer:
                 for name, own in (("rna", 0), ("protein", 1))}
 
 
+class Explainer:
+    """Why the model scores a pair as it does: gradient x input attribution of every pair's target to the nodes and the
+    input features of its enclosing subgraph (include/npi.h npi_input_attribution for the semantics).  One eager sweep
+    on the fused engine: per batch the extraction, the evaluation-mode forward, a backward pass seeded on the target
+    class and one call of npi_input_attribution.
+
+    The engine runs with ``contexts=False``: the per-context backward of conv1 sums the gradient rows of identical
+    layer-1 contexts across subgraphs, which would mix pairs.  The small-subgraph path stays where the engine's size
+    rule selects it (its layer-1 gradient is per row).  The weight gradients the backward pass also computes go to a
+    scratch buffer and are discarded.
+
+    ``index`` (optional): explain pairset[index] in that order; positions of the result refer to the view, so a pair
+    listed twice appears twice.  To explain the output of ``Scorer.top_partners``, build a PairSet of the (node,
+    partner) pairs it lists on the same graph and pass it here; ``top_nodes`` then names the nodes behind each score."""
+
+    def __init__(self, pairset, params, batch_size=200, index=None):
+        self.ps, self.params = pairset, params
+        self.B = int(batch_size)
+        if self.B < 1:
+            raise ValueError("Explainer: batch_size = %d, expected >= 1" % self.B)
+        P = len(pairset)
+        if index is not None:
+            index = np.ascontiguousarray(index, dtype=np.int64).reshape(-1)
+            if len(index) and (index.min() < 0 or index.max() >= P):
+                raise ValueError("Explainer: index entries must lie in [0, %d)" % P)
+        self.index = index
+        self.P = P if index is None else len(index)
+        if self.P == 0:
+            raise ValueError("Explainer: nothing to explain (empty pair set or index view)")
+        n = pairset.n_h if index is None else pairset.n_h[index]
+        e = pairset.e_h if index is None else pairset.e_h[index]
+        self.n_rows = np.asarray(n, dtype=np.int64)        # rows of every pair's subgraph, in view order
+        starts = np.arange(0, self.P, self.B)
+        n0 = max(2, int(np.add.reduceat(n, starts).max()))
+        e0 = max(2, int(np.add.reduceat(e, starts).max()))
+        mx = max(2, int(n.max()))
+        g = pairset.graph
+        self.device = g.device
+        self.engine = Engine(g.F, self.B, n0, e0, mx, device=self.device, graph=g, need_backward=True, contexts=False)
+        self.scratch = FlatParams(g.F, self.device)
+        self.ws = torch.empty(ops.input_attribution_workspace_bytes(self.engine.n_cap[0], self.B, g.F), dtype=torch.uint8,
+                              device=self.device)
+        self._seed = torch.zeros(self.B, 2, dtype=torch.float32, device=self.device)
+        self._onehot = torch.zeros(self.B, 2, dtype=torch.float32, device=self.device)
+        self._pair_index = None
+        if index is not None:            # the view's pair indices, padded so that a batch read never runs off the end
+            host = torch.from_numpy(np.concatenate([index, np.full(self.B, index[-1])]).astype(np.int32))
+            self._host_index = host.pin_memory() if torch.cuda.is_available() else host
+            self._pair_index = torch.zeros(self.B, dtype=torch.int32, device=self.device)
+
+    def explain(self, target=1, wrt="logp", full=False):
+        """Attributions of every pair of the view.  ``target``: the class whose score is explained (1 = interacts);
+        ``wrt``: "logp" explains logp[p, target], "prob" explains exp(logp[p, target]); ``full``: also return the input
+        gradient of every row.  Returns a dict of device tensors:
+          logp          float32 [P, 2]  the evaluation-mode log-probabilities
+          node_ptr      int64 [P + 1]   rows node_ptr[p] .. node_ptr[p+1]-1 belong to pair p
+          node, hop     int32 [R]       node serial and hop distance of every row, in extraction order (the target pair
+                                        first)
+          node_attr     float32 [R]     sum_c x_i[c] d target / d x_i[c]   (gradient x input per row)
+          feature_attr  float32 [P, F]  sum over the pair's rows of x_i[c] d target / d x_i[c]; column 0 is the
+                                        structural label, columns 1.. the feature table's
+          grad_x        float32 [R, F]  d target / d x_i (full=True only)
+        Runs eagerly; synchronises once, at the end (a batch that overflowed the extraction buffers raises NPIError).
+        Bad arguments raise ValueError before the device is touched."""
+        if target not in (0, 1):
+            raise ValueError("explain: target = %r, expected class 0 or 1" % (target,))
+        if wrt not in ("logp", "prob"):
+            raise ValueError("explain: wrt = %r, expected \"logp\" or \"prob\"" % (wrt,))
+        target = int(target)
+        g, F, P, B = self.ps.graph, self.ps.graph.F, self.P, self.B
+        node_ptr_h = np.zeros(P + 1, dtype=np.int64)
+        np.cumsum(self.n_rows, out=node_ptr_h[1:])
+        R = int(node_ptr_h[-1])
+        if full:
+            need = R * F * 4
+            free = torch.cuda.mem_get_info(self.device)[0]
+            if need > free:
+                raise ValueError("explain: full=True needs %d bytes for grad_x [%d, %d], %d bytes of device memory are free"
+                                 % (need, R, F, free))
+        dev = self.device
+        out = dict(logp=torch.empty(P, 2, dtype=torch.float32, device=dev),
+                   node_ptr=torch.from_numpy(node_ptr_h).to(dev),
+                   node=torch.empty(R, dtype=torch.int32, device=dev), hop=torch.empty(R, dtype=torch.int32, device=dev),
+                   node_attr=torch.empty(R, dtype=torch.float32, device=dev),
+                   feature_attr=torch.empty(P, F, dtype=torch.float32, device=dev))
+        grad_x = torch.empty(R, F, dtype=torch.float32, device=dev) if full else None
+        if full:
+            out["grad_x"] = grad_x
+        eng, w1 = self.engine, self.params.view("conv1.weight")
+        self._onehot.zero_()
+        self._onehot[:, target] = 1.0
+        if wrt == "logp":
+            self._seed.copy_(self._onehot)
+        for first in range(0, P, B):
+            cnt = min(B, P - first)
+            if self.index is None:
+                eng.load_pairs(self.ps, first=first, count=cnt)
+            else:
+                self._pair_index.copy_(self._host_index[first:first + B], non_blocking=True)
+                eng.load_pairs(self.ps, count=cnt, pair_index=self._pair_index)
+            logp = eng.forward(self.params, training=False)
+            if wrt == "prob":            # d exp(logp_c) / d logp_c = p_c
+                torch.mul(torch.exp(logp), self._onehot[:cnt], out=self._seed[:cnt])
+            eng.backward(self.params, self.scratch, d_logp=self._seed[:cnt])
+            r0, r1 = int(node_ptr_h[first]), int(node_ptr_h[first + cnt])
+            out["logp"][first:first + cnt].copy_(logp)
+            out["node"][r0:r1].copy_(eng.gid[:r1 - r0])
+            out["hop"][r0:r1].copy_(eng.dist[:r1 - r0])
+            ops.input_attribution(eng.big, eng.gid, eng.dist, eng._gp[0], cnt, r1 - r0, g.table, F, w1,
+                                  out["node_attr"][r0:r1], out["feature_attr"][first:first + cnt], self.ws,
+                                  grad_x=None if grad_x is None else grad_x[r0:r1])
+        eng.check_overflow()
+        return out
+
+    @staticmethod
+    def top_nodes(result, k):
+        """The ``k`` rows of largest |node_attr| in every pair of an ``explain`` result (``top_k_by_group`` with the pair
+        as the group; ties by ascending row, i.e. extraction order).  Returns dict of device tensors: node int32 [P, k]
+        (the node serials, -1 past count), attr float32 [P, k] (the signed node_attr, NaN past count), count int32 [P] =
+        min(k, rows of the pair)."""
+        if not 1 <= int(k) <= 1024:
+            raise ValueError("top_nodes: k = %d outside 1..1024" % k)
+        na, ptr = result["node_attr"], result["node_ptr"]
+        P, R = ptr.numel() - 1, na.numel()
+        pair = torch.repeat_interleave(torch.arange(P, dtype=torch.int32, device=na.device), ptr.diff(), output_size=R)
+        r = top_k_by_group(na.abs(), pair, P, k)
+        hit = r["pos"] >= 0
+        row = r["pos"].clamp(min=0).long()
+        return dict(node=torch.where(hit, result["node"][row], -1),
+                    attr=torch.where(hit, na[row], float("nan")), count=r["count"])
+
+
 def metrics(TP, FN, TN, FP):
     """Accuracy, Precision, Sensitivity, Specificity, MCC exactly as src/methods.py:107-127."""
     tot = TP + TN + FP + FN
