@@ -38,6 +38,15 @@ static int64_t at_max_chunks(int32_t n_rows, int32_t B) {
     return (int64_t)(n_rows > 0 ? n_rows : 0) / AT_ROWS + (B > 0 ? B : 0);
 }
 
+// carves the workspace: chunk_ptr [B + 1] | part [max chunks][F]; returns the bytes it needs (ws may be null for the query).
+// The last region is not padded.
+static int64_t attrib_layout(int32_t n_rows, int32_t B, int32_t F, char* ws, int32_t** chunk_ptr, float** part) {
+    WsCarver c{ws};
+    *chunk_ptr = c.take<int32_t>(4 * ((int64_t)B + 1));
+    *part = c.take<float>(0);
+    return c.off + at_max_chunks(n_rows, B) * (int64_t)F * (int64_t)sizeof(float);
+}
+
 __device__ __forceinline__ int at_rows_of(const int32_t* gptr, int p, int N) {
     return min(gptr[p + 1], N) - min(gptr[p], N);
 }
@@ -165,9 +174,9 @@ __global__ void __launch_bounds__(AT_THREADS) attrib_pairs_kernel(const int32_t*
 using namespace npi;
 
 extern "C" int64_t npi_input_attribution_workspace_bytes(int32_t n_rows, int32_t B, int32_t F) {
-    const int64_t ptr_bytes = ((int64_t)(B > 0 ? B : 0) + 1) * 4;
-    const int64_t part_off = (ptr_bytes + 255) / 256 * 256;
-    return part_off + at_max_chunks(n_rows, B) * (int64_t)(F > 0 ? F : 1) * (int64_t)sizeof(float);
+    int32_t* chunk_ptr;
+    float* part;
+    return attrib_layout(n_rows, B > 0 ? B : 0, F > 0 ? F : 1, nullptr, &chunk_ptr, &part);
 }
 
 extern "C" int npi_input_attribution(const float* dxa, const int32_t* gid, const uint8_t* dist, const int32_t* graph_ptr,
@@ -185,8 +194,9 @@ extern "C" int npi_input_attribution(const float* dxa, const int32_t* gid, const
     NPI_REQUIRE(workspace_bytes >= need, "input_attribution: workspace of %lld bytes, %lld needed", (long long)workspace_bytes,
                 (long long)need);
     cudaStream_t st = (cudaStream_t)stream;
-    int32_t* chunk_ptr = (int32_t*)workspace;
-    float* part = (float*)((char*)workspace + ((int64_t)(B + 1) * 4 + 255) / 256 * 256);
+    int32_t* chunk_ptr;
+    float* part;
+    attrib_layout(n_rows, B, F, (char*)workspace, &chunk_ptr, &part);
     attrib_chunks_kernel<<<1, AT_SCAN, 0, st>>>(graph_ptr, B, n_rows, chunk_ptr);
     NPI_CHECK_LAUNCH();
     const int64_t max_chunks = at_max_chunks(n_rows, B);

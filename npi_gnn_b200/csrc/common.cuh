@@ -170,6 +170,69 @@ __device__ __forceinline__ uint32_t rank_key(float s) {
     return ~u;                                               // ascending key = descending score
 }
 
+// Workspace carver of the ranking entry points: consecutive regions, each rounded up to 256 bytes.  A null base carves
+// nothing and only counts the bytes (the *_workspace_bytes query); `off` is the total.
+struct WsCarver {
+    char* base;
+    int64_t off = 0;
+    template <typename T>
+    T* take(int64_t bytes) {
+        char* p = base ? base + off : nullptr;
+        off += (bytes + 255) / 256 * 256;
+        return (T*)p;
+    }
+};
+
+// Block sum of one value per thread in a fixed order (warp butterflies, then the warp partials in warp order):
+// bit-reproducible for fp64.  `sh` holds NT / 32 values; every thread of the NT-thread block must call it.
+template <int NT, typename T>
+__device__ __forceinline__ T block_sum(T v, T* sh) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    __syncthreads();                                         // protect sh from the previous call's readers
+    if (lane == 0) sh[w] = v;
+    __syncthreads();
+    T s = sh[0];
+    for (int k = 1; k < NT / 32; ++k) s += sh[k];
+    return s;
+}
+
+// True in the last CTA of the grid to arrive here, false in every other one (block-uniform).  Every thread calls it
+// after its CTA has written its per-CTA partials; the last CTA then reads all partials with __ldcg.  The ticket counts
+// the arrivals and is reset by the last CTA, so it is zero again for the next launch.
+__device__ __forceinline__ bool last_cta(unsigned int* ticket) {
+    __threadfence();
+    __syncthreads();
+    if (!__syncthreads_or(threadIdx.x == 0 && atomicAdd(ticket, 1u) == gridDim.x - 1u)) return false;
+    __threadfence();
+    if (threadIdx.x == 0) *ticket = 0u;
+    return true;
+}
+
+// OR of a status word over the block, bits 0 .. NBITS - 1.  Every thread of the block must call it.
+template <int NBITS>
+__device__ __forceinline__ int block_or_bits(int st) {
+    int r = 0;
+#pragma unroll
+    for (int b = 0; b < NBITS; ++b) r |= __syncthreads_or(st & (1 << b)) ? 1 << b : 0;
+    return r;
+}
+
+// npi_sort_pairs_u32 of (keys_a, vals_a) by `bits` key bits with (keys_b, vals_b) as the other buffer pair.  On return
+// (keys, vals) is the pair holding the sorted result and (free_keys, free_vals) the other one.
+struct SortedPairs {
+    uint32_t* keys; int32_t* vals;
+    uint32_t* free_keys; int32_t* free_vals;
+};
+inline int sort_pairs(uint32_t* keys_a, int32_t* vals_a, uint32_t* keys_b, int32_t* vals_b, int64_t n, int bits, void* ws,
+                      int64_t ws_bytes, cudaStream_t st, SortedPairs* out) {
+    const int rc = npi_sort_pairs_u32(keys_a, vals_a, keys_b, vals_b, n, bits, ws, ws_bytes, st);
+    if (npi_sort_passes(bits) & 1) *out = {keys_b, vals_b, keys_a, vals_a};
+    else *out = {keys_a, vals_a, keys_b, vals_b};
+    return rc;
+}
+
 __device__ __forceinline__ float4 ldg4(const float* p) { return __ldg(reinterpret_cast<const float4*>(p)); }
 __device__ __forceinline__ void st4(float* p, float4 v) { *reinterpret_cast<float4*>(p) = v; }
 __device__ __forceinline__ float4 add4(float4 a, float4 b) { return make_float4(a.x + b.x, a.y + b.y, a.z + b.z, a.w + b.w); }

@@ -29,7 +29,6 @@ constexpr int GR_ITEMS = 4;
 constexpr int GR_TILE = GR_THREADS * GR_ITEMS;     // 4096 items per CTA
 constexpr int GG_THREADS = 256;                    // groups per CTA of gr_group_kernel
 constexpr int GR_MAXH = 8;                         // Hits@K cut-offs per call
-constexpr int64_t GR_ALIGN = 256;
 
 struct GrHits { int32_t k[GR_MAXH]; int32_t n; };
 
@@ -46,29 +45,26 @@ struct GrWs {
     int32_t* part_hits;                 // [GR_MAXH][item tiles]
 };
 
-static int64_t gr_up(int64_t b) { return (b + GR_ALIGN - 1) / GR_ALIGN * GR_ALIGN; }
-
 // carves the workspace; returns the bytes it needs (ws may be null for the query)
 static int64_t group_rank_layout(int64_t n, int32_t num_groups, char* ws, GrWs* w) {
     const int64_t ntiles = (n + GR_TILE - 1) / GR_TILE;
     const int64_t gctas = ((int64_t)num_groups + GG_THREADS - 1) / GG_THREADS;
-    int64_t off = 0;
-    auto take = [&](int64_t bytes) { char* p = ws ? ws + off : nullptr; off += gr_up(bytes); return p; };
-    w->keys_a = (uint32_t*)take(4 * (n + 1));
-    w->vals_a = (int32_t*)take(4 * (n + 1));
-    w->keys_b = (uint32_t*)take(4 * (n + 1));
-    w->vals_b = (int32_t*)take(4 * (n + 1));
+    WsCarver c{ws};
+    w->keys_a = c.take<uint32_t>(4 * (n + 1));
+    w->vals_a = c.take<int32_t>(4 * (n + 1));
+    w->keys_b = c.take<uint32_t>(4 * (n + 1));
+    w->vals_b = c.take<int32_t>(4 * (n + 1));
     w->sort_bytes = npi_sort_workspace_bytes(n);
-    w->sort_ws = take(w->sort_bytes);
-    w->neg = (int32_t*)take(4 * n);
-    w->tile_status = (int32_t*)take(4 * ntiles);
-    w->scan_tiles = (int32_t*)take(4 * ntiles);
-    w->gptr = (int32_t*)take(4 * ((int64_t)num_groups + 1));
-    w->gpart = (int32_t*)take(4 * 3 * gctas);
-    w->ticket = (unsigned int*)take(4);
-    w->part_rr = (double*)take(8 * ntiles);
-    w->part_hits = (int32_t*)take(4 * GR_MAXH * ntiles);
-    return off;
+    w->sort_ws = c.take<void>(w->sort_bytes);
+    w->neg = c.take<int32_t>(4 * n);
+    w->tile_status = c.take<int32_t>(4 * ntiles);
+    w->scan_tiles = c.take<int32_t>(4 * ntiles);
+    w->gptr = c.take<int32_t>(4 * ((int64_t)num_groups + 1));
+    w->gpart = c.take<int32_t>(4 * 3 * gctas);
+    w->ticket = c.take<unsigned int>(4);
+    w->part_rr = c.take<double>(8 * ntiles);
+    w->part_hits = c.take<int32_t>(4 * GR_MAXH * ntiles);
+    return c.off;
 }
 
 __global__ void __launch_bounds__(GR_THREADS) gr_key_kernel(const float* __restrict__ scores, const int32_t* __restrict__ labels,
@@ -88,7 +84,7 @@ __global__ void __launch_bounds__(GR_THREADS) gr_key_kernel(const float* __restr
             vals[i] = (int32_t)i;
         }
     }
-    bad = (__syncthreads_or(bad & 1) ? 1 : 0) | (__syncthreads_or(bad & 2) ? 2 : 0) | (__syncthreads_or(bad & 4) ? 4 : 0);
+    bad = block_or_bits<3>(bad);
     if (threadIdx.x == 0) {
         tile_status[blockIdx.x] = bad;
         if (blockIdx.x == 0) *ticket = 0u;       // the caller's workspace need not be zeroed: the emit kernel runs later in stream order
@@ -127,19 +123,6 @@ __global__ void __launch_bounds__(GR_THREADS) gr_flags_kernel(const int32_t* __r
     }
 }
 
-template <typename T>
-__device__ __forceinline__ T gr_block_sum(T v, T* sh) {            // fixed-order tree: bit-reproducible for fp64
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    __syncthreads();                                               // protect sh from the previous call's readers
-    if (lane == 0) sh[w] = v;
-    __syncthreads();
-    T s = sh[0];
-    for (int k = 1; k < (int)(blockDim.x >> 5); ++k) s += sh[k];
-    return s;
-}
-
 __global__ void __launch_bounds__(GG_THREADS) gr_group_kernel(const int32_t* __restrict__ gptr, const int32_t* __restrict__ cumneg,
                                                               int32_t num_groups, int32_t* __restrict__ n_pos, int32_t* __restrict__ n_neg,
                                                               int64_t* __restrict__ twice_u, int32_t* __restrict__ gpart) {
@@ -155,9 +138,9 @@ __global__ void __launch_bounds__(GG_THREADS) gr_group_kernel(const int32_t* __r
         if (nn > 0) ranked = np; else unranked = np;
         scored = np > 0 && nn > 0;
     }
-    ranked = gr_block_sum(ranked, sh);
-    unranked = gr_block_sum(unranked, sh);
-    scored = gr_block_sum(scored, sh);
+    ranked = block_sum<GG_THREADS>(ranked, sh);
+    unranked = block_sum<GG_THREADS>(unranked, sh);
+    scored = block_sum<GG_THREADS>(scored, sh);
     if (threadIdx.x == 0) {
         gpart[blockIdx.x] = ranked;
         gpart[gridDim.x + blockIdx.x] = unranked;
@@ -176,7 +159,6 @@ __global__ void __launch_bounds__(GR_THREADS) gr_emit_kernel(const uint32_t* __r
     __shared__ double sh_d[GR_THREADS / 32];
     __shared__ long long sh_l[GR_THREADS / 32];
     __shared__ int sh_i[GR_THREADS / 32];
-    __shared__ int s_last;
     const int ntiles = (int)gridDim.x;
     const int64_t j0 = (int64_t)blockIdx.x * GR_TILE + threadIdx.x;
     double rr = 0.0;
@@ -227,31 +209,26 @@ __global__ void __launch_bounds__(GR_THREADS) gr_emit_kernel(const uint32_t* __r
         if (tied_out) tied_out[p] = query ? t : -1;
     }
 
-    rr = gr_block_sum(rr, sh_d);
+    rr = block_sum<GR_THREADS>(rr, sh_d);
     if (threadIdx.x == 0) part_rr[blockIdx.x] = rr;
 #pragma unroll
     for (int h = 0; h < GR_MAXH; ++h) {
         if (h < hk.n) {
-            const int s = gr_block_sum(hits[h], sh_i);               // <= 4096: the tile's items
+            const int s = block_sum<GR_THREADS>(hits[h], sh_i);      // <= 4096: the tile's items
             if (threadIdx.x == 0) part_hits[(int64_t)h * ntiles + blockIdx.x] = s;
         }
     }
-    __threadfence();
-    __syncthreads();
-    if (threadIdx.x == 0) s_last = (atomicAdd(ticket, 1u) == (unsigned)ntiles - 1u) ? 1 : 0;
-    __syncthreads();
-    if (!s_last) return;
-    __threadfence();
+    if (!last_cta(ticket)) return;
     rr = 0.0;
     for (int b = threadIdx.x; b < ntiles; b += GR_THREADS) rr += __ldcg(&part_rr[b]);     // CTA b always lands in thread b % 1024, in order
-    rr = gr_block_sum(rr, sh_d);
+    rr = block_sum<GR_THREADS>(rr, sh_d);
     if (threadIdx.x == 0) *sum_rr = rr;
 #pragma unroll
     for (int h = 0; h < GR_MAXH; ++h) {
         if (h < hk.n) {
             long long s = 0;
             for (int b = threadIdx.x; b < ntiles; b += GR_THREADS) s += __ldcg(&part_hits[(int64_t)h * ntiles + b]);
-            s = gr_block_sum(s, sh_l);
+            s = block_sum<GR_THREADS>(s, sh_l);
             if (threadIdx.x == 0) summary[3 + h] = s;
         }
     }
@@ -259,10 +236,9 @@ __global__ void __launch_bounds__(GR_THREADS) gr_emit_kernel(const uint32_t* __r
     for (int c = 0; c < 3; ++c) {                                  // ranked queries, unranked queries, scored groups
         long long s = 0;
         for (int b = threadIdx.x; b < gctas; b += GR_THREADS) s += gpart[(int64_t)c * gctas + b];
-        s = gr_block_sum(s, sh_l);
+        s = block_sum<GR_THREADS>(s, sh_l);
         if (threadIdx.x == 0) summary[c] = s;
     }
-    if (threadIdx.x == 0) *ticket = 0u;
 }
 
 }  // namespace npi
@@ -298,22 +274,19 @@ extern "C" int npi_group_rank(const float* scores, const int32_t* labels, const 
     const int gctas = (int)(((int64_t)num_groups + GG_THREADS - 1) / GG_THREADS);
     gr_key_kernel<<<ntiles, GR_THREADS, 0, st>>>(scores, labels, group, n, num_groups, w.keys_a, w.vals_a, w.tile_status, w.ticket);
     NPI_CHECK_LAUNCH();
-    int rc = npi_sort_pairs_u32(w.keys_a, w.vals_a, w.keys_b, w.vals_b, n, 32, w.sort_ws, w.sort_bytes, stream);
+    SortedPairs by_score, by_group;
+    int rc = sort_pairs(w.keys_a, w.vals_a, w.keys_b, w.vals_b, n, 32, w.sort_ws, w.sort_bytes, st, &by_score);
     if (rc != NPI_OK) return rc;
-    // (k1, v1): the pair holding the score order; (k2, v2): the other one
-    const bool in_b1 = npi_sort_passes(32) & 1;
-    uint32_t* k1 = in_b1 ? w.keys_b : w.keys_a; int32_t* v1 = in_b1 ? w.vals_b : w.vals_a;
-    uint32_t* k2 = in_b1 ? w.keys_a : w.keys_b; int32_t* v2 = in_b1 ? w.vals_a : w.vals_b;
-    gr_gather_kernel<<<ntiles, GR_THREADS, 0, st>>>(v1, labels, group, n, num_groups, k2, v2);
+    gr_gather_kernel<<<ntiles, GR_THREADS, 0, st>>>(by_score.vals, labels, group, n, num_groups, by_score.free_keys,
+                                                    by_score.free_vals);
     NPI_CHECK_LAUNCH();
-    const int bits = group_bits(num_groups);
-    rc = npi_sort_pairs_u32(k2, v2, k1, v1, n, bits, w.sort_ws, w.sort_bytes, stream);
+    rc = sort_pairs(by_score.free_keys, by_score.free_vals, by_score.keys, by_score.vals, n, group_bits(num_groups), w.sort_ws,
+                    w.sort_bytes, st, &by_group);
     if (rc != NPI_OK) return rc;
-    const bool in_1 = npi_sort_passes(bits) & 1;
-    const uint32_t* gkeys = in_1 ? k1 : k2;
-    const int32_t* gvals = in_1 ? v1 : v2;
-    uint32_t* skey = in_1 ? k2 : k1;                              // the free pair: sorted score keys and cumneg
-    int32_t* cumneg = in_1 ? v2 : v1;
+    const uint32_t* gkeys = by_group.keys;
+    const int32_t* gvals = by_group.vals;
+    uint32_t* skey = by_group.free_keys;                          // the free pair: sorted score keys and cumneg
+    int32_t* cumneg = by_group.free_vals;
     rc = launch_group_bounds(gkeys, n, num_groups, w.tile_status, ntiles, w.gptr, status, st);
     if (rc != NPI_OK) return rc;
     gr_flags_kernel<<<ntiles, GR_THREADS, 0, st>>>(gvals, scores, n, skey, w.neg);

@@ -15,8 +15,6 @@
 // tied keys, so every output is bit-identical under any permutation of the input.  No floating-point atomics.
 #include "common.cuh"
 
-extern "C" int32_t npi_sort_passes(int32_t key_bits);
-
 namespace npi {
 
 constexpr int RK_THREADS = 1024;
@@ -24,7 +22,6 @@ constexpr int RK_ITEMS = 4;
 constexpr int RK_TILE = RK_THREADS * RK_ITEMS;      // 4096 items per CTA
 constexpr int RA_THREADS = 256;
 constexpr int RA_MAX_CTAS = 1024;                   // area partials (one per CTA), summed by the last CTA
-constexpr int64_t RK_ALIGN = 256;
 
 __device__ __forceinline__ float rank_score(uint32_t key) {
     const uint32_t o = ~key;
@@ -40,51 +37,46 @@ struct RankWs {
     long long* part_u; double* part_ap; double* part_tr;
 };
 
-static int64_t rk_up(int64_t b) { return (b + RK_ALIGN - 1) / RK_ALIGN * RK_ALIGN; }
-
 // carves the workspace; returns the bytes it needs (ws may be null for the query)
 static int64_t rank_layout(int64_t n, char* ws, RankWs* w) {
     const int64_t ntiles = (n + RK_TILE - 1) / RK_TILE;
-    int64_t off = 0;
-    auto take = [&](int64_t bytes) { char* p = ws ? ws + off : nullptr; off += rk_up(bytes); return p; };
-    w->keys_a = (uint32_t*)take(4 * n);
-    w->vals_a = (int32_t*)take(4 * n);
-    w->keys_b = (uint32_t*)take(4 * n);
-    w->vals_b = (int32_t*)take(4 * n);
+    WsCarver c{ws};
+    w->keys_a = c.take<uint32_t>(4 * n);
+    w->vals_a = c.take<int32_t>(4 * n);
+    w->keys_b = c.take<uint32_t>(4 * n);
+    w->vals_b = c.take<int32_t>(4 * n);
     w->sort_bytes = npi_sort_workspace_bytes(n);
-    w->sort_ws = take(w->sort_bytes);
-    w->tile_status = (int32_t*)take(4 * ntiles);
-    w->tile_pos = (int32_t*)take(4 * ntiles);
-    w->tile_end = (int32_t*)take(4 * ntiles);
-    w->totals = (int32_t*)take(8);
-    w->ticket = (unsigned int*)take(4);
-    w->part_u = (long long*)take(8 * RA_MAX_CTAS);
-    w->part_ap = (double*)take(8 * RA_MAX_CTAS);
-    w->part_tr = (double*)take(8 * RA_MAX_CTAS);
-    return off;
+    w->sort_ws = c.take<void>(w->sort_bytes);
+    w->tile_status = c.take<int32_t>(4 * ntiles);
+    w->tile_pos = c.take<int32_t>(4 * ntiles);
+    w->tile_end = c.take<int32_t>(4 * ntiles);
+    w->totals = c.take<int32_t>(8);
+    w->ticket = c.take<unsigned int>(4);
+    w->part_u = c.take<long long>(8 * RA_MAX_CTAS);
+    w->part_ap = c.take<double>(8 * RA_MAX_CTAS);
+    w->part_tr = c.take<double>(8 * RA_MAX_CTAS);
+    return c.off;
 }
 
 __global__ void __launch_bounds__(RK_THREADS) rank_key_kernel(const float* __restrict__ scores, const int32_t* __restrict__ labels,
                                                               int64_t n, uint32_t* __restrict__ keys, int32_t* __restrict__ vals,
                                                               int32_t* __restrict__ tile_status, unsigned int* __restrict__ ticket) {
     const int64_t i0 = (int64_t)blockIdx.x * RK_TILE + threadIdx.x;
-    int bad_score = 0, bad_label = 0;
+    int bad = 0;
 #pragma unroll
     for (int q = 0; q < RK_ITEMS; ++q) {
         const int64_t i = i0 + (int64_t)q * RK_THREADS;
         if (i < n) {
             const float s = scores[i];
             const int32_t y = labels[i];
-            bad_score |= (s != s);
-            bad_label |= (y != 0 && y != 1);
+            bad |= (s != s ? 1 : 0) | (y != 0 && y != 1 ? 2 : 0);
             keys[i] = rank_key(s);
             vals[i] = y;
         }
     }
-    bad_score = __syncthreads_or(bad_score);
-    bad_label = __syncthreads_or(bad_label);
+    bad = block_or_bits<2>(bad);
     if (threadIdx.x == 0) {
-        tile_status[blockIdx.x] = (bad_score ? 1 : 0) | (bad_label ? 2 : 0);
+        tile_status[blockIdx.x] = bad;
         if (blockIdx.x == 0) *ticket = 0u;       // the caller's workspace need not be zeroed: the area kernel runs later in stream order
     }
 }
@@ -127,7 +119,7 @@ __global__ void __launch_bounds__(RK_THREADS) rank_scan_kernel(int32_t* __restri
         if (t < ntiles) { tile_pos[t] = run_p + xp; tile_end[t] = run_e + xe; }
         run_p += tp; run_e += te;
     }
-    st = __syncthreads_or(st & 1) | (__syncthreads_or(st & 2) ? 2 : 0);
+    st = block_or_bits<2>(st);
     if (threadIdx.x == 0) { totals[0] = run_p; totals[1] = run_e; *status = st; }
 }
 
@@ -159,19 +151,6 @@ __global__ void __launch_bounds__(RK_THREADS) rank_emit_kernel(const uint32_t* _
     }
 }
 
-template <typename T>
-__device__ __forceinline__ T rank_block_sum(T v, T* sh) {          // fixed-order tree: bit-reproducible for fp64
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    __syncthreads();
-    if (lane == 0) sh[w] = v;
-    __syncthreads();
-    T s = sh[0];
-    for (int k = 1; k < RA_THREADS / 32; ++k) s += sh[k];
-    return s;
-}
-
 __global__ void __launch_bounds__(RA_THREADS) rank_area_kernel(const int32_t* __restrict__ w_tps, const int32_t* __restrict__ w_fps, int64_t n,
                                                                const int32_t* __restrict__ totals, long long* __restrict__ part_u,
                                                                double* __restrict__ part_ap, double* __restrict__ part_tr,
@@ -179,7 +158,6 @@ __global__ void __launch_bounds__(RA_THREADS) rank_area_kernel(const int32_t* __
                                                                double* __restrict__ areas) {
     __shared__ long long sh_u[RA_THREADS / 32];
     __shared__ double sh_d[RA_THREADS / 32];
-    __shared__ int s_last;
     const int T = totals[1];
     long long u = 0;
     double ap = 0.0, tr = 0.0;
@@ -194,29 +172,23 @@ __global__ void __launch_bounds__(RA_THREADS) rank_area_kernel(const int32_t* __
             tr += (double)(t - tp) * (prec + prev);
         }
     }
-    u = rank_block_sum(u, sh_u);
-    ap = rank_block_sum(ap, sh_d);
-    tr = rank_block_sum(tr, sh_d);
+    u = block_sum<RA_THREADS>(u, sh_u);
+    ap = block_sum<RA_THREADS>(ap, sh_d);
+    tr = block_sum<RA_THREADS>(tr, sh_d);
     if (threadIdx.x == 0) { part_u[blockIdx.x] = u; part_ap[blockIdx.x] = ap; part_tr[blockIdx.x] = tr; }
-    __threadfence();
-    __syncthreads();
-    if (threadIdx.x == 0) s_last = (atomicAdd(ticket, 1u) == gridDim.x - 1u) ? 1 : 0;
-    __syncthreads();
-    if (!s_last) return;
-    __threadfence();
+    if (!last_cta(ticket)) return;
     u = 0; ap = 0.0; tr = 0.0;
     for (int b = threadIdx.x; b < (int)gridDim.x; b += RA_THREADS) {      // CTA b always lands in thread b % 256, in order
         u += __ldcg(&part_u[b]); ap += __ldcg(&part_ap[b]); tr += __ldcg(&part_tr[b]);
     }
-    u = rank_block_sum(u, sh_u);
-    ap = rank_block_sum(ap, sh_d);
-    tr = rank_block_sum(tr, sh_d);
+    u = block_sum<RA_THREADS>(u, sh_u);
+    ap = block_sum<RA_THREADS>(ap, sh_d);
+    tr = block_sum<RA_THREADS>(tr, sh_d);
     if (threadIdx.x == 0) {
         const int64_t n_pos = totals[0];
         summary[0] = n_pos; summary[1] = n - n_pos; summary[2] = T; summary[3] = u;
         areas[0] = ap / (double)n_pos;
         areas[1] = 0.5 * tr / (double)n_pos;
-        *ticket = 0u;
     }
 }
 
@@ -242,18 +214,16 @@ extern "C" int npi_rank_curve(const float* scores, const int32_t* labels, int64_
     const int ntiles = (int)((n + RK_TILE - 1) / RK_TILE);
     rank_key_kernel<<<ntiles, RK_THREADS, 0, st>>>(scores, labels, n, w.keys_a, w.vals_a, w.tile_status, w.ticket);
     NPI_CHECK_LAUNCH();
-    int rc = npi_sort_pairs_u32(w.keys_a, w.vals_a, w.keys_b, w.vals_b, n, 32, w.sort_ws, w.sort_bytes, stream);
+    SortedPairs sp;
+    int rc = sort_pairs(w.keys_a, w.vals_a, w.keys_b, w.vals_b, n, 32, w.sort_ws, w.sort_bytes, st, &sp);
     if (rc != NPI_OK) return rc;
-    const bool in_b = npi_sort_passes(32) & 1;
-    const uint32_t* keys = in_b ? w.keys_b : w.keys_a;
-    const int32_t* vals = in_b ? w.vals_b : w.vals_a;
-    int32_t* w_tps = (int32_t*)(in_b ? w.keys_a : w.keys_b);       // the sort's other buffer pair holds the curve
-    int32_t* w_fps = in_b ? w.vals_a : w.vals_b;
-    rank_tile_kernel<<<ntiles, RK_THREADS, 0, st>>>(keys, vals, n, w.tile_pos, w.tile_end);
+    int32_t* w_tps = (int32_t*)sp.free_keys;                         // the sort's other buffer pair holds the curve
+    int32_t* w_fps = sp.free_vals;
+    rank_tile_kernel<<<ntiles, RK_THREADS, 0, st>>>(sp.keys, sp.vals, n, w.tile_pos, w.tile_end);
     NPI_CHECK_LAUNCH();
     rank_scan_kernel<<<1, RK_THREADS, 0, st>>>(w.tile_pos, w.tile_end, w.tile_status, ntiles, w.totals, status);
     NPI_CHECK_LAUNCH();
-    rank_emit_kernel<<<ntiles, RK_THREADS, 0, st>>>(keys, vals, n, w.tile_pos, w.tile_end, w_tps, w_fps, thresholds, tps, fps);
+    rank_emit_kernel<<<ntiles, RK_THREADS, 0, st>>>(sp.keys, sp.vals, n, w.tile_pos, w.tile_end, w_tps, w_fps, thresholds, tps, fps);
     NPI_CHECK_LAUNCH();
     const int64_t want = (n + 8 * RA_THREADS - 1) / (8 * RA_THREADS);
     const int actas = (int)(want < RA_MAX_CTAS ? want : RA_MAX_CTAS);

@@ -26,7 +26,6 @@ constexpr int KK_THREADS = 1024;
 constexpr int KK_ITEMS = 4;
 constexpr int KK_TILE = KK_THREADS * KK_ITEMS;
 constexpr int TB_THREADS = 256;
-constexpr int64_t TK_ALIGN = 256;
 
 struct TopkWs {
     uint32_t* keys_a; int32_t* vals_a; uint32_t* keys_b; int32_t* vals_b;
@@ -35,29 +34,26 @@ struct TopkWs {
     int32_t* gptr;                      // [num_groups + 1]
 };
 
-static int64_t tk_up(int64_t b) { return (b + TK_ALIGN - 1) / TK_ALIGN * TK_ALIGN; }
-
 // carves the workspace; returns the bytes it needs (ws may be null for the query)
 static int64_t topk_layout(int64_t n, int32_t num_groups, char* ws, TopkWs* w) {
     const int64_t ntiles = (n + KK_TILE - 1) / KK_TILE;
-    int64_t off = 0;
-    auto take = [&](int64_t bytes) { char* p = ws ? ws + off : nullptr; off += tk_up(bytes); return p; };
-    w->keys_a = (uint32_t*)take(4 * n);
-    w->vals_a = (int32_t*)take(4 * n);
-    w->keys_b = (uint32_t*)take(4 * n);
-    w->vals_b = (int32_t*)take(4 * n);
+    WsCarver c{ws};
+    w->keys_a = c.take<uint32_t>(4 * n);
+    w->vals_a = c.take<int32_t>(4 * n);
+    w->keys_b = c.take<uint32_t>(4 * n);
+    w->vals_b = c.take<int32_t>(4 * n);
     w->sort_bytes = npi_sort_workspace_bytes(n);
-    w->sort_ws = take(w->sort_bytes);
-    w->tile_status = (int32_t*)take(4 * ntiles);
-    w->gptr = (int32_t*)take(4 * ((int64_t)num_groups + 1));
-    return off;
+    w->sort_ws = c.take<void>(w->sort_bytes);
+    w->tile_status = c.take<int32_t>(4 * ntiles);
+    w->gptr = c.take<int32_t>(4 * ((int64_t)num_groups + 1));
+    return c.off;
 }
 
 __global__ void __launch_bounds__(KK_THREADS) topk_key_kernel(const float* __restrict__ scores, const int32_t* __restrict__ group,
                                                               int64_t n, int32_t num_groups, uint32_t* __restrict__ keys,
                                                               int32_t* __restrict__ vals, int32_t* __restrict__ tile_status) {
     const int64_t i0 = (int64_t)blockIdx.x * KK_TILE + threadIdx.x;
-    int bad_score = 0, bad_group = 0;
+    int bad = 0;
 #pragma unroll
     for (int q = 0; q < KK_ITEMS; ++q) {
         const int64_t i = i0 + (int64_t)q * KK_THREADS;
@@ -65,15 +61,13 @@ __global__ void __launch_bounds__(KK_THREADS) topk_key_kernel(const float* __res
             const float s = scores[i];
             const int32_t g = group[i];
             const bool out = g < 0 || g >= num_groups;
-            bad_score |= (s != s);
-            bad_group |= out;
+            bad |= (s != s ? 1 : 0) | (out ? 2 : 0);
             keys[i] = out ? 0u : (uint32_t)g;      // keeps every later access in bounds; the status marks the result void
             vals[i] = (int32_t)i;
         }
     }
-    bad_score = __syncthreads_or(bad_score);
-    bad_group = __syncthreads_or(bad_group);
-    if (threadIdx.x == 0) tile_status[blockIdx.x] = (bad_score ? 1 : 0) | (bad_group ? 2 : 0);
+    bad = block_or_bits<2>(bad);
+    if (threadIdx.x == 0) tile_status[blockIdx.x] = bad;
 }
 
 __global__ void __launch_bounds__(TB_THREADS) topk_bounds_kernel(const uint32_t* __restrict__ keys, int64_t n, int32_t num_groups,
@@ -91,7 +85,7 @@ __global__ void __launch_bounds__(TB_THREADS) topk_bounds_kernel(const uint32_t*
     if (blockIdx.x == 0) {
         int st = 0;
         for (int t = threadIdx.x; t < ntiles; t += TB_THREADS) st |= tile_status[t];
-        st = (__syncthreads_or(st & 1) ? 1 : 0) | (__syncthreads_or(st & 2) ? 2 : 0) | (__syncthreads_or(st & 4) ? 4 : 0);
+        st = block_or_bits<3>(st);
         if (threadIdx.x == 0) *status = st;
     }
 }
@@ -238,17 +232,15 @@ extern "C" int npi_group_topk(const float* scores, const int32_t* group, int64_t
     topk_key_kernel<<<ntiles, KK_THREADS, 0, st>>>(scores, group, n, num_groups, w.keys_a, w.vals_a, w.tile_status);
     NPI_CHECK_LAUNCH();
     const int bits = group_bits(num_groups);
-    int rc = npi_sort_pairs_u32(w.keys_a, w.vals_a, w.keys_b, w.vals_b, n, bits, w.sort_ws, w.sort_bytes, stream);
+    SortedPairs sp;
+    int rc = sort_pairs(w.keys_a, w.vals_a, w.keys_b, w.vals_b, n, bits, w.sort_ws, w.sort_bytes, st, &sp);
     if (rc != NPI_OK) return rc;
-    const bool in_b = npi_sort_passes(bits) & 1;
-    const uint32_t* keys = in_b ? w.keys_b : w.keys_a;
-    const int32_t* vals = in_b ? w.vals_b : w.vals_a;
-    rc = launch_group_bounds(keys, n, num_groups, w.tile_status, ntiles, w.gptr, status, st);
+    rc = launch_group_bounds(sp.keys, n, num_groups, w.tile_status, ntiles, w.gptr, status, st);
     if (rc != NPI_OK) return rc;
     static OncePerDevice once;
     if (once.need())
         NPI_CHECK_CUDA(cudaFuncSetAttribute(group_topk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TK_STAGE * 4));
-    group_topk_kernel<<<num_groups, TK_THREADS, TK_STAGE * 4, st>>>(scores, vals, w.gptr, k, out_pos, out_score, out_count);
+    group_topk_kernel<<<num_groups, TK_THREADS, TK_STAGE * 4, st>>>(scores, sp.vals, w.gptr, k, out_pos, out_score, out_count);
     NPI_CHECK_LAUNCH();
     return NPI_OK;
 }

@@ -193,12 +193,9 @@ class PairSet:
         return len(self.pairs_h)
 
     def batch_caps(self, batch_size, order=None):
-        """Largest (N0, E0, n_graph) over the batches of a sequential pass in ``order``."""
-        P = len(self)
-        idx = np.arange(P) if order is None else np.asarray(order)
+        """Largest (N0, E0, n_graph) over the batches of a sequential pass in ``order`` (pair indices, any length;
+        default: the whole pair set)."""
+        idx = np.arange(len(self)) if order is None else np.asarray(order)
         n, e = self.n_h[idx], self.e_h[idx]
-        nb = (P + batch_size - 1) // batch_size
-        pad = nb * batch_size - P
-        ns = np.concatenate([n, np.zeros(pad, dtype=np.int64)]).reshape(nb, batch_size).sum(1)
-        es = np.concatenate([e, np.zeros(pad, dtype=np.int64)]).reshape(nb, batch_size).sum(1)
-        return int(ns.max()), int(es.max()), int(n.max())
+        starts = np.arange(0, len(idx), batch_size)
+        return int(np.add.reduceat(n, starts).max()), int(np.add.reduceat(e, starts).max()), int(n.max())

@@ -483,6 +483,13 @@ def rank_curve(scores, labels, summary, areas, status, ws, thresholds=None, tps=
            L.ptr(tps), L.ptr(fps), L.ptr(status), L.ptr(ws), _i64(ws.numel() * ws.element_size()), _s())
 
 
+def _group_sort_count_as(entry, num_groups):
+    """Launch-count key of npi_group_topk / npi_group_rank: their launches grow with the passes of the sort by group id
+    (ceil(log2 num_groups) key bits); None for the two-pass default."""
+    passes = L.query("npi_sort_passes", _i32(max(1, (int(num_groups) - 1).bit_length())))
+    return None if passes == 2 else "%s/%dpass" % (entry, passes)
+
+
 def group_topk_workspace_bytes(n_max, num_groups):
     return L.query("npi_group_topk_workspace_bytes", _i64(n_max), _i32(num_groups))
 
@@ -497,10 +504,9 @@ def group_topk(scores, group, num_groups, k, out_pos, out_score, out_count, stat
         raise L.NPIError("group_topk: contiguous float32 scores and int32 group ids of equal length expected")
     if out_pos.numel() < num_groups * k or out_score.numel() < num_groups * k or out_count.numel() < num_groups:
         raise L.NPIError("group_topk: outputs hold fewer than num_groups x k entries")
-    passes = L.query("npi_sort_passes", _i32(max(1, (int(num_groups) - 1).bit_length())))
     L.call("npi_group_topk", L.ptr(scores), L.ptr(group), _i64(n), _i32(num_groups), _i32(k), L.ptr(out_pos),
            L.ptr(out_score), L.ptr(out_count), L.ptr(status), L.ptr(ws), _i64(ws.numel() * ws.element_size()), _s(),
-           count_as=None if passes == 2 else "npi_group_topk/%dpass" % passes)
+           count_as=_group_sort_count_as("npi_group_topk", num_groups))
 
 
 def group_rank_workspace_bytes(n_max, num_groups):
@@ -525,10 +531,9 @@ def group_rank(scores, labels, group, num_groups, hits_k, n_pos, n_neg, twice_u,
             raise L.NPIError("group_rank: outputs of the wrong dtype or holding too few entries (num_groups = %d, n = %d, %d hits)"
                              % (G, n, nh))
     ks = (_i32 * max(nh, 1))(*[int(k) for k in hits_k])
-    passes = L.query("npi_sort_passes", _i32(max(1, (G - 1).bit_length())))
     L.call("npi_group_rank", L.ptr(scores), L.ptr(labels), L.ptr(group), _i64(n), _i32(G), ks, _i32(nh), L.ptr(n_pos),
            L.ptr(n_neg), L.ptr(twice_u), L.ptr(summary), L.ptr(sum_rr), L.ptr(above), L.ptr(tied), L.ptr(status), L.ptr(ws),
-           _i64(ws.numel() * ws.element_size()), _s(), count_as=None if passes == 2 else "npi_group_rank/%dpass" % passes)
+           _i64(ws.numel() * ws.element_size()), _s(), count_as=_group_sort_count_as("npi_group_rank", G))
 
 
 def input_attribution_workspace_bytes(n_rows, B, F):

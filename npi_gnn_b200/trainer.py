@@ -369,11 +369,8 @@ class Scorer:
         self.B = int(batch_size)
         n0 = e0 = mx = 2
         if self.hi > self.lo:
-            sel = slice(self.lo, self.hi) if self.index is None else self.index[self.lo:self.hi]
-            n, e = pairset.n_h[sel], pairset.e_h[sel]
-            starts = np.arange(0, len(n), self.B)
-            n0 = max(n0, int(np.add.reduceat(n, starts).max())); e0 = max(e0, int(np.add.reduceat(e, starts).max()))
-            mx = max(mx, int(n.max()))
+            own = np.arange(self.lo, self.hi) if self.index is None else self.index[self.lo:self.hi]
+            n0, e0, mx = (max(2, v) for v in pairset.batch_caps(self.B, own))
         self.ctx_policy = context_policy(pairset, self.B, n0, e0, mx, g.device, first=self.lo) \
             if (self.index is None and self.hi - self.lo >= self.B) else (None, None)
         self.engine = Engine(g.F, self.B, n0, e0, mx, device=g.device, graph=g, need_backward=False, contexts=self.ctx_policy[0])
@@ -385,12 +382,8 @@ class Scorer:
         self.batches_scored = 0
         self._from_host = False
         self._host_index = None
-        if self.index is not None:       # this rank's slice of the view, padded so a full-batch read never runs off the end
-            own = self.index[self.lo:self.hi].astype(np.int32)
-            pad = np.full(self.B, own[-1] if len(own) else 0, dtype=np.int32)
-            self._host_index = torch.from_numpy(np.concatenate([own, pad]))
-            if torch.cuda.is_available():
-                self._host_index = self._host_index.pin_memory()
+        if self.index is not None:       # this rank's slice of the view
+            self._host_index = _padded_host_index(self.index[self.lo:self.hi], self.B)
 
     def _set_index(self, slot, first):
         if self._from_host or self.index is not None:     # pair indices from pinned host memory (4*B bytes H2D)
@@ -481,9 +474,7 @@ class Scorer:
         ``probabilities()`` returns against the pair labels, plus ``confusion`` = (TP, FN, TN, FP) of the argmax rule,
         all from ONE sweep.  With world_size > 1 every rank's shard is gathered (torch.distributed must be initialised)
         and every rank computes the same, bit-identical result over all pairs -- the confusion counts included."""
-        from . import dist as D
-        if self.world_size > 1 and not D.dist.is_initialized():
-            raise L.NPIError("Scorer.rank_metrics with world_size > 1 needs an initialised torch.distributed process group")
+        self._require_process_group("rank_metrics")
         n = self.hi - self.lo
         scores = torch.empty(n, dtype=torch.float32, device=self.device)
         labels = torch.empty(n, dtype=torch.int32, device=self.device)
@@ -494,10 +485,9 @@ class Scorer:
             labels[o:o + cnt].copy_(self.engine.y_b[:cnt])
             ops.confusion_counts(logp, self.engine.y_b, cnt, -1.0, counts)
         if self.world_size > 1:
-            scores = D.gather_shards(scores, self.P)
-            labels = D.gather_shards(labels, self.P)
+            from . import dist as D
             D.allreduce_sum(counts)
-        out = rank_metrics(scores, labels, curve=curve)
+        out = rank_metrics(self._gathered(scores), self._gathered(labels), curve=curve)
         out["confusion"] = tuple(int(v) for v in counts.cpu())
         return out
 
@@ -510,15 +500,8 @@ class Scorer:
         Ties break by position in the pair set (in ``index`` order when a view was given).  With world_size > 1 every
         rank's shard is gathered (torch.distributed must be initialised) and every rank computes the same,
         bit-identical result over all pairs."""
-        from . import dist as D
-        if not 1 <= int(k) <= 1024:
-            raise ValueError("top_partners: k = %d outside 1..1024" % k)
-        if self.world_size > 1 and not D.dist.is_initialized():
-            raise L.NPIError("Scorer.top_partners with world_size > 1 needs an initialised torch.distributed process group")
-        probs = self.probabilities()
-        if self.world_size > 1:
-            probs = D.gather_shards(probs, self.P)
-        pairs = self.ps.pairs if self.index is None else self.ps.pairs[torch.from_numpy(self.index).to(self.device)]
+        _check_k(k, "top_partners")
+        probs, pairs, _ = self._view_probabilities("top_partners")
         out = {}
         for name, own, other in (("rna", 0, 1), ("protein", 1, 0)):
             r = top_k_by_group(probs, pairs[:, own].contiguous(), self.ps.graph.num_nodes, k)
@@ -544,19 +527,41 @@ class Scorer:
         Honours an ``index`` view.  The result does not depend on the order of the pairs.  With world_size > 1 every
         rank's shard is gathered (torch.distributed must be initialised) and every rank computes the same, bit-identical
         result over all pairs."""
-        from . import dist as D
         ks = _hits_cutoffs(hits, "partner_ranks")
+        probs, pairs, labels = self._view_probabilities("partner_ranks")
+        return {name: group_rank_metrics(probs, labels, pairs[:, own].contiguous(), self.ps.graph.num_nodes, ks)
+                for name, own in (("rna", 0), ("protein", 1))}
+
+    def _require_process_group(self, who):
+        from . import dist as D
         if self.world_size > 1 and not D.dist.is_initialized():
-            raise L.NPIError("Scorer.partner_ranks with world_size > 1 needs an initialised torch.distributed process group")
-        probs = self.probabilities()
-        if self.world_size > 1:
-            probs = D.gather_shards(probs, self.P)
+            raise L.NPIError("Scorer.%s with world_size > 1 needs an initialised torch.distributed process group" % who)
+
+    def _gathered(self, t):
+        """This rank's shard ``t`` of a per-pair tensor -> the whole view's, gathered across ranks."""
+        if self.world_size == 1:
+            return t
+        from . import dist as D
+        return D.gather_shards(t, self.P)
+
+    def _view_probabilities(self, who):
+        """(probabilities, pairs, labels) of the whole view, from one sweep of ``probabilities()`` gathered across ranks;
+        ``who`` names the calling method in the process-group error."""
+        self._require_process_group(who)
+        probs = self._gathered(self.probabilities())
         pairs, labels = self.ps.pairs, self.ps.y
         if self.index is not None:
             idx = torch.from_numpy(self.index).to(self.device)
             pairs, labels = pairs[idx], labels[idx]
-        return {name: group_rank_metrics(probs, labels, pairs[:, own].contiguous(), self.ps.graph.num_nodes, ks)
-                for name, own in (("rna", 0), ("protein", 1))}
+        return probs, pairs, labels
+
+
+def _padded_host_index(index, B):
+    """The pair indices of a view as int32 host memory (pinned when CUDA is available), padded with ``B`` copies of the
+    last entry so that a full-batch read never runs off the end."""
+    own = np.asarray(index).astype(np.int32)
+    host = torch.from_numpy(np.concatenate([own, np.full(B, own[-1] if len(own) else 0, dtype=np.int32)]))
+    return host.pin_memory() if torch.cuda.is_available() else host
 
 
 class Explainer:
@@ -589,12 +594,8 @@ class Explainer:
         if self.P == 0:
             raise ValueError("Explainer: nothing to explain (empty pair set or index view)")
         n = pairset.n_h if index is None else pairset.n_h[index]
-        e = pairset.e_h if index is None else pairset.e_h[index]
         self.n_rows = np.asarray(n, dtype=np.int64)        # rows of every pair's subgraph, in view order
-        starts = np.arange(0, self.P, self.B)
-        n0 = max(2, int(np.add.reduceat(n, starts).max()))
-        e0 = max(2, int(np.add.reduceat(e, starts).max()))
-        mx = max(2, int(n.max()))
+        n0, e0, mx = (max(2, v) for v in pairset.batch_caps(self.B, index))
         g = pairset.graph
         self.device = g.device
         self.engine = Engine(g.F, self.B, n0, e0, mx, device=self.device, graph=g, need_backward=True, contexts=False)
@@ -604,9 +605,8 @@ class Explainer:
         self._seed = torch.zeros(self.B, 2, dtype=torch.float32, device=self.device)
         self._onehot = torch.zeros(self.B, 2, dtype=torch.float32, device=self.device)
         self._pair_index = None
-        if index is not None:            # the view's pair indices, padded so that a batch read never runs off the end
-            host = torch.from_numpy(np.concatenate([index, np.full(self.B, index[-1])]).astype(np.int32))
-            self._host_index = host.pin_memory() if torch.cuda.is_available() else host
+        if index is not None:
+            self._host_index = _padded_host_index(index, self.B)
             self._pair_index = torch.zeros(self.B, dtype=torch.int32, device=self.device)
 
     def explain(self, target=1, wrt="logp", full=False):
@@ -679,8 +679,7 @@ class Explainer:
         as the group; ties by ascending row, i.e. extraction order).  Returns dict of device tensors: node int32 [P, k]
         (the node serials, -1 past count), attr float32 [P, k] (the signed node_attr, NaN past count), count int32 [P] =
         min(k, rows of the pair)."""
-        if not 1 <= int(k) <= 1024:
-            raise ValueError("top_nodes: k = %d outside 1..1024" % k)
+        _check_k(k, "top_nodes")
         na, ptr = result["node_attr"], result["node_ptr"]
         P, R = ptr.numel() - 1, na.numel()
         pair = torch.repeat_interleave(torch.arange(P, dtype=torch.int32, device=na.device), ptr.diff(), output_size=R)
@@ -703,6 +702,28 @@ def metrics(TP, FN, TN, FP):
     return acc, pre, sen, spe, mcc
 
 
+def _check_k(k, who):
+    if not 1 <= int(k) <= 1024:
+        raise ValueError("%s: k = %d outside 1..1024" % (who, k))
+
+
+def _inputs_and_workspace(tensors, workspace_bytes, *args):
+    """The CUDA ``tensors`` flattened and contiguous, and a device workspace of workspace_bytes(n, *args) bytes for their
+    n items (at least 1)."""
+    L.require_cuda(*tensors)
+    flat = [t.reshape(-1).contiguous() for t in tensors]
+    ws = torch.empty(workspace_bytes(max(flat[0].numel(), 1), *args), dtype=torch.uint8, device=flat[0].device)
+    return flat, ws
+
+
+def _raise_status(st, *messages):
+    """Raises NPIError with messages[b] for the lowest bit b set in the nonzero status word ``st`` of an entry point;
+    ``messages`` lists the meanings of its status bits 0, 1, ...."""
+    for b, msg in enumerate(messages):
+        if st >> b & 1:
+            raise L.NPIError(msg)
+
+
 def rank_metrics(scores, labels, curve=False):
     """Threshold-free metrics of CUDA float32 ``scores`` against int32 0/1 ``labels`` in ONE call of npi_rank_curve and
     one synchronising read: dict(auroc, ap, pr_auc_trapz, n_pos, n_neg, twice_u) -- sklearn's roc_auc_score,
@@ -710,13 +731,11 @@ def rank_metrics(scores, labels, curve=False):
     src/compare_withKmer_noKmer.py.  ``curve=True`` adds the device tensors thresholds (float32), fpr, tpr, precision
     and recall (float64), one entry per distinct score in descending order.  NaN scores or labels other than 0/1 raise
     NPIError; a single class raises ValueError (ROC AUC is undefined)."""
-    L.require_cuda(scores, labels)
-    scores, labels = scores.reshape(-1).contiguous(), labels.reshape(-1).contiguous()
+    (scores, labels), ws = _inputs_and_workspace((scores, labels), ops.rank_workspace_bytes)
     n = scores.numel()
     dev = scores.device
     res = torch.zeros(7, dtype=torch.int64, device=dev)     # summary[4] | areas[2] (fp64) | status (int32)
     summary, areas, status = res[:4], res[4:6].view(torch.float64), res[6:7].view(torch.int32)[:1]
-    ws = torch.empty(ops.rank_workspace_bytes(max(n, 1)), dtype=torch.uint8, device=dev)
     thr = tps = fps = None
     if curve:
         thr = torch.empty(n, dtype=torch.float32, device=dev)
@@ -725,10 +744,8 @@ def rank_metrics(scores, labels, curve=False):
     ops.rank_curve(scores, labels, summary, areas, status, ws, thr, tps, fps)
     h = res.cpu()
     st = int(h[6:7].view(torch.int32)[0])
-    if st & 1:
-        raise L.NPIError("rank_metrics: NaN score")
-    if st & 2:
-        raise L.NPIError("rank_metrics: label other than 0 or 1")
+    if st:
+        _raise_status(st, "rank_metrics: NaN score", "rank_metrics: label other than 0 or 1")
     n_pos, n_neg, T, twice_u = (int(v) for v in h[:4])
     if n_pos == 0 or n_neg == 0:
         raise ValueError("Only one class present in the labels: ROC AUC is not defined in that case")
@@ -751,23 +768,18 @@ def top_k_by_group(scores, group, num_groups, k):
     +0.0 tie), -1 past count; score float32 [num_groups, k], those scores bit for bit, NaN past count; count int32
     [num_groups] = min(k, group size).  NaN scores or group ids out of range raise NPIError; k outside 1..1024 raises
     ValueError."""
-    if not 1 <= int(k) <= 1024:
-        raise ValueError("top_k_by_group: k = %d outside 1..1024" % k)
-    L.require_cuda(scores, group)
-    scores, group = scores.reshape(-1).contiguous(), group.reshape(-1).contiguous()
+    _check_k(k, "top_k_by_group")
+    (scores, group), ws = _inputs_and_workspace((scores, group), ops.group_topk_workspace_bytes, int(num_groups))
     dev = scores.device
     G, k = int(num_groups), int(k)
     pos = torch.empty((G, k), dtype=torch.int32, device=dev)
     score = torch.empty((G, k), dtype=torch.float32, device=dev)
     count = torch.empty(G, dtype=torch.int32, device=dev)
     status = torch.empty(1, dtype=torch.int32, device=dev)
-    ws = torch.empty(ops.group_topk_workspace_bytes(max(scores.numel(), 1), G), dtype=torch.uint8, device=dev)
     ops.group_topk(scores, group, G, k, pos, score, count, status, ws)
     st = int(status.item())
-    if st & 1:
-        raise L.NPIError("top_k_by_group: NaN score")
-    if st & 2:
-        raise L.NPIError("top_k_by_group: group id out of range [0, %d)" % G)
+    if st:
+        _raise_status(st, "top_k_by_group: NaN score", "top_k_by_group: group id out of range [0, %d)" % G)
     return dict(pos=pos, score=score, count=count)
 
 
@@ -803,8 +815,7 @@ def group_rank_metrics(scores, labels, group, num_groups, hits=(1, 3, 10), per_i
     G = int(num_groups)
     if G < 1:
         raise ValueError("group_rank_metrics: num_groups = %d, expected >= 1" % G)
-    L.require_cuda(scores, labels, group)
-    scores, labels, group = (t.reshape(-1).contiguous() for t in (scores, labels, group))
+    (scores, labels, group), ws = _inputs_and_workspace((scores, labels, group), ops.group_rank_workspace_bytes, G)
     n, nh, dev = scores.numel(), len(ks), scores.device
     res = torch.zeros(16, dtype=torch.int64, device=dev)    # summary[3 + nh] | sum_rr | sum of defined AUCs | status
     summary = res[:3 + nh]
@@ -815,19 +826,15 @@ def group_rank_metrics(scores, labels, group, num_groups, hits=(1, 3, 10), per_i
     twice_u = torch.empty(G, dtype=torch.int64, device=dev)
     above = torch.empty(n, dtype=torch.int32, device=dev) if per_item else None
     tied = torch.empty(n, dtype=torch.int32, device=dev) if per_item else None
-    ws = torch.empty(ops.group_rank_workspace_bytes(max(n, 1), G), dtype=torch.uint8, device=dev)
     ops.group_rank(scores, labels, group, G, ks, n_pos, n_neg, twice_u, summary, sum_rr, status, ws, above, tied)
     both = (n_pos > 0) & (n_neg > 0)
     auc = torch.where(both, twice_u.double() / (2.0 * n_pos.double() * n_neg.double()), float("nan"))
     auc_sum.copy_(torch.where(both, auc, 0.0).sum().reshape(1))
     h = res.cpu()
     st = int(h[13:14].view(torch.int32)[0])
-    if st & 1:
-        raise L.NPIError("group_rank_metrics: NaN score")
-    if st & 2:
-        raise L.NPIError("group_rank_metrics: label other than 0 or 1")
-    if st & 4:
-        raise L.NPIError("group_rank_metrics: group id out of range [0, %d)" % G)
+    if st:
+        _raise_status(st, "group_rank_metrics: NaN score", "group_rank_metrics: label other than 0 or 1",
+                      "group_rank_metrics: group id out of range [0, %d)" % G)
     nq, nu, ng = (int(v) for v in h[:3])
     if nq == 0:
         raise ValueError("group_rank_metrics: no query has a competitor in its group: MRR is not defined in that case")

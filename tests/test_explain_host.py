@@ -71,3 +71,16 @@ def test_top_nodes_rejects_k(k):
     res = dict(node_attr=torch.zeros(4), node_ptr=torch.tensor([0, 4]), node=torch.zeros(4, dtype=torch.int32))
     with pytest.raises(ValueError, match="k"):
         Explainer.top_nodes(res, k)
+
+
+@pytest.mark.parametrize("order", [None, [3], [7, 2, 9], np.arange(10)[::-1], [1, 1, 1, 1, 1, 1, 1, 1, 1, 1, 1, 1, 1]])
+def test_batch_caps_of_a_view_sums_each_batch_of_the_view(order):
+    """PairSet.batch_caps over an ``order`` of any length (the Scorer and Explainer views) against plain per-batch sums."""
+    from npi_gnn_b200.graph import PairSet
+    ps, B = _HostPairSet(10), 4
+    ps.n_h = np.arange(10, dtype=np.int64) + 2
+    ps.e_h = 3 * np.arange(10, dtype=np.int64)[::-1] + 1
+    idx = np.arange(10) if order is None else np.asarray(order)
+    batches = [idx[i:i + B] for i in range(0, len(idx), B)]
+    want = (max(int(ps.n_h[b].sum()) for b in batches), max(int(ps.e_h[b].sum()) for b in batches), int(ps.n_h[idx].max()))
+    assert PairSet.batch_caps(ps, B, order) == want

@@ -9,6 +9,7 @@ import numpy as np
 import pytest
 import torch
 
+from tests.common import config5_pairs, fold0, grouped, ties
 from tests.test_partner_rank_host import oracle
 
 pytestmark = pytest.mark.gpu
@@ -47,18 +48,6 @@ def _check(s, y, grp, G, hits=HITS):
     r = _gpu(s, y, grp, G, hits)
     _assert_same(r, oracle(s, y, grp, G, hits), hits)
     return r
-
-
-def _ties(rng, n):
-    """Scores on a grid of 49 values (heavy ties), 5 % of them -0.0."""
-    s = (rng.integers(-24, 25, n) / 8.0).astype(np.float32)
-    s[rng.random(n) < 0.05] = -0.0
-    return s
-
-
-def _grouped(rng, sizes):
-    grp = np.repeat(np.arange(len(sizes), dtype=np.int32), sizes)
-    return grp[rng.permutation(len(grp))]
 
 
 def _labels(rng, n, p=0.2):
@@ -100,9 +89,9 @@ def test_infinities_are_ordinary_scores():
 def test_empty_groups_first_last_and_between():
     rng = np.random.default_rng(2)
     sizes = [0, 4, 0, 0, 9, 1, 0, 30, 0, 300, 0]
-    grp = _grouped(rng, sizes)
+    grp = grouped(rng, sizes)
     y = _labels(rng, len(grp), 0.4)
-    r = _check(_ties(rng, len(grp)), y, grp, len(sizes))
+    r = _check(ties(rng, len(grp)), y, grp, len(sizes))
     for g in (0, 2, 3, 6, 8, 10):
         assert r["n_pos"][g] == 0 and r["n_neg"][g] == 0 and r["twice_u"][g] == 0 and torch.isnan(r["auc"][g])
 
@@ -111,7 +100,7 @@ def test_groups_of_queries_only_are_unranked_and_groups_of_competitors_only_unsc
     rng = np.random.default_rng(4)
     grp = np.array([0] * 5 + [1] * 7 + [2] * 9 + [3] * 3, dtype=np.int32)
     y = np.array([1] * 5 + [0] * 7 + [1, 0] * 4 + [1] + [1, 1, 0], dtype=np.int32)
-    r = _check(_ties(rng, len(grp)), y, grp, 4)
+    r = _check(ties(rng, len(grp)), y, grp, 4)
     assert r["n_unranked"] == 5 and r["n_queries"] == 5 + 2 and r["n_groups_scored"] == 2
     assert (r["above"].cpu().numpy()[:5] == 0).all() and (r["tied"].cpu().numpy()[:5] == 0).all()
     assert torch.isnan(r["auc"][:2]).all()
@@ -137,9 +126,9 @@ def test_single_item():
 def test_one_group_of_2_20_items():
     rng = np.random.default_rng(20)
     n = 1 << 20
-    _check(_ties(rng, n), _labels(rng, n, 0.01), np.zeros(n, dtype=np.int32), 1)
+    _check(ties(rng, n), _labels(rng, n, 0.01), np.zeros(n, dtype=np.int32), 1)
     grp = np.where(rng.random(n) < 0.001, 2, 1).astype(np.int32)     # one huge group between an empty and a small one
-    _check(_ties(rng, n), _labels(rng, n, 0.3), grp, 3, hits=(1, 2, 5, 10, 100, 1000, 10000, 100000))
+    _check(ties(rng, n), _labels(rng, n, 0.3), grp, 3, hits=(1, 2, 5, 10, 100, 1000, 10000, 100000))
 
 
 def test_more_than_2_18_groups():
@@ -148,16 +137,16 @@ def test_more_than_2_18_groups():
     G = (1 << 18) + 4321
     sizes = rng.integers(0, 8, G)
     sizes[rng.random(G) < 0.001] = 700
-    grp = _grouped(rng, sizes)
-    _check(_ties(rng, len(grp)), _labels(rng, len(grp), 0.3), grp, G)
+    grp = grouped(rng, sizes)
+    _check(ties(rng, len(grp)), _labels(rng, len(grp), 0.3), grp, G)
 
 
 def test_shuffled_group_ids():
     """Group ids relabelled by a random permutation: the per-group outputs follow the labels, the summary stays."""
     rng = np.random.default_rng(6)
     sizes = rng.integers(0, 400, 1000)
-    grp = _grouped(rng, sizes)
-    s, y = _ties(rng, len(grp)), _labels(rng, len(grp))
+    grp = grouped(rng, sizes)
+    s, y = ties(rng, len(grp)), _labels(rng, len(grp))
     relabel = rng.permutation(1000).astype(np.int32)
     r = _check(s, y, relabel[grp], 1000)
     r0 = _gpu(s, y, grp, 1000)
@@ -242,21 +231,10 @@ def test_argument_checks():
 
 
 # ----------------------------------------------------------------------------- full size
-def _config5():
-    from npi_gnn_b200 import synth
-    d = synth.npinter2_shaped()
-    allp = synth.all_candidate_pairs(d)
-    V = len(d["is_rna"])
-    pos = np.asarray(d["pos"])
-    key = allp[:, 0].astype(np.int64) * V + allp[:, 1]
-    y = np.isin(key, pos[:, 0].astype(np.int64) * V + pos[:, 1]).astype(np.int32)
-    return allp, y, V
-
-
 def test_config5_groupings_full_size():
     """All 2,081,564 RNA x protein pairs of the NPInter2-shaped graph, the known interactions as queries, probabilities on
     a 1e-4 grid, grouped by RNA and by protein with node serials as group ids."""
-    allp, y, V = _config5()
+    allp, y, V = config5_pairs()
     assert 5000 < y.sum() < 20000
     s = np.round(np.random.default_rng(7).random(len(allp)), 4).astype(np.float32)
     for col in (0, 1):
@@ -277,9 +255,9 @@ def _out(bufs):
 def test_bit_identical_on_rerun_and_under_permutation():
     rng = np.random.default_rng(8)
     G = 3000
-    grp_np = _grouped(rng, rng.integers(0, 300, G))
+    grp_np = grouped(rng, rng.integers(0, 300, G))
     n = len(grp_np)
-    s_np, y_np = _ties(rng, n), _labels(rng, n, 0.1)
+    s_np, y_np = ties(rng, n), _labels(rng, n, 0.1)
     s, y, grp = _t(s_np, np.float32), _t(y_np, np.int32), _t(grp_np, np.int32)
     bufs = _bufs(n, G, 3)
     _run(s, y, grp, G, bufs)
@@ -305,9 +283,9 @@ def test_bit_identical_on_rerun_and_under_permutation():
 def test_cuda_graph_capture_and_replay_on_new_scores():
     rng = np.random.default_rng(9)
     G = 700
-    grp_np = _grouped(rng, rng.integers(0, 500, G))
+    grp_np = grouped(rng, rng.integers(0, 500, G))
     n = len(grp_np)
-    s0, s1, y_np = _ties(rng, n), _ties(rng, n), _labels(rng, n)
+    s0, s1, y_np = ties(rng, n), ties(rng, n), _labels(rng, n)
     s, y, grp = _t(s0, np.float32), _t(y_np, np.int32), _t(grp_np, np.int32)
     bufs = _bufs(n, G, 3)
     side = torch.cuda.Stream()
@@ -341,7 +319,7 @@ def test_launch_count_matches_kernels_per_call(G):
     from npi_gnn_b200 import _lib as L
     rng = np.random.default_rng(G)
     n = 20000
-    s, y, grp = _t(_ties(rng, n), np.float32), _t(_labels(rng, n), np.int32), _t(rng.integers(0, G, n), np.int32)
+    s, y, grp = _t(ties(rng, n), np.float32), _t(_labels(rng, n), np.int32), _t(rng.integers(0, G, n), np.int32)
     bufs = _bufs(n, G, 3)
     _run(s, y, grp, G, bufs)
     torch.cuda.synchronize()
@@ -360,8 +338,7 @@ def _fold0_with_candidates():
     """The NPInter2 fold-0 graph with the test pairs masked, the shipped checkpoint, and a pair set of the test positives
     (label 1), the test negatives and the candidate pairs of the first 100 RNAs with a test positive (label 0)."""
     from npi_gnn_b200.graph import PairSet
-    from tests.test_gpu_rank import _fold0
-    d, og, omask, pairs, ys, ps, params = _fold0()
+    d, og, omask, pairs, ys, ps, params = fold0()
     g = ps.graph
     cand = g.candidate_pairs()
     cand = cand[np.isin(cand[:, 0], np.unique(d["test_pos"][:, 0])[:100])]
@@ -400,8 +377,7 @@ def test_scorer_partner_ranks_on_npinter2_fold0():
 def test_scorer_partner_ranks_needs_a_process_group_when_sharded():
     from npi_gnn_b200 import NPIError
     from npi_gnn_b200.trainer import Scorer
-    from tests.test_gpu_rank import _fold0
-    d, og, omask, pairs, ys, ps, params = _fold0()
+    d, og, omask, pairs, ys, ps, params = fold0()
     with pytest.raises(NPIError, match="process group"):
         Scorer(ps, params, batch_size=200, world_size=2, rank=0).partner_ranks()
 
@@ -409,7 +385,8 @@ def test_scorer_partner_ranks_needs_a_process_group_when_sharded():
 @pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs")
 def test_partner_ranks_two_gpus_match_one():
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node=2",
-           "--master-addr", "127.0.0.1", "--master-port", "29643", os.path.join(ROOT, "tests", "partner_rank_worker.py")]
+           "--master-addr", "127.0.0.1", "--master-port", "29643", os.path.join(ROOT, "tests", "scorer_dp_worker.py"),
+           "partner_ranks"]
     out = subprocess.run(cmd, capture_output=True, text=True, timeout=600)
     print(out.stdout[-3000:])
     assert out.returncode == 0, out.stderr[-3000:]

@@ -10,7 +10,7 @@ import numpy as np
 import pytest
 import torch
 
-from tests.common import load_ckpt, npinter2_oracle_graph, oracle_batches
+from tests.common import fold0, load_ckpt, oracle_batches
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -234,23 +234,10 @@ def test_cuda_graph_capture_and_replay_on_new_inputs():
 
 
 # ----------------------------------------------------------------------------- Scorer on the real fold-0 test set
-def _fold0():
-    from npi_gnn_b200.engine import FlatParams
-    from npi_gnn_b200.graph import BipartiteGraph, PairSet
-    d, og, omask = npinter2_oracle_graph()
-    g = BipartiteGraph(d["edges"], d["is_rna"], d["table"])
-    g.set_mask(np.concatenate([d["test_pos"], d["test_neg"]]))
-    pairs = np.concatenate([d["test_pos"], d["test_neg"]])
-    ys = np.concatenate([np.ones(len(d["test_pos"])), np.zeros(len(d["test_neg"]))]).astype(np.int32)
-    ps = PairSet(g, pairs, ys, h=1)
-    params = FlatParams(g.F, "cuda").load_state_dict(load_ckpt("ckpt_1223_1_15.npz"))
-    return d, og, omask, pairs, ys, ps, params
-
-
 def test_scorer_rank_metrics_on_npinter2_fold0():
     from npi_gnn_b200.trainer import Scorer
     from oracle import net as onet
-    d, og, omask, pairs, ys, ps, params = _fold0()
+    d, og, omask, pairs, ys, ps, params = fold0()
     sc = Scorer(ps, params, batch_size=200)
     r = sc.rank_metrics(curve=True)
     p = sc.probabilities().cpu().numpy()
@@ -284,7 +271,7 @@ def test_scorer_rank_metrics_on_npinter2_fold0():
 def test_scorer_rank_metrics_needs_a_process_group_when_sharded():
     from npi_gnn_b200 import NPIError
     from npi_gnn_b200.trainer import Scorer
-    d, og, omask, pairs, ys, ps, params = _fold0()
+    d, og, omask, pairs, ys, ps, params = fold0()
     with pytest.raises(NPIError, match="process group"):
         Scorer(ps, params, batch_size=200, world_size=2, rank=0).rank_metrics()
 
@@ -292,7 +279,8 @@ def test_scorer_rank_metrics_needs_a_process_group_when_sharded():
 @pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs")
 def test_rank_metrics_two_gpus_match_one():
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node=2",
-           "--master-addr", "127.0.0.1", "--master-port", "29637", os.path.join(ROOT, "tests", "rank_worker.py")]
+           "--master-addr", "127.0.0.1", "--master-port", "29637", os.path.join(ROOT, "tests", "scorer_dp_worker.py"),
+           "rank_metrics"]
     out = subprocess.run(cmd, capture_output=True, text=True, timeout=600)
     print(out.stdout[-3000:])
     assert out.returncode == 0, out.stderr[-3000:]

@@ -9,7 +9,7 @@ import numpy as np
 import pytest
 import torch
 
-from tests.common import synthetic_bipartite
+from tests.common import config5_pairs, fold0, grouped, synthetic_bipartite, ties
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -57,24 +57,11 @@ def _check(s, grp, G, k):
     _assert_same(_gpu(s, grp, G, k), oracle(s, grp, G, k))
 
 
-def _ties(rng, n):
-    """Scores on a grid of 49 values (heavy ties), 5 % of them -0.0."""
-    s = (rng.integers(-24, 25, n) / 8.0).astype(np.float32)
-    s[rng.random(n) < 0.05] = -0.0
-    return s
-
-
-def _grouped(rng, sizes):
-    """Group ids with the given member counts (empty groups allowed), items in shuffled order."""
-    grp = np.repeat(np.arange(len(sizes), dtype=np.int32), sizes)
-    return grp[rng.permutation(len(grp))]
-
-
 # ----------------------------------------------------------------------------- hand cases
 def test_k_larger_than_every_group():
     rng = np.random.default_rng(1)
-    grp = _grouped(rng, [3, 1, 5, 2, 4])
-    s = _ties(rng, len(grp))
+    grp = grouped(rng, [3, 1, 5, 2, 4])
+    s = ties(rng, len(grp))
     got = _gpu(s, grp, 5, 7)
     assert list(got[2]) == [3, 1, 5, 2, 4]
     _assert_same(got, oracle(s, grp, 5, 7))
@@ -83,8 +70,8 @@ def test_k_larger_than_every_group():
 def test_empty_groups_first_last_and_between():
     rng = np.random.default_rng(2)
     sizes = [0, 4, 0, 0, 9, 1, 0, 30, 0]
-    grp = _grouped(rng, sizes)
-    s = _ties(rng, len(grp))
+    grp = grouped(rng, sizes)
+    s = ties(rng, len(grp))
     pos, sc, cnt = _gpu(s, grp, len(sizes), 8)
     assert list(cnt) == [min(c, 8) for c in sizes]
     for g in (0, 2, 3, 6, 8):
@@ -126,8 +113,8 @@ def test_infinities_are_ordinary_scores():
 def test_smallest_and_largest_k(k):
     rng = np.random.default_rng(k)
     sizes = [1, 2, 1023, 1024, 1025, 3000, 0, 20000]
-    grp = _grouped(rng, sizes)
-    _check(_ties(rng, len(grp)), grp, len(sizes), k)
+    grp = grouped(rng, sizes)
+    _check(ties(rng, len(grp)), grp, len(sizes), k)
 
 
 def test_single_item():
@@ -194,8 +181,8 @@ def test_group_sizes_across_the_stage(size, k):
     holds its unique top score, so a group cut at the stage loses its first entry."""
     rng = np.random.default_rng(size * 7 + k)
     sizes = [size, 5, size, 0, size, 1500]
-    grp = _grouped(rng, sizes)
-    s = _ties(rng, len(grp))
+    grp = grouped(rng, sizes)
+    s = ties(rng, len(grp))
     for g in range(len(sizes)):
         members = np.nonzero(grp == g)[0]
         if len(members):
@@ -211,9 +198,9 @@ def test_group_sizes_across_the_stage(size, k):
 def test_one_group_of_2_20_items(k):
     rng = np.random.default_rng(20 + k)
     n = 1 << 20
-    _check(_ties(rng, n), np.zeros(n, dtype=np.int32), 1, k)
+    _check(ties(rng, n), np.zeros(n, dtype=np.int32), 1, k)
     grp = np.where(rng.random(n) < 0.001, 2, 1).astype(np.int32)    # one huge group between an empty and a small one
-    _check(_ties(rng, n), grp, 3, k)
+    _check(ties(rng, n), grp, 3, k)
 
 
 def test_more_groups_than_eight_per_sm():
@@ -222,16 +209,16 @@ def test_more_groups_than_eight_per_sm():
     G = 8 * ops.sm_count() + 37
     sizes = rng.integers(0, 60, G)
     sizes[rng.random(G) < 0.02] = 2000
-    grp = _grouped(rng, sizes)
-    _check(_ties(rng, len(grp)), grp, G, 16)
+    grp = grouped(rng, sizes)
+    _check(ties(rng, len(grp)), grp, G, 16)
 
 
 def test_shuffled_group_ids():
     """Group ids relabelled by a random permutation and items in random order: rows follow the labels."""
     rng = np.random.default_rng(5)
     sizes = rng.integers(0, 400, 1000)
-    grp = _grouped(rng, sizes)
-    s = _ties(rng, len(grp))
+    grp = grouped(rng, sizes)
+    s = ties(rng, len(grp))
     relabel = rng.permutation(1000).astype(np.int32)
     _check(s, relabel[grp], 1000, 50)
     pos, sc, cnt = _gpu(s, relabel[grp], 1000, 50)
@@ -239,17 +226,11 @@ def test_shuffled_group_ids():
     assert np.array_equal(pos[relabel], p0) and np.array_equal(cnt[relabel], c0)
 
 
-def _config5():
-    from npi_gnn_b200 import synth
-    d = synth.npinter2_shaped()
-    return synth.all_candidate_pairs(d), len(d["is_rna"])
-
-
 @pytest.mark.parametrize("k", [10, 100])
 def test_config5_groupings_full_size(k):
     """All 2,081,564 RNA x protein pairs of the NPInter2-shaped graph, probabilities on a 1/64 grid, grouped by RNA
     (449 members per group) and by protein (4,636 members), node serials as group ids (num_groups = all nodes)."""
-    allp, V = _config5()
+    allp, _, V = config5_pairs()
     rng = np.random.default_rng(k)
     s = (rng.integers(0, 65, len(allp)) / 64.0).astype(np.float32)
     for col, members in ((0, 449), (1, 4636)):
@@ -280,8 +261,8 @@ def _out(bufs):
 def test_bit_identical_on_rerun():
     rng = np.random.default_rng(6)
     sizes = rng.integers(0, 3 * STAGE, 300)
-    grp_np = _grouped(rng, sizes)
-    s, grp = torch.as_tensor(_ties(rng, len(grp_np))).cuda(), torch.as_tensor(grp_np).cuda()
+    grp_np = grouped(rng, sizes)
+    s, grp = torch.as_tensor(ties(rng, len(grp_np))).cuda(), torch.as_tensor(grp_np).cuda()
     bufs = _bufs(len(grp_np), 300, 200)
     _run(s, grp, 300, 200, bufs)
     first = _out(bufs)
@@ -311,9 +292,9 @@ def test_cuda_graph_capture_and_replay_on_new_scores():
     G, k = 500, 64
     sizes = rng.integers(0, 2 * STAGE // 50, G)
     sizes[:3] = (STAGE + 100, 0, 3 * STAGE)                           # the reread path inside the graph too
-    grp_np = _grouped(rng, sizes)
+    grp_np = grouped(rng, sizes)
     n = len(grp_np)
-    s0, s1 = _ties(rng, n), _ties(rng, n)
+    s0, s1 = ties(rng, n), ties(rng, n)
     s, grp = torch.as_tensor(s0).cuda(), torch.as_tensor(grp_np).cuda()
     bufs = _bufs(n, G, k)
     side = torch.cuda.Stream()
@@ -348,8 +329,7 @@ def _check_partners(r, probs, pairs, V, k):
 
 def test_scorer_top_partners_on_npinter2_fold0():
     from npi_gnn_b200.trainer import Scorer
-    from tests.test_gpu_rank import _fold0
-    d, og, omask, pairs, ys, ps, params = _fold0()
+    d, og, omask, pairs, ys, ps, params = fold0()
     sc = Scorer(ps, params, batch_size=200)
     r = sc.top_partners(5)
     probs = sc.probabilities().cpu().numpy()
@@ -380,8 +360,7 @@ def test_scorer_top_partners_over_candidate_pairs():
 def test_scorer_top_partners_needs_a_process_group_when_sharded():
     from npi_gnn_b200 import NPIError
     from npi_gnn_b200.trainer import Scorer
-    from tests.test_gpu_rank import _fold0
-    d, og, omask, pairs, ys, ps, params = _fold0()
+    d, og, omask, pairs, ys, ps, params = fold0()
     with pytest.raises(NPIError, match="process group"):
         Scorer(ps, params, batch_size=200, world_size=2, rank=0).top_partners(5)
 
@@ -389,7 +368,8 @@ def test_scorer_top_partners_needs_a_process_group_when_sharded():
 @pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs")
 def test_top_partners_two_gpus_match_one():
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node=2",
-           "--master-addr", "127.0.0.1", "--master-port", "29641", os.path.join(ROOT, "tests", "topk_worker.py")]
+           "--master-addr", "127.0.0.1", "--master-port", "29641", os.path.join(ROOT, "tests", "scorer_dp_worker.py"),
+           "top_partners"]
     out = subprocess.run(cmd, capture_output=True, text=True, timeout=600)
     print(out.stdout[-3000:])
     assert out.returncode == 0, out.stderr[-3000:]
